@@ -4,7 +4,7 @@
 A "step" is ONE reverse-rate evaluation fused with the tau-leaping state update (TauL predictor step,
 reference lib/sampling/sampling.py:119-160) over the per-GPU batch of the named workload, on synthetic logits.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C4|C3|C2|C1] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C4|C3|C2|C1] [--impl ours|reference] [--dump-outputs DIR]
 
 Workloads (BASELINE.json configs / SURVEY.md §8d):
   C4  CIFAR10-shape  S=256 D=3072 B=1024/GPU GaussianTargetRate, TauL   <- default (the metric's config)
@@ -240,6 +240,26 @@ def flops_per_step(B, D, S):
     return 2.0 * B * D * S * S
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(d, arrays):
+    """Write the arrays of the last timed step as d/<name>.npy: integer states as float32 (exact below 2^24), int64
+    counters as float64, 64 MB at most in all.  Arrays are taken smallest first, each whole when it fits an equal share of
+    what is left, else as a fixed, seeded sample of its flat elements of that size."""
+    os.makedirs(d, exist_ok=True)
+    out = {k: v.detach().cpu().numpy().astype(np.float64 if v.dtype in (torch.int64, torch.float64) else np.float32)
+           for k, v in arrays.items()}
+    left = DUMP_BYTES
+    for i, (k, a) in enumerate(sorted(out.items(), key=lambda kv: kv[1].nbytes)):
+        share = left // (len(out) - i)
+        if a.nbytes > share:
+            keep = max(1, share // a.itemsize)
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        left -= a.nbytes
+        np.save(os.path.join(d, k + ".npy"), a)
+
+
 def run_reference(args, w, rank, world):
     if rank != 0:
         return
@@ -340,6 +360,8 @@ def run_ours(args, w, rank, world, local_rank):
     if world > 1:
         dist.all_reduce(t_ms, op=dist.ReduceOp.MAX)
     ms = float(t_ms.item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"x": x, "stats": stats[W + K - 1]})
 
     # ---- end to end through the C ABI with HOST buffers: H2D logits + state, step, D2H new state, every step ----
     e2e_steps = max(1, min(K, args.e2e_steps))
@@ -820,9 +842,9 @@ def run_ours_c5(args, w, rank, world, local_rank):
             ctx.__enter__()
         for i in range(K):
             ev[0].record()
-            mid(W + i, i % 3)
+            xm = mid(W + i, i % 3)
             ev[1].record()
-            loss_step()
+            loss = loss_step()
             ev[2].record()
             torch.cuda.synchronize(dev)
             tm += ev[0].elapsed_time(ev[1])
@@ -831,6 +853,7 @@ def run_ours_c5(args, w, rank, world, local_rank):
             ctx.__exit__(None, None, None)
         barrier()
         launches = nat.launch_count() - n0
+        last = {"x": xm, "loss": loss.detach(), "grad_w": model.w.grad.detach().clone()}
         # end to end through the public API with HOST inputs: the minibatch comes from pinned host memory, the loss value
         # is read back (.item()), one MidPointTauL-style step on the resident logits in between
         host_mb = torch.empty((B, D), dtype=torch.int64, pin_memory=True)
@@ -848,13 +871,15 @@ def run_ours_c5(args, w, rank, world, local_rank):
         t = torch.tensor([tm / K, tl / K, e2e], dtype=torch.float64, device=dev)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        return float(t[0]), float(t[1]), float(t[2]), launches, (ctx.summary() if ctx else None)
+        return float(t[0]), float(t[1]), float(t[2]), launches, (ctx.summary() if ctx else None), last
 
     rows = []
     for tot in totals:
         B = -(-tot // world)
-        tmid, tloss, e2e, launches, clocks = one(B, clk=(tot == totals[-1]))
+        tmid, tloss, e2e, launches, clocks, last = one(B, clk=(tot == totals[-1]))
         rows.append(dict(total_batch=B * world, per_gpu=B, midpoint_ms=tmid, loss_ms=tloss, e2e_ms=e2e, launches=launches, clocks=clocks))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)       # the largest batch of a sweep
     if rank != 0:
         return
     r = rows[-1]
@@ -922,7 +947,15 @@ def main():
     ap.add_argument("--batch", type=int, default=0, help="override the per-GPU batch of the workload (diagnostic)")
     ap.add_argument("--total-batch", type=int, default=0, help="C5: total batch over all GPUs (64..4096)")
     ap.add_argument("--sweep", action="store_true", help="C5: run the whole batch sweep 64..4096 (the line reports the largest)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (new states; C1-C4: its counters, C5: "
+                         "loss and gradient) as DIR/<name>.npy, rank 0's rows; inputs are seeded, so runs compare (C5's "
+                         "loss and gradient are float sums in no fixed order: compare those with a tolerance)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the CUDA path computed (--impl ours)")
     # stdout carries exactly ONE JSON line: libraries that write to file descriptor 1 (NCCL prints its version banner
     # there when NCCL_DEBUG is set) are sent to stderr for the whole run; the result line goes to the saved descriptor
     global _RESULT_OUT
@@ -930,6 +963,9 @@ def main():
     _RESULT_OUT = os.fdopen(os.dup(1), "w")
     os.dup2(2, 1)
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
+    # the default generators draw the starting states (C1-C4) and the loss's time draws (C5): seeded, so that the same
+    # arguments give the same inputs in every run
+    torch.manual_seed(0xC7DD)
     w = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
