@@ -24,11 +24,11 @@ NVCC_FLAGS = [
 ]
 
 
-if os.environ.get("CTDD_TRACE"):   # diagnostic build: per-tile clock stamps in the tcgen05 kernel (tools/tc_trace.py)
+if os.environ.get("CTDD_TRACE"):   # diagnostic build: per-tile clock stamps in step_q_kernel (tools/tcq_trace.py)
     NVCC_FLAGS.append("-DCTDD_TC_TRACE")
 
 
-for _flag in os.environ.get("CTDD_DEFINES", "").split():   # diagnostic builds, e.g. CTDD_DEFINES="CTDD_EXP_NOSAMPLE"
+for _flag in os.environ.get("CTDD_DEFINES", "").split():   # diagnostic builds, e.g. CTDD_DEFINES="CTDD_EXP_NOPICK"
     NVCC_FLAGS.append("-D" + _flag)
 
 

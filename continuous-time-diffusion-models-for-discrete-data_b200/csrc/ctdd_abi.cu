@@ -19,6 +19,7 @@ void count_launch(int n) { g_launches.fetch_add(n, std::memory_order_relaxed); }
 
 int launch_step_simt(const ctdd_step_params* p, cudaStream_t st);
 int launch_step_tc(const ctdd_step_params* p, cudaStream_t st);
+int launch_step_tcq(const ctdd_step_params* p, cudaStream_t st);
 bool tc_supports(const ctdd_step_params* p);
 long long tc_workspace_bytes(long long rows, int S);
 
@@ -58,7 +59,9 @@ extern "C" int ctdd_reverse_step(const ctdd_step_params* p, void* stream) {
   const bool want_tc = (p->impl == CTDD_IMPL_TC) || (p->impl == CTDD_IMPL_AUTO && tc_supports(p));
   if (want_tc) {
     if (!tc_supports(p)) { set_error("ctdd_reverse_step: tcgen05 path does not support S=%d mode=%d branch=%d (or tc_tables/workspace missing)", p->S, p->mode, p->branch); return 3; }
-    return launch_step_tc(p, st);
+    // Euler modes need a row's total rate before its one pick: the row-gather kernel; every other mode: chunk-local
+    if (p->mode == CTDD_MODE_EULER || p->mode == CTDD_MODE_EULER_CORR) return launch_step_tc(p, st);
+    return launch_step_tcq(p, st);
   }
   if (p->head != CTDD_HEAD_LOGITS) {
     set_error("ctdd_reverse_step: the fused logistic head exists on the tcgen05 path only (S == 256, tc tables given); "

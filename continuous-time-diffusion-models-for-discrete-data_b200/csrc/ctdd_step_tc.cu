@@ -1,7 +1,8 @@
-// tcgen05 reverse-step kernel for S == 256 (configs C3/C4/C5): the (N*D x S)(S x S) contraction of
-// lib/sampling/sampling.py:57 on 5th-generation tensor cores, fused with softmax, the q_{t|0} denominators, the
-// forward-rate multiply and the Philox state update of every sampler (tau-leap / corrector sampling.py:127-221,
-// midpoint :423-503, Euler :278-341, rates only :31-78).
+// tcgen05 reverse-step kernel for S == 256, Euler modes (lib/sampling/sampling.py:278-341, with and without the
+// corrector rates): the (N*D x S)(S x S) contraction of sampling.py:57 on 5th-generation tensor cores, fused with softmax,
+// the q_{t|0} denominators, the forward-rate multiply and one categorical draw per row over
+// {h * rate_s (s != x), max(0, 1 - h * sum)}.  That draw needs the row's total rate before its pick, so each row is
+// sampled with all 256 states in one place; every other mode runs on step_q_kernel (ctdd_step_tcq.cu).
 //
 // One CTA PAIR (thread-block cluster of 2, tcgen05 cta_group::2) owns a sequence of 64-row tiles:
 //   D[s, row] = sum_k Q^T[s, k] * a[row, k]        M = 256 states (128 per CTA), N = 64 rows, K = 256
@@ -10,20 +11,19 @@
 //   * N side = data rows. Each CTA's 8 producer warps build 32 of the tile's 64 rows, two rows per pass with 16 lanes
 //     per row: raw fp32 logits arrive through a per-warp smem ring filled by cp.async.bulk (HBM -> L2 prefetch eight
 //     tiles ahead), row softmax by half-warp butterflies, gathered reciprocal denominators 1/(Q[k,x]+eps), bf16 hi/mid
-//     split, K-major 128B-swizzled smem stage.  Every row is produced exactly once.  The producer also computes the
-//     row's TOTAL jump rate as one table dot product (Lambda = c * sum_k e_k G[x][k], G = (Q Rbz)[k,x] / (Q[k,x]+eps)).
-//   * Count warp (lane = row): total jump count K ~ Poisson(Lambda) and the uniforms of the first 11 picks.
+//     split, K-major 128B-swizzled smem stage.  Every row is produced exactly once.
+//   * Count warp (lane = row): the row's Euler uniform (Philox, STREAM_ROW).
 //   * 3 tensor passes  Qh*ah + Qh*am + Qm*ah  accumulate in fp32 TMEM (48 tcgen05.mma per tile).
 //   * Epilogue phase A: each CTA reads its 128 states x 64 rows with tcgen05.ld and scatters them (local st.shared /
 //     remote st.async with mbarrier complete_tx) into the [row][state] gather buffer of the CTA that OWNS the row, so
 //     that each owner sees all 256 states of its 32 rows.  Two gather buffers: phase A of tile i+1 runs before the
 //     sampling of tile i.
 //   * Row sampler (the same 8 warps, one warp per row, two rows in flight): lam_s = D_s * c * Rbz[s,x], warp prefix
-//     sum, K inverse-CDF picks (superposition map of ctdd_common.cuh), clamp, rejection, statistics, x_out.  Rows with
-//     K == 0 are settled by one lane.  The side record and the R_b table rows (L2 gathers) of the NEXT row pair are requested
-//     while the current pair is searched; the first pair's before phase A of the next tile, which hides their latency.
-//   * Producers finish the row reductions (sum e, sum e*G) and the side record of a pass in the head of the NEXT pass, next
-//     to its row-maximum butterfly; only the operand rows are completed inside the pass.
+//     sum, the stay probability added at x, one inverse-CDF pick per row, statistics, x_out.  The side record and the
+//     R_b table rows (L2 gathers) of the NEXT row pair are requested while the current pair is searched; the first
+//     pair's before phase A of the next tile, which hides their latency.
+//   * Producers finish the row reductions (sum e, and sum e*Q[.,x] for SDDM) and the side record of a pass in the head of
+//     the NEXT pass, next to its row-maximum butterfly; only the operand rows are completed inside the pass.
 //   * The MMA-issue thread acquires the partner CTA's release-arrive with ONE mbarrier.test_wait.acquire.cluster on the
 //     already flipped barrier; a stand-alone fence.acq_rel.cluster there cost 0.2 ms per launch.
 // Warp roles per CTA (5 warpgroups, setmaxnreg 104 / 64): 8 epilogue/sampler warps, 8 producer warps, and a light
@@ -44,7 +44,7 @@ constexpr int NUM_EPI_WARPS = 8;       // warps 0-7: TMEM quadrant w&3, column h
 constexpr int FIRST_PROD_WARP = 8;     // warps 8-15
 constexpr int NUM_PROD_WARPS = 8;
 constexpr int MMA_WARP = 16;           // warps 16-19 form the light warpgroup: MMA issue / relay, count warp, 2 idle
-constexpr int COUNT_WARP = 17;         // draws the jump counts of a tile, lane = row
+constexpr int COUNT_WARP = 17;         // draws the Euler uniforms of a tile, lane = row
 constexpr int NUM_THREADS = 20 * 32;   // 640: register allocation is per 4-warp group, so 18 warps cost the same
 // setmaxnreg targets: samplers + producers / the light warpgroup.  The registers handed out by .inc are the ones the
 // CTA's own warps released with .dec: 16 * HEAVY + 4 * LIGHT must not exceed 20 * 96 (the launch allocation), or
@@ -61,11 +61,8 @@ constexpr int PREFETCH_TILES = 8;      // HBM -> L2 bulk-prefetch distance (tile
 constexpr int LRING = 2;               // per-producer-warp ring of raw logits row pairs filled by cp.async.bulk
 constexpr uint32_t IDESC = make_idesc(NT);
 
-// per-row hand-over producer -> count warp -> sampler: rate scale, state, jump count K and the uniforms of picks 0..10
-// (pick uniforms beyond that are regenerated by the sampler; rare)
-constexpr int SIDE_PICKS = 11;
-struct __align__(16) Side { float c1, c0; int x; int K; uint32_t w[SIDE_PICKS]; int valid; };
-struct __align__(16) SideHead { float c1, c0; int x; int K; };
+// per-row hand-over producer -> count warp -> sampler: rate scale, state (x < 0: row past the end), Euler uniform
+struct __align__(16) Side { float c1, c0; int x; uint32_t w; };
 
 struct Smem {
   alignas(1024) uint8_t stage[STAGES][STAGE_BYTES];
@@ -76,7 +73,7 @@ struct Smem {
   uint64_t full_local[STAGES];       // partner CTA: its 8 producer warps; the partner's idle MMA warp relays the phase
   uint64_t empty[STAGES];            // multicast tcgen05.commit
   uint64_t pre_full[RING];           // local producers -> count warp (row scalars written)
-  uint64_t side_full[RING];          // count warp -> local samplers (jump counts and pick uniforms written)
+  uint64_t side_full[RING];          // count warp -> local samplers (Euler uniforms written)
   uint64_t lring_full[NUM_PROD_WARPS][LRING];   // cp.async.bulk complete_tx of one row pair
   uint64_t tmem_full[ACC];           // multicast tcgen05.commit
   uint64_t tmem_empty[ACC];          // used in the leader CTA: 8 local + 8 remote epilogue warps
@@ -89,60 +86,30 @@ struct Smem {
 static_assert(sizeof(Smem) + 1024 <= 232448, "shared memory budget of one CTA (227 KB) exceeded");
 
 
-// First index whose inclusive prefix sum (256 floats at shared address P) exceeds T, for NB independent (P, T) pairs per
-// lane: three rounds of INDEPENDENT loads (7 splitters of stride 32, 7 of stride 4, 3 neighbours) instead of eight
-// dependent binary-search steps; the rounds of the NB searches are interleaved.
-template <int NB>
-__device__ __forceinline__ void prefix_search(const uint32_t (&P)[NB], const float (&T)[NB], int (&lo)[NB]) {
-#ifdef CTDD_EXP_NOSEARCH    // diagnostic build: no search
+// First index whose inclusive prefix sum (256 floats at shared address P) exceeds T: three rounds of INDEPENDENT loads
+// (7 splitters of stride 32, 7 of stride 4, 3 neighbours) instead of eight dependent binary-search steps.
+__device__ __forceinline__ int prefix_search(uint32_t P, float T) {
+  int c1 = 0;
 #pragma unroll
-  for (int b = 0; b < NB; ++b) lo[b] = (T[b] > 1e30f) ? 1 : 0;
-#else
-  int c1[NB], c2[NB];
-  uint32_t P1[NB], P2[NB];
+  for (int m = 0; m < 7; ++m) c1 += (lds32(P + 4 * (32 * m + 31)) <= T) ? 1 : 0;
+  const uint32_t P1 = P + 128 * c1;
+  int c2 = 0;
 #pragma unroll
-  for (int b = 0; b < NB; ++b) {
-    c1[b] = 0;
-#pragma unroll
-    for (int m = 0; m < 7; ++m) c1[b] += (lds32(P[b] + 4 * (32 * m + 31)) <= T[b]) ? 1 : 0;
-    P1[b] = P[b] + 128 * c1[b];
-  }
-#pragma unroll
-  for (int b = 0; b < NB; ++b) {
-    c2[b] = 0;
-#pragma unroll
-    for (int n = 0; n < 7; ++n) c2[b] += (lds32(P1[b] + 4 * (4 * n + 3)) <= T[b]) ? 1 : 0;
-    P2[b] = P1[b] + 16 * c2[b];
-  }
-#pragma unroll
-  for (int b = 0; b < NB; ++b) {
-    const int c3 = ((lds32(P2[b]) <= T[b]) ? 1 : 0) + ((lds32(P2[b] + 4) <= T[b]) ? 1 : 0) + ((lds32(P2[b] + 8) <= T[b]) ? 1 : 0);
-    lo[b] = 32 * c1[b] + 4 * c2[b] + c3;
-  }
-#endif
+  for (int n = 0; n < 7; ++n) c2 += (lds32(P1 + 4 * (4 * n + 3)) <= T) ? 1 : 0;
+  const uint32_t P2 = P1 + 16 * c2;
+  const int c3 = ((lds32(P2) <= T) ? 1 : 0) + ((lds32(P2 + 4) <= T) ? 1 : 0) + ((lds32(P2 + 8) <= T) ? 1 : 0);
+  return 32 * c1 + 4 * c2 + c3;
 }
 
 // ---------------------------------------------------------------------------------------------- the kernel
-#ifdef CTDD_TC_TRACE
-// diagnostic build only (CTDD_TRACE=1 python build.py): per-tile clock stamps of one CTA's roles, read back with
-// ctdd_debug_trace_read; never compiled into the product library
-constexpr int TRACE_TILES = 1024, TRACE_EVENTS = 8, TRACE_ROLES = 4;
-__device__ long long g_trace[2][TRACE_ROLES][TRACE_TILES][TRACE_EVENTS];
-#define TRACE(role, tile, ev)                                                                       \
-  do {                                                                                              \
-    if (blockIdx.x < 2 && (tile) < TRACE_TILES) g_trace[blockIdx.x][role][tile][ev] = clock64();    \
-  } while (0)
-#else
-#define TRACE(role, tile, ev) do { } while (0)
-#endif
-
-
-// TAULDR: tauLDR rates (else SDDM reverse_prob); KM: KM_JUMP / KM_CORR / KM_RATES / KM_DRIFT / KM_EULER / KM_EULER_CORR;
+// TAULDR: tauLDR rates (else SDDM reverse_prob); CORR: the corrector variant adds h * R_t[x,:] to the rates;
 // HEAD: the rows' softmax numerators come from the truncated-logistic head (mu, log_scale per row) instead of logits
-template <bool TAULDR, int KM, bool HEAD>
+template <bool TAULDR, bool CORR, bool HEAD>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step_tc_kernel(const Args a) {
   extern __shared__ uint8_t smem_raw[];
-  Smem& sm = *reinterpret_cast<Smem*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
+  // aligned by offsetting the shared array itself (not through an integer): the compiler keeps `sm` a shared-space
+  // pointer, so its accesses are 32-bit LDS/STS and no 64-bit generic base stays live (that base was spilled at 96 registers)
+  Smem& sm = *reinterpret_cast<Smem*>(smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u));
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t rank = cluster_ctarank();       // state half owned by this CTA; rank 0 issues the MMAs
   const int pair = blockIdx.x >> 1;
@@ -205,9 +172,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
     // (two independent rows per warp keep the pipes busy).  The raw logits rows arrive through a small smem ring that
     // cp.async.bulk fills two passes ahead, so no global-memory latency sits on the warp's critical path.
     const float* tabA = reinterpret_cast<const float*>(a.tab + TAB_A_OFF) + 4 * l16;
-    const float* tabG = reinterpret_cast<const float*>(a.tab + TAB_G_OFF) + 4 * l16;
-    const float* rowsumZ = reinterpret_cast<const float*>(a.stat + ST_ROWSUM_OFF);
-    const float hb = (KM == KM_RATES) ? 1.0f : a.h * a.beta;   // rates-only ignores the step length
+    const float hb = a.h * a.beta;
     const bool contiguous = (a.ld == S) && (a.batch_stride == (long long)a.D * S);
     uint64_t* const full_bar = rank == 0 ? &sm.full[0] : &sm.full_local[0];
     constexpr int PASSES = ROWS_PER_PROD / 2;                    // passes per tile; warp pw builds rows ROWS_PER_PROD*pw ..
@@ -270,29 +235,22 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
     float mu_cur = f_mu, ls_cur = f_ls;
     int x_n1 = fetch();
     float mu_n1 = f_mu, ls_n1 = f_ls;
-    float4 t4[4], g4[4];
+    float4 t4[4];
     {
       const size_t xo = (size_t)(x_cur < 0 ? 0 : x_cur) << 8;
 #pragma unroll
-      for (int c = 0; c < 4; ++c) {
-        t4[c] = __ldg(reinterpret_cast<const float4*>(tabA + xo + 64 * c));
-        g4[c] = __ldg(reinterpret_cast<const float4*>(tabG + xo + 64 * c));
-      }
+      for (int c = 0; c < 4; ++c) t4[c] = __ldg(reinterpret_cast<const float4*>(tabA + xo + 64 * c));
     }
-    // The row reductions (sum e, sum e*G, sum e*a) and the row scalars of a pass are FINISHED IN THE NEXT PASS: its
-    // per-lane partial sums are carried over, their butterflies run next to the next pass's row-maximum butterfly (three
-    // independent shuffle chains instead of one after the other), and the side record / pre_full arrival follow there.
+    // The row reductions (sum e, sum e*a) and the row scalars of a pass are FINISHED IN THE NEXT PASS: its per-lane
+    // partial sums are carried over, their butterflies run next to the next pass's row-maximum butterfly (independent
+    // shuffle chains instead of one after the other), and the side record / pre_full arrival follow there.
     // Only the operand rows (what the MMA waits for) are completed inside the pass itself.
-    float p_sum = 1.f, p_dotg = 0.f, p_dot = 0.f;
+    float p_sum = 1.f, p_dot = 0.f;
     int p_x = 0, p_r = 0, p_slot = 0;
-    bool p_ok = false, p_have = false, p_close = false;
-    auto finish_prev = [&]() {          // p_sum / p_dotg / p_dot hold the reduced values
+    bool p_have = false, p_close = false;
+    auto finish_prev = [&]() {          // p_sum / p_dot hold the reduced values
       if (!p_have) return;
-#ifdef CTDD_EXP_NOPRODUCE
-      const float c1 = 1e-6f, c0 = 0.f, lam_tot = CTDD_EXP_NOPRODUCE;
-#else
       const float rs = __frcp_rn(p_sum);
-      const float rz = (!TAULDR || km_corr(KM)) ? __ldg(rowsumZ + p_x) : 0.f;
       float c1, c0;
       if (TAULDR) {
         c1 = hb * rs;                                            // lam_s = D_s * c1 * Rb[s,x]
@@ -302,16 +260,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
         c1 = hb * rs * inv;                                      // lam_s = (D_s * c1 + c0) * Rb[x,s]
         c0 = hb * 1e-35f * inv;
       }
-      float lam_tot = fmaf(c1, p_dotg, c0 * rz);
-      if (km_corr(KM)) lam_tot = fmaf(hb, rz, lam_tot);
-#endif
-      // row scalars for the count warp and the samplers (one lane per half-warp)
-      if (l16 == 0) {
-        Side si;
-        si.c1 = c1; si.c0 = c0; si.x = p_x; si.valid = p_ok ? 1 : 0;
-        si.K = 0; si.w[0] = __float_as_uint(lam_tot);
-        sm.side[p_slot][p_r] = si;
-      }
+      // row scalars for the count warp and the samplers (one lane per half-warp); the count warp adds the uniform
+      if (l16 == 0) sm.side[p_slot][p_r] = Side{c1, c0, p_x, 0u};
       if (p_close) {                    // that pass closed its tile: the tile's row scalars are complete now
         __syncwarp();
         if (lane == 0) mbar_arrive(&sm.pre_full[p_slot]);
@@ -319,33 +269,21 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
       p_have = false;
     };
     // running state of the compute stream
-    int i = 0, ps = 0, st = 0, slot = 0, rslot = 0;
+    int ps = 0, st = 0, slot = 0, rslot = 0;
     uint32_t st_par = 1, ring_par = 0;      // parity to wait for on empty[st] / lring_full[rslot]
 #pragma unroll 1
     for (int pi = 0; pi < npass; ++pi) {
       const bool ok = x_cur >= 0;
-      const int x = ok ? x_cur : 0;
-      if (ps == 0) {
-        if (pw == 0 && lane == 0) TRACE(0, i, 0);
-        mbar_wait(&sm.empty[st], st_par);
-        if (pw == 0 && lane == 0) TRACE(0, i, 1);
-      }
+      if (ps == 0) mbar_wait(&sm.empty[st], st_par);
       const uint32_t stage_s = smem_u32(sm.stage[st]);
       if (!HEAD) mbar_wait(&sm.lring_full[pw][rslot], ring_par);
-      if (pw == 0 && lane == 0) TRACE(0, i, 5 + (ps & 1));
       const int r = ROWS_PER_PROD * pw + 2 * ps + half;
-#ifdef CTDD_EXP_NOPRODUCE   // diagnostic build: producers only run the barrier protocol (isolates MMA + phase A + samplers)
-      (void)stage_s;
-      finish_prev();
-      const float sum = 1.f, dotg = 0.f, dot = 0.f;
-#else
       float v[16];
       float ml = 0.f;
       if (HEAD) {
 #pragma unroll
         for (int o = 8; o > 0; o >>= 1) {     // previous pass's reductions: independent of the head arithmetic below
           p_sum += __shfl_xor_sync(0xffffffffu, p_sum, o);
-          p_dotg += __shfl_xor_sync(0xffffffffu, p_dotg, o);
           if (!TAULDR) p_dot += __shfl_xor_sync(0xffffffffu, p_dot, o);
         }
         head_numerators(mu_cur, ls_cur, a.head_fix != 0, l16, v);
@@ -361,54 +299,46 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
         for (int c = 0; c < 4; ++c) m4[c] = fmaxf(fmaxf(v[4 * c], v[4 * c + 1]), fmaxf(v[4 * c + 2], v[4 * c + 3]));
         float m = fmaxf(fmaxf(m4[0], m4[1]), fmaxf(m4[2], m4[3]));
 #pragma unroll
-        for (int o = 8; o > 0; o >>= 1) {     // this pass's row maximum next to the previous pass's three reductions
+        for (int o = 8; o > 0; o >>= 1) {     // this pass's row maximum next to the previous pass's reductions
           m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
           p_sum += __shfl_xor_sync(0xffffffffu, p_sum, o);
-          p_dotg += __shfl_xor_sync(0xffffffffu, p_dotg, o);
           if (!TAULDR) p_dot += __shfl_xor_sync(0xffffffffu, p_dot, o);
         }
         ml = -m * 1.4426950408889634f;
       }
       finish_prev();
       // four independent accumulation chains of packed pairs
-      float2 sum2[4], dot2[4], dotg2[4];
+      float2 sum2[4], dot2[4];
       const float2 l2e2 = make_float2(1.4426950408889634f, 1.4426950408889634f), ml2 = make_float2(ml, ml);
 #pragma unroll
       for (int c = 0; c < 4; ++c) {
-        sum2[c] = make_float2(0.f, 0.f); dot2[c] = make_float2(0.f, 0.f); dotg2[c] = make_float2(0.f, 0.f);
+        sum2[c] = make_float2(0.f, 0.f); dot2[c] = make_float2(0.f, 0.f);
 #pragma unroll
         for (int e = 0; e < 4; e += 2) {
           const float2 tq = e == 0 ? make_float2(t4[c].x, t4[c].y) : make_float2(t4[c].z, t4[c].w);
-          const float2 gq = e == 0 ? make_float2(g4[c].x, g4[c].y) : make_float2(g4[c].z, g4[c].w);
           float2 ex = make_float2(v[4 * c + e], v[4 * c + e + 1]);                 // HEAD: already the numerators
           if (!HEAD) {
             const float2 arg = ffma2(ex, l2e2, ml2);
             ex = make_float2(ex2_approx(arg.x), ex2_approx(arg.y));                // exp(v - max)
           }
           sum2[c] = fadd2(sum2[c], ex);
-          dotg2[c] = ffma2(ex, gq, dotg2[c]);
           if (!TAULDR) dot2[c] = ffma2(ex, tq, dot2[c]);
           const float2 op = TAULDR ? fmul2(ex, tq) : ex;   // tauLDR operand: e_k / (Q[k,x] + eps); 1/sum applied by the sampler
           v[4 * c + e] = op.x; v[4 * c + e + 1] = op.y;
         }
       }
       const float2 s01 = fadd2(sum2[0], sum2[1]), s23 = fadd2(sum2[2], sum2[3]), sall = fadd2(s01, s23);
-      const float2 g01 = fadd2(dotg2[0], dotg2[1]), g23 = fadd2(dotg2[2], dotg2[3]), gall = fadd2(g01, g23);
       float sum = sall.x + sall.y;
-      float dotg = gall.x + gall.y;
       float dot = 0.f;
       if (!TAULDR) {
         const float2 d01 = fadd2(dot2[0], dot2[1]), d23 = fadd2(dot2[2], dot2[3]), dall = fadd2(d01, d23);
         dot = dall.x + dall.y;
       }
-      // the tables of the NEXT pass are requested as soon as this pass's have been consumed
+      // the table row of the NEXT pass is requested as soon as this pass's has been consumed
       {
         const size_t xo = (size_t)(x_n1 < 0 ? 0 : x_n1) << 8;
 #pragma unroll
-        for (int c = 0; c < 4; ++c) {
-          t4[c] = __ldg(reinterpret_cast<const float4*>(tabA + xo + 64 * c));
-          g4[c] = __ldg(reinterpret_cast<const float4*>(tabG + xo + 64 * c));
-        }
+        for (int c = 0; c < 4; ++c) t4[c] = __ldg(reinterpret_cast<const float4*>(tabA + xo + 64 * c));
       }
       // k = 64c + 4*l16 .. +3 lives in K block c, 16-byte chunk l16/2 (XOR-swizzled by the row), half l16&1
       const uint32_t off = (uint32_t)r * 128 + (uint32_t)((((l16 >> 1) ^ (r & 7)) << 4) | ((l16 & 1) << 3));
@@ -421,24 +351,20 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
         sts64(stage_s + c * KBLOCK_BYTES + off, h0, h1);
         sts64(stage_s + SPLIT_BYTES + c * KBLOCK_BYTES + off, m0, m1);
       }
-#endif
       // this pass's partial sums and row identity travel to the next pass (finish_prev)
-      p_sum = sum; p_dotg = dotg; p_dot = dot;
-      p_x = x; p_ok = ok; p_r = r; p_slot = slot; p_close = (ps + 1 == PASSES); p_have = true;
+      p_sum = sum; p_dot = dot;
+      p_x = x_cur; p_r = r; p_slot = slot; p_close = (ps + 1 == PASSES); p_have = true;
       if (++rslot == LRING) { rslot = 0; ring_par ^= 1u; }
       __syncwarp();            // every lane is done with this pass's ring slot: refill it for the pass after next
       x_cur = x_n1;
       if (HEAD) { mu_cur = mu_n1; ls_cur = ls_n1; }
       x_n1 = fetch();
       if (HEAD) { mu_n1 = f_mu; ls_n1 = f_ls; }
-      if (pw == 0 && lane == 0) TRACE(0, i, 2 + (ps & 1));
       if (++ps == PASSES) {     // last pass of the tile
         fence_proxy_async();
         __syncwarp();
         if (lane == 0) mbar_arrive(full_bar + st);   // operand rows are in place (the row scalars follow in finish_prev)
-        if (pw == 0 && lane == 0) TRACE(0, i, 4);
         ps = 0;
-        ++i;
         slot = (slot + 1) & (RING - 1);
         if (++st == STAGES) { st = 0; st_par ^= 1u; }
       }
@@ -447,7 +373,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
 #pragma unroll
     for (int o = 8; o > 0; o >>= 1) {
       p_sum += __shfl_xor_sync(0xffffffffu, p_sum, o);
-      p_dotg += __shfl_xor_sync(0xffffffffu, p_dotg, o);
       if (!TAULDR) p_dot += __shfl_xor_sync(0xffffffffu, p_dot, o);
     }
     finish_prev();
@@ -456,41 +381,13 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
   } else if (warp == COUNT_WARP) {
     asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(REGS_LIGHT));
     // ======================================================================== count warp: lane = row of the tile
-    // total jump count K ~ Poisson(Lambda) and the first pick uniforms of every row (superposition map, ctdd_common.cuh)
+    // one categorical draw per valid row: its uniform from the per-row Euler stream
     for (int i = 0; i < my_tiles; ++i) {
       const int tile = pair + i * npairs, slot = i % RING;
       const long long g0 = (long long)tile * NT + (long long)rank * NH;
       mbar_wait(&sm.pre_full[slot], (i / RING) & 1);
-      Side si = sm.side[slot][lane];
-      const float lam = __uint_as_float(si.w[0]);
-      si.w[0] = 0u;
-      if (si.valid) {
-        if (KM == KM_RATES || KM == KM_DRIFT) {
-          si.K = 1;
-        } else if (km_euler(KM)) {   // one categorical draw per row: the per-row uniform of the Euler stream
-          si.K = 1;
-          si.w[0] = philox_row_word((uint64_t)(a.row_offset + g0 + lane), 0, a.offset, STREAM_ROW, a.seed);
-        } else {
-          const Philox4 p0 = philox_rowjump((uint64_t)(a.row_offset + g0 + lane), 0, a.offset, a.seed);
-#ifdef CTDD_EXP_NOSAMPLE   // diagnostic build: no row ever jumps (isolates producer + MMA + phase A)
-          const int K = 0;
-          (void)lam;
-#else
-          const int K = poisson_from_unit(lam, u32_to_unit(p0.w[0]));
-#endif
-          si.K = K > JUMP_PICK_CAP ? JUMP_PICK_CAP : K;
-          si.w[0] = p0.w[1]; si.w[1] = p0.w[2]; si.w[2] = p0.w[3];
-          // picks 3..10: a call here serves a whole tile of rows (lane = row); in the sampler it would cost a warp per row
-#pragma unroll
-          for (int c = 1; c <= (SIDE_PICKS - 3) / 4; ++c) {
-            if (K > 4 * c - 1) {
-              const Philox4 pc = philox_rowjump((uint64_t)(a.row_offset + g0 + lane), (uint32_t)c, a.offset, a.seed);
-              si.w[4 * c - 1] = pc.w[0]; si.w[4 * c] = pc.w[1]; si.w[4 * c + 1] = pc.w[2]; si.w[4 * c + 2] = pc.w[3];
-            }
-          }
-        }
-      }
-      sm.side[slot][lane] = si;
+      if (sm.side[slot][lane].x >= 0)
+        sm.side[slot][lane].w = philox_row_word((uint64_t)(a.row_offset + g0 + lane), 0, a.offset, STREAM_ROW, a.seed);
       __syncwarp();
       if (lane == 0) mbar_arrive(&sm.side_full[slot]);
     }
@@ -500,21 +397,15 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
     if (rank == 0 && lane == 0) {
       for (int i = 0; i < my_tiles; ++i) {
         const int st = i % STAGES, b = i % ACC;
-        TRACE(1, i, 0);
         mbar_wait_cluster(&sm.full[st], (i / STAGES) & 1);
-        TRACE(1, i, 1);
         mbar_wait(&sm.tmem_empty[b], ((i / ACC) & 1) ^ 1);
-        TRACE(1, i, 2);
         tc_fence_after();
         const uint32_t d_tmem = tmem + TM_ACC + b * NT;
         // one descriptor per tile; the 48 instructions differ only by compile-time offsets (16-byte units, low word)
         const uint64_t bd0 = make_b_desc(smem_u32(sm.stage[st]));
         const uint32_t bd_lo = (uint32_t)bd0, bd_hi = (uint32_t)(bd0 >> 32);
 #pragma unroll 1
-#ifndef CTDD_EXP_PASSES
-#define CTDD_EXP_PASSES 3     // diagnostic builds issue fewer tensor passes (wrong numerics, timing only)
-#endif
-        for (int pass = 0; pass < CTDD_EXP_PASSES; ++pass) {
+        for (int pass = 0; pass < 3; ++pass) {
           const uint32_t a_tmem = tmem + (pass == 2 ? TM_QM : TM_QH);
           const uint32_t lo = bd_lo + (pass == 1 ? (uint32_t)(SPLIT_BYTES >> 4) : 0u);
 #pragma unroll
@@ -525,7 +416,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
         }
         umma_commit_pair(&sm.empty[st]);
         umma_commit_pair(&sm.tmem_full[b]);
-        TRACE(1, i, 3);
       }
     } else if (rank != 0 && lane == 0) {
       // partner CTA: relay "my 8 producer warps have filled stage st" to the leader as ONE cluster-scope arrival
@@ -551,19 +441,14 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
     uint64_t* const gfree_wait = (owner == rank) ? &sm.gather_free_local[0] : &sm.gather_free_remote[0];
     const float* tabE = reinterpret_cast<const float*>(a.stat + (TAULDR ? ST_RBZT_OFF : ST_RBZ_OFF)) + 8 * lane;
     const float* tabC = reinterpret_cast<const float*>(a.stat + ST_RBZ_OFF) + 8 * lane;   // corrector add: Rb[x][s], zero diag
-    const float* tabFull = (TAULDR ? a.RbT : a.Rb) + 8 * lane;                             // diagonal kept, for rr_out
     const float hb = a.h * a.beta;
     RowStats stt = {0, 0, 0, 0, 0};
 
     // phase A of tile i: accumulator (this CTA's 128 states x this warp's 32 rows) -> gather buffer of the rows' owner
     auto phase_a = [&](int i) {
       const int b = i % ACC, gb = i % GBUF;
-      const int trole = 2 + (warp >> 2);
-      if ((warp & 3) == 0 && lane == 0) TRACE(trole, i, 0);
       mbar_wait(&sm.tmem_full[b], (i / ACC) & 1);
-      if ((warp & 3) == 0 && lane == 0) TRACE(trole, i, 1);
       mbar_wait(gfree_wait + gb, ((i / GBUF) & 1) ^ 1);
-      if ((warp & 3) == 0 && lane == 0) TRACE(trole, i, 2);
       tc_fence_after();
       uint32_t acc[32];
       tmem_ld32(tmem + ((uint32_t)(q * 32) << 16) + TM_ACC + b * NT + owner * NH, acc);
@@ -581,7 +466,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
       }
       tc_fence_before();   // accumulator has been read: hand the buffer back to the MMA warp
       __syncwarp();
-      if ((warp & 3) == 0 && lane == 0) TRACE(trole, i, 3);
       if (lane == 0) {
         mbar_arrive_cluster_relaxed(tempty_dst + (uint32_t)b * 8u);
         if (owner == rank) {
@@ -590,7 +474,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
           else mbar_arrive(&sm.gather_full[gb]);
         }
       }
-      if ((warp & 3) == 0 && lane == 0) TRACE(trole, i, 4);
     };
 
     if (my_tiles > 0) phase_a(0);
@@ -598,34 +481,16 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
       // ---- phase B: sample the rows this CTA owns (warp w: rows 4w .. 4w+3 of the CTA's 32)
       const int tile = pair + i * npairs;
       const int slot = i % RING, gb = i % GBUF;
-      if ((warp & 3) == 0 && lane == 0) TRACE(2 + (warp >> 2), i, 5);
       mbar_wait(&sm.side_full[slot], (i / RING) & 1);
       const long long g0 = (long long)tile * NT + (long long)rank * NH;
-      // lanes 0..3 settle the rows without a jump in one go; the rest are processed two rows per iteration
-      uint32_t todo;
-      {
-        bool need = false;
-        if (lane < ROWS_PER_SAMPLER) {
-          const int r = warp * ROWS_PER_SAMPLER + lane;
-          const Side sj = sm.side[slot][r];
-          if (sj.valid) {
-            if (KM != KM_RATES && KM != KM_DRIFT && sj.K == 0) {
-              const long long g = g0 + r;
-              const int xb = a.x_base ? a.x_base[g] : sj.x;
-              a.x_out[g] = finalize_jump(xb, sj.x, 0, 0, a.reject_multi, S, stt);
-            } else {
-              need = true;
-            }
-          }
-        }
-        todo = __ballot_sync(0xffffffffu, need);
-      }
-      // Jump modes: the rows are processed two at a time, and the side record + rate-table rows (L2 gathers) of the NEXT
-      // pair are requested while the current pair is searched / finalized; the first pair's before the wait for the
-      // accumulator rows.  The table registers are dead between the rate computation and the next iteration.
+      // the warp's rows that exist, processed two per iteration
+      uint32_t todo = __ballot_sync(0xffffffffu, lane < ROWS_PER_SAMPLER && sm.side[slot][warp * ROWS_PER_SAMPLER + lane].x >= 0);
+      // The side record + rate-table rows (L2 gathers) of the NEXT pair are requested while the current pair is searched;
+      // the first pair's before the wait for the accumulator rows.  The table registers are dead between the rate
+      // computation and the next iteration.
       int rrow[2] = {0, 0};
       bool two = false;
-      SideHead si[2];
+      Side si[2];
       float4 e0[2], e1[2], c0v[2], c1v[2];
       auto load_pair = [&]() {
         rrow[0] = __ffs(todo) - 1;
@@ -634,202 +499,111 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
         rrow[1] = two ? __ffs(todo) - 1 : rrow[0];
         todo &= todo - 1;   // no-op when todo == 0
 #pragma unroll
-        for (int u = 0; u < 2; ++u)
-          si[u] = *reinterpret_cast<const SideHead*>(&sm.side[slot][warp * ROWS_PER_SAMPLER + rrow[u]]);
+        for (int u = 0; u < 2; ++u) si[u] = sm.side[slot][warp * ROWS_PER_SAMPLER + rrow[u]];
 #pragma unroll
         for (int u = 0; u < 2; ++u) {
           const size_t xo = (size_t)si[u].x << 8;
-#ifdef CTDD_EXP_NOTABE      // diagnostic build: no rate-table gather in the sampler
-          e0[u] = make_float4(1.f, 1.f, 1.f, 1.f); e1[u] = e0[u]; (void)xo;
-#else
           // lane owns states 4*lane .. +3 (elements 0-3) and 128 + 4*lane .. +3 (elements 4-7): every 128-bit access of
           // the warp to a gather row is then one contiguous 512-byte run (no bank conflicts)
           e0[u] = __ldg(reinterpret_cast<const float4*>(tabE - 4 * lane + xo));
           e1[u] = __ldg(reinterpret_cast<const float4*>(tabE - 4 * lane + xo + 128));
-#endif
-          if (km_corr(KM)) {
+          if (CORR) {
             c0v[u] = __ldg(reinterpret_cast<const float4*>(tabC - 4 * lane + xo));
             c1v[u] = __ldg(reinterpret_cast<const float4*>(tabC - 4 * lane + xo + 128));
           }
         }
       };
-      bool have = false;
-      if constexpr (!(KM == KM_RATES || KM == KM_DRIFT)) {
-        have = todo != 0;
-        if (have) load_pair();
-      }
+      bool have = todo != 0;
+      if (have) load_pair();
       // the next tile's accumulator is moved now: the cross-CTA hand-shakes of tile i and the L2 latency of the first
       // pair's table rows complete in its shadow
       if (i + 1 < my_tiles) phase_a(i + 1);
       mbar_wait(&sm.gather_full[gb], (i / GBUF) & 1);
-      if ((warp & 3) == 0 && lane == 0) TRACE(2 + (warp >> 2), i, 6);
-      if constexpr (KM == KM_RATES || KM == KM_DRIFT) {
+      // two rows in flight per iteration (independent dependency chains hide the shuffle / smem latency)
 #pragma unroll 1
-        while (todo) {
-          const int rr = __ffs(todo) - 1;
-          todo &= todo - 1;
-          const int r = warp * ROWS_PER_SAMPLER + rr;
-          const SideHead si = *reinterpret_cast<const SideHead*>(&sm.side[slot][r]);
-          const long long g = g0 + r;
-          const int x = si.x;
-          const uint32_t grow_p = smem_u32(&sm.gather[gb][r][0]);
-          const float4 d0 = lds128(grow_p + 32 * lane);
-          const float4 d1 = lds128(grow_p + 32 * lane + 16);
-          const float d[8] = {d0.x, d0.y, d0.z, d0.w, d1.x, d1.y, d1.z, d1.w};
-          const size_t xo = (size_t)x << 8;
-          if constexpr (KM == KM_RATES) {
-            const float4 f0 = __ldg(reinterpret_cast<const float4*>(tabFull + xo));
-            const float4 f1 = __ldg(reinterpret_cast<const float4*>(tabFull + xo + 4));
-            const float f[8] = {f0.x, f0.y, f0.z, f0.w, f1.x, f1.y, f1.z, f1.w};
-            float ratio[8], rfull[8];
+      while (have) {
+        // the current pair's identifiers survive the preload of the next pair
+        const int rc0 = rrow[0], rc1 = rrow[1];
+        const bool two_c = two;
+        const int xc0 = si[0].x, xc1 = si[1].x;
+        uint32_t gp[2];   // shared-space address of the row's gather slot
+        float d[2][8];
+        float total[2];
+        gp[0] = smem_u32(&sm.gather[gb][warp * ROWS_PER_SAMPLER + rc0][0]);
+        gp[1] = smem_u32(&sm.gather[gb][warp * ROWS_PER_SAMPLER + rc1][0]);
 #pragma unroll
-            for (int e = 0; e < 8; ++e) {
-              ratio[e] = fmaf(d[e], si.c1, si.c0);
-              rfull[e] = TAULDR ? a.beta * f[e] * ratio[e] : ratio[e] * (a.beta * f[e]);
-            }
-            if (a.rr_out) {
-              float4* o = reinterpret_cast<float4*>(a.rr_out + g * S + 8 * lane);
-              o[0] = make_float4(rfull[0], rfull[1], rfull[2], rfull[3]);
-              o[1] = make_float4(rfull[4], rfull[5], rfull[6], rfull[7]);
-            }
-            if (a.ratio_out) {
-              float4* o = reinterpret_cast<float4*>(a.ratio_out + g * S + 8 * lane);
-              o[0] = make_float4(ratio[0], ratio[1], ratio[2], ratio[3]);
-              o[1] = make_float4(ratio[4], ratio[5], ratio[6], ratio[7]);
-            }
-          } else {
-            // sampling.py:433-453: x' = clip(x + round_half_even(h/2 * sum_s rr_s (s - x)))
-            const float4 e0 = __ldg(reinterpret_cast<const float4*>(tabE + xo));
-            const float4 e1 = __ldg(reinterpret_cast<const float4*>(tabE + xo + 4));
-            const float ev[8] = {e0.x, e0.y, e0.z, e0.w, e1.x, e1.y, e1.z, e1.w};
-            float acc = 0.f;
+        for (int u = 0; u < 2; ++u) {
+          const float4 d0 = lds128(gp[u] + 16 * lane);
+          const float4 d1 = lds128(gp[u] + 512 + 16 * lane);
+          const float dv[8] = {d0.x, d0.y, d0.z, d0.w, d1.x, d1.y, d1.z, d1.w};
+          const float ev[8] = {e0[u].x, e0[u].y, e0[u].z, e0[u].w, e1[u].x, e1[u].y, e1[u].z, e1[u].w};
+          // lam_s (zero at s == x through the zero-diagonal tables)
 #pragma unroll
-            for (int e = 0; e < 8; ++e) acc = fmaf(fmaf(d[e], si.c1, si.c0) * ev[e], (float)(8 * lane + e - x), acc);
-            acc = warp_sum(acc);
-            if (lane == 0) {
-              const int ch = (int)rintf(0.5f * acc);
-              int xn = x + ch;
-              xn = xn < 0 ? 0 : (xn > S - 1 ? S - 1 : xn);
-              a.x_out[g] = xn;
-              stt.changed_base += (xn != x);
-              stt.changed_eval += (xn != x);
-              stt.nonzero += (ch != 0);
+          for (int e = 0; e < 8; ++e) d[u][e] = fmaf(dv[e], si[u].c1, si[u].c0) * ev[e];
+          if (CORR) {
+            const float cv[8] = {c0v[u].x, c0v[u].y, c0v[u].z, c0v[u].w, c1v[u].x, c1v[u].y, c1v[u].z, c1v[u].w};
+#pragma unroll
+            for (int e = 0; e < 8; ++e) d[u][e] = fmaf(hb, cv[e], d[u][e]);
+          }
+          // inclusive prefix sums over the 256 states: in-lane per 4-state group, then across lanes per half
+#pragma unroll
+          for (int e = 1; e < 4; ++e) { d[u][e] += d[u][e - 1]; d[u][4 + e] += d[u][3 + e]; }
+        }
+        float incl[2][2] = {{d[0][3], d[0][7]}, {d[1][3], d[1][7]}};   // [row][half]
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+#pragma unroll
+          for (int u = 0; u < 2; ++u)
+#pragma unroll
+            for (int hf = 0; hf < 2; ++hf) {
+              const float n = __shfl_up_sync(0xffffffffu, incl[u][hf], o);
+              if (lane >= o) incl[u][hf] += n;
             }
+        }
+        __syncwarp();
+#pragma unroll
+        for (int u = 0; u < 2; ++u) {
+          float excl_a = __shfl_up_sync(0xffffffffu, incl[u][0], 1);
+          float excl_b = __shfl_up_sync(0xffffffffu, incl[u][1], 1);
+          const float tot_a = __shfl_sync(0xffffffffu, incl[u][0], 31);
+          const float tot_b = __shfl_sync(0xffffffffu, incl[u][1], 31);
+          if (lane == 0) { excl_a = 0.f; excl_b = 0.f; }
+          excl_b += tot_a;
+          total[u] = tot_a + tot_b;
+#pragma unroll
+          for (int e = 0; e < 4; ++e) { d[u][e] += excl_a; d[u][4 + e] += excl_b; }
+          // stay-probability max(0, 1 - sum) enters the cumulative sums at position x
+          const float diag = fmaxf(0.f, 1.0f - total[u]);
+#pragma unroll
+          for (int e = 0; e < 4; ++e) {
+            d[u][e] += (4 * lane + e >= si[u].x) ? diag : 0.f;
+            d[u][4 + e] += (128 + 4 * lane + e >= si[u].x) ? diag : 0.f;
+          }
+          total[u] += diag;
+          if (u == 0 || two_c) {
+            sts128(gp[u] + 16 * lane, make_float4(d[u][0], d[u][1], d[u][2], d[u][3]));
+            sts128(gp[u] + 512 + 16 * lane, make_float4(d[u][4], d[u][5], d[u][6], d[u][7]));
           }
         }
-      } else {
-        // jump modes: two rows in flight per iteration (independent dependency chains hide the shuffle / smem latency)
-#pragma unroll 1
-        while (have) {
-          // the current pair's identifiers survive the preload of the next pair
-          const int rc0 = rrow[0], rc1 = rrow[1];
-          const bool two_c = two;
-          const int xc0 = si[0].x, xc1 = si[1].x;
-          const int K0 = si[0].K, K1 = two_c ? si[1].K : 0;
-          uint32_t gp[2];   // shared-space address of the row's gather slot
-          float d[2][8];
-          float total[2];
-          gp[0] = smem_u32(&sm.gather[gb][warp * ROWS_PER_SAMPLER + rc0][0]);
-          gp[1] = smem_u32(&sm.gather[gb][warp * ROWS_PER_SAMPLER + rc1][0]);
-#pragma unroll
-          for (int u = 0; u < 2; ++u) {
-            const float4 d0 = lds128(gp[u] + 16 * lane);
-            const float4 d1 = lds128(gp[u] + 512 + 16 * lane);
-            const float dv[8] = {d0.x, d0.y, d0.z, d0.w, d1.x, d1.y, d1.z, d1.w};
-            const float ev[8] = {e0[u].x, e0[u].y, e0[u].z, e0[u].w, e1[u].x, e1[u].y, e1[u].z, e1[u].w};
-            // lam_s (zero at s == x through the zero-diagonal tables)
-#pragma unroll
-            for (int e = 0; e < 8; ++e) d[u][e] = fmaf(dv[e], si[u].c1, si[u].c0) * ev[e];
-            if (km_corr(KM)) {
-              const float cv[8] = {c0v[u].x, c0v[u].y, c0v[u].z, c0v[u].w, c1v[u].x, c1v[u].y, c1v[u].z, c1v[u].w};
-#pragma unroll
-              for (int e = 0; e < 8; ++e) d[u][e] = fmaf(hb, cv[e], d[u][e]);
-            }
-            // inclusive prefix sums over the 256 states: in-lane per 4-state group, then across lanes per half
-#pragma unroll
-            for (int e = 1; e < 4; ++e) { d[u][e] += d[u][e - 1]; d[u][4 + e] += d[u][3 + e]; }
-          }
-          float incl[2][2] = {{d[0][3], d[0][7]}, {d[1][3], d[1][7]}};   // [row][half]
-#pragma unroll
-          for (int o = 1; o < 32; o <<= 1) {
-#pragma unroll
-            for (int u = 0; u < 2; ++u)
-#pragma unroll
-              for (int hf = 0; hf < 2; ++hf) {
-                const float n = __shfl_up_sync(0xffffffffu, incl[u][hf], o);
-                if (lane >= o) incl[u][hf] += n;
-              }
-          }
-          __syncwarp();
-#pragma unroll
-          for (int u = 0; u < 2; ++u) {
-            float excl_a = __shfl_up_sync(0xffffffffu, incl[u][0], 1);
-            float excl_b = __shfl_up_sync(0xffffffffu, incl[u][1], 1);
-            const float tot_a = __shfl_sync(0xffffffffu, incl[u][0], 31);
-            const float tot_b = __shfl_sync(0xffffffffu, incl[u][1], 31);
-            if (lane == 0) { excl_a = 0.f; excl_b = 0.f; }
-            excl_b += tot_a;
-            total[u] = tot_a + tot_b;
-#pragma unroll
-            for (int e = 0; e < 4; ++e) { d[u][e] += excl_a; d[u][4 + e] += excl_b; }
-            if (km_euler(KM)) {   // stay-probability max(0, 1 - sum) enters the cumulative sums at position x
-              const float diag = fmaxf(0.f, 1.0f - total[u]);
-#pragma unroll
-              for (int e = 0; e < 4; ++e) {
-                d[u][e] += (4 * lane + e >= si[u].x) ? diag : 0.f;
-                d[u][4 + e] += (128 + 4 * lane + e >= si[u].x) ? diag : 0.f;
-              }
-              total[u] += diag;
-            }
-            if (u == 0 || two_c) {
-              sts128(gp[u] + 16 * lane, make_float4(d[u][0], d[u][1], d[u][2], d[u][3]));
-              sts128(gp[u] + 512 + 16 * lane, make_float4(d[u][4], d[u][5], d[u][6], d[u][7]));
-            }
-          }
-          __syncwarp();
-          have = todo != 0;
-          if (have) load_pair();      // next pair: side record and table rows in flight during the search below
-          // K0 + K1 picks, one per lane (row 0's picks first): first state whose prefix sum exceeds v * total
-          const int Kt = K0 + K1;
-          int jump[2] = {0, 0};
-          for (int base = 0; base < Kt; base += 32) {
-            const int idx = base + lane;
-            const int u = idx >= K0 ? 1 : 0;          // row of this lane's pick
-            const int j = u ? idx - K0 : idx;         // pick number within the row
-            const bool active = idx < Kt;
-            const int rsel = warp * ROWS_PER_SAMPLER + (u ? rc1 : rc0);
-            uint32_t w = sm.side[slot][rsel].w[j < SIDE_PICKS ? j : 0];
-            if (active && j >= SIDE_PICKS) {          // more picks than the count warp prepared (large rates only)
-              const int jj = j - 3;
-              const Philox4 pc = philox_rowjump((uint64_t)(a.row_offset + g0 + rsel), 1u + (uint32_t)(jj >> 2), a.offset, a.seed);
-              w = philox_word(pc, jj & 3);
-            }
-            // lanes without a pick get a target below every prefix sum: they all walk the same (broadcast) addresses
-            // instead of scattering random shared-memory reads over the banks
-            const uint32_t P[1] = {u ? gp[1] : gp[0]};
-            const float T[1] = {active ? fminf(u32_to_unit(w), 0.99999994f) * (u ? total[1] : total[0]) : -1.0f};
-            int lo[1];
-            prefix_search<1>(P, T, lo);
-            const int dj = active ? lo[0] - (u ? xc1 : xc0) : 0;
-            jump[0] += u ? 0 : dj;
-            jump[1] += u ? dj : 0;
-          }
-          jump[0] = __reduce_add_sync(0xffffffffu, jump[0]);     // integer sums: one redux.sync each
-          jump[1] = __reduce_add_sync(0xffffffffu, jump[1]);
-          if (lane < 2 && (lane == 0 || two_c)) {
-            const int u = lane;
-            const long long g = g0 + warp * ROWS_PER_SAMPLER + (u ? rc1 : rc0);
-            const int x = u ? xc1 : xc0;
-            const int xb = a.x_base ? a.x_base[g] : x;
-            if (km_euler(KM)) {   // the pick IS the new state (jump holds pick - x)
-              const int xn = x + (u ? jump[1] : jump[0]);
-              a.x_out[g] = xn;
-              stt.changed_base += (xn != xb);
-              stt.changed_eval += (xn != x);
-            } else {
-              a.x_out[g] = finalize_jump(xb, x, u ? jump[1] : jump[0], u ? K1 : K0, a.reject_multi, S, stt);
-            }
-          }
+        __syncwarp();
+        have = todo != 0;
+        if (have) load_pair();      // next pair: side record and table rows in flight during the search below
+        // lane 0 picks for the first row, lane 1 for the second: the first state whose prefix sum exceeds v * total.
+        // The other lanes get a target below every prefix sum and walk the second row's (broadcast) addresses instead of
+        // scattering random shared-memory reads over the banks.
+        const int u = lane == 0 ? 0 : 1;
+        const bool active = lane == 0 || (lane == 1 && two_c);
+        const int r = warp * ROWS_PER_SAMPLER + (u ? rc1 : rc0);
+        const uint32_t w = sm.side[slot][r].w;
+        const float T = active ? fminf(u32_to_unit(w), 0.99999994f) * (u ? total[1] : total[0]) : -1.0f;
+        const int xn = prefix_search(u ? gp[1] : gp[0], T);   // the pick IS the new state
+        if (active) {
+          const long long g = g0 + r;
+          const int x = u ? xc1 : xc0;
+          const int xb = a.x_base ? a.x_base[g] : x;
+          a.x_out[g] = xn;
+          stt.changed_base += (xn != xb);
+          stt.changed_eval += (xn != x);
         }
       }
       __syncwarp();
@@ -837,7 +611,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
         mbar_arrive(&sm.gather_free_local[gb]);
         mbar_arrive_cluster_relaxed(gfree_remote_dst + (uint32_t)gb * 8u);
       }
-      if ((warp & 3) == 0 && lane == 0) TRACE(2 + (warp >> 2), i, 7);
     }
     if (a.stats) {
       const int v[5] = {stt.changed_base, stt.nonzero, stt.changed_eval, stt.jumped, stt.multi};
@@ -879,33 +652,9 @@ __global__ void prep_tables_kernel(const float* __restrict__ QT, int T, float ep
   }
 }
 
-// Total-rate table: sum_s lam_s of a row is one dot product of the row's exponentials with G[x][.]
-//   tauLDR: G[x][k] = (sum_s Rb[s][x] [s != x] Q[k][s]) / (Q[k][x] + eps)     (lam_s = c * Rb[s,x] * sum_k e_k Q[k,s] / (Q[k,x]+eps))
-//   SDDM  : G[x][k] =  sum_s Rb[x][s] [s != x] Q[k][s]                        (lam_s = (c1 * sum_k e_k Q[k,s] + c0) * Rb[x,s])
-__global__ void __launch_bounds__(256) prep_g_kernel(const float* __restrict__ QT, const float* __restrict__ Rb, float eps,
-                                                    int branch, uint8_t* __restrict__ out) {
-  __shared__ float sA[16][17], sB[16][17];
-  const int t = blockIdx.z, tx = threadIdx.x, ty = threadIdx.y;
-  const int x = blockIdx.y * 16 + ty, k = blockIdx.x * 16 + tx;
-  const float* qt = QT + (size_t)t * S * S;
-  float* G = reinterpret_cast<float*>(out + (size_t)t * TAB_BYTES + TAB_G_OFF);
-  float acc = 0.f;
-  for (int s0 = 0; s0 < S; s0 += 16) {
-    const int sa = s0 + tx, sb = s0 + ty;
-    sA[ty][tx] = (sa == x) ? 0.f : (branch == CTDD_BRANCH_TAULDR ? Rb[(size_t)sa * S + x] : Rb[(size_t)x * S + sa]);
-    sB[ty][tx] = qt[(size_t)sb * S + k];
-    __syncthreads();
-#pragma unroll
-    for (int m = 0; m < 16; ++m) acc = fmaf(sA[ty][m], sB[m][tx], acc);
-    __syncthreads();
-  }
-  G[(size_t)x * S + k] = (branch == CTDD_BRANCH_TAULDR) ? acc / (qt[(size_t)x * S + k] + eps) : acc;
-}
-
 __global__ void prep_static_kernel(const float* __restrict__ Rb, uint8_t* __restrict__ out) {
   float* rbzt = reinterpret_cast<float*>(out + ST_RBZT_OFF);
   float* rbz = reinterpret_cast<float*>(out + ST_RBZ_OFF);
-  float* rowsum = reinterpret_cast<float*>(out + ST_ROWSUM_OFF);
   float* rbt = reinterpret_cast<float*>(out + ST_RBT_OFF);
   float* rbf = reinterpret_cast<float*>(out + ST_RB_OFF);
   float* zero = reinterpret_cast<float*>(out + ST_ZERO_OFF);
@@ -921,16 +670,13 @@ __global__ void prep_static_kernel(const float* __restrict__ Rb, uint8_t* __rest
   int* bandT = reinterpret_cast<int*>(out + ST_BANDT_OFF);
   int* bandR = reinterpret_cast<int*>(out + ST_BANDR_OFF);
   for (int x = blockIdx.x * blockDim.x + threadIdx.x; x < S; x += gridDim.x * blockDim.x) {
-    float acc = 0.f;
     int loT = S - 1, hiT = 0, loR = S - 1, hiR = 0;   // exact zero pattern of column x / row x without the diagonal
     for (int s = 0; s < S; ++s) {
       if (s == x) continue;
       const float r = Rb[(size_t)x * S + s], c = Rb[(size_t)s * S + x];
-      acc += r;
       if (r != 0.f) { loR = s < loR ? s : loR; hiR = s > hiR ? s : hiR; }
       if (c != 0.f) { loT = s < loT ? s : loT; hiT = s > hiT ? s : hiT; }
     }
-    rowsum[x] = acc;
     bandT[x] = loT | (hiT << 8);
     bandR[x] = loR | (hiR << 8);
   }
@@ -960,13 +706,10 @@ long long tc_workspace_bytes(long long rows, int S) {
   return 0;   // every row is finished inside the kernel (no cross-kernel partials)
 }
 
-int launch_step_tcq(const ctdd_step_params* p, cudaStream_t st);
-
-// Euler modes (one categorical draw per row over all 256 states) run on the row-gather kernel of this file; every other
-// mode runs on the chunk-local kernel of ctdd_step_tcq.cu.
+// Euler modes (one categorical draw per row over all 256 states); ctdd_reverse_step sends every other mode to
+// launch_step_tcq.
 int launch_step_tc(const ctdd_step_params* p, cudaStream_t st) {
   using namespace tc;
-  if (p->mode != CTDD_MODE_EULER && p->mode != CTDD_MODE_EULER_CORR) return launch_step_tcq(p, st);
   // per-device one-time setup (function attributes live in the device's context): a bit per device ordinal
   static int num_sms[64] = {0};
   static unsigned long long attr_done = 0ull;
@@ -975,7 +718,7 @@ int launch_step_tc(const ctdd_step_params* p, cudaStream_t st) {
   const bool attr_set = dev >= 0 && dev < 64 && ((attr_done >> dev) & 1ull);
   const size_t smem_bytes = sizeof(Smem) + 1024;
   typedef void (*kern_t)(const Args);
-#define CTDD_TC_ROW(T, H) {step_tc_kernel<T, KM_EULER, H>, step_tc_kernel<T, KM_EULER_CORR, H>}
+#define CTDD_TC_ROW(T, H) {step_tc_kernel<T, false, H>, step_tc_kernel<T, true, H>}
   static const kern_t kerns[4][2] = {CTDD_TC_ROW(false, false), CTDD_TC_ROW(true, false), CTDD_TC_ROW(false, true),
                                      CTDD_TC_ROW(true, true)};
 #undef CTDD_TC_ROW
@@ -990,18 +733,7 @@ int launch_step_tc(const ctdd_step_params* p, cudaStream_t st) {
         }
     if (dev >= 0 && dev < 64) attr_done |= 1ull << dev;
   }
-  Args a;
-  a.branch = p->branch; a.D = p->D; a.reject_multi = p->reject_multi;
-  a.rows = (long long)p->N * p->D; a.row_offset = p->row_offset;
-  a.logits = p->logits; a.ld = p->ld_logits; a.batch_stride = p->batch_stride_logits;
-  a.x_eval = p->x_eval; a.x_base = p->x_base;
-  a.tab = reinterpret_cast<const uint8_t*>(p->tc_tables);
-  a.stat = reinterpret_cast<const uint8_t*>(p->tc_static);
-  a.RbT = p->RbT; a.Rb = p->Rb; a.beta = p->beta; a.h = p->h; a.seed = p->seed; a.offset = p->offset;
-  a.x_out = p->x_out; a.rr_out = p->rr_out; a.ratio_out = p->ratio_out;
-  a.stats = reinterpret_cast<unsigned long long*>(p->stats_out);
-  a.head_fix = p->head == CTDD_HEAD_LOGISTIC_FIX;
-  a.head_mu = p->head_mu; a.head_ls = p->head_log_scale; a.head_bs = p->head_batch_stride;
+  Args a = make_args(p);
   a.num_tiles = (int)((a.rows + NT - 1) / NT);
   int pairs = num_sms[dev & 63] / 2;                 // one CTA pair (cluster of 2) per TPC
   if (pairs > a.num_tiles) pairs = a.num_tiles;
@@ -1022,18 +754,15 @@ extern "C" int64_t ctdd_tc_static_align(void) { return (int64_t)ctdd::tc::ST_ALI
 extern "C" int ctdd_prep_tc_tables(const float* Q, const float* QT, const float* Rb, int T, int S, float eps,
                                    int branch, void* tables_out, void* stream) {
   using namespace ctdd;
-  (void)Q;
+  (void)Q; (void)Rb;
   if (S != tc::S) { set_error("ctdd_prep_tc_tables: the tcgen05 path needs S == 256 (got %d)", S); return 2; }
-  if (!QT || !Rb || !tables_out || T <= 0) { set_error("ctdd_prep_tc_tables: bad arguments"); return 2; }
+  if (!QT || !tables_out || T <= 0) { set_error("ctdd_prep_tc_tables: bad arguments"); return 2; }
   for (int t0 = 0; t0 < T; t0 += 32768) {
     const int nt = (T - t0) < 32768 ? (T - t0) : 32768;
     uint8_t* out = reinterpret_cast<uint8_t*>(tables_out) + (size_t)t0 * tc::TAB_BYTES;
     dim3 grid(32, nt);
     tc::prep_tables_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(QT + (size_t)t0 * S * S, nt, eps, branch, out);
     CTDD_CHECK_LAUNCH("prep_tables_kernel");
-    dim3 ggrid(S / 16, S / 16, nt), gblock(16, 16);
-    tc::prep_g_kernel<<<ggrid, gblock, 0, (cudaStream_t)stream>>>(QT + (size_t)t0 * S * S, Rb, eps, branch, out);
-    CTDD_CHECK_LAUNCH("prep_g_kernel");
   }
   return 0;
 }
@@ -1050,9 +779,3 @@ extern "C" int ctdd_prep_tc_static(const float* Rb, int S, void* static_out, voi
   CTDD_CHECK_LAUNCH("prep_static_kernel");
   return 0;
 }
-
-#ifdef CTDD_TC_TRACE
-extern "C" int ctdd_debug_trace_read(void* host, long long bytes) {
-  return (int)cudaMemcpyFromSymbol(host, ctdd::tc::g_trace, (size_t)bytes);
-}
-#endif

@@ -1037,18 +1037,7 @@ int launch_step_tcq(const ctdd_step_params* p, cudaStream_t st) {
     set_error("ctdd_reverse_step: tc_static must be aligned to ctdd_tc_static_align() = %zu bytes", tc::ST_ALIGN);
     return 2;
   }
-  tc::Args a;
-  a.branch = p->branch; a.D = p->D; a.reject_multi = p->reject_multi;
-  a.rows = (long long)p->N * p->D; a.row_offset = p->row_offset;
-  a.logits = p->logits; a.ld = p->ld_logits; a.batch_stride = p->batch_stride_logits;
-  a.x_eval = p->x_eval; a.x_base = p->x_base;
-  a.tab = reinterpret_cast<const uint8_t*>(p->tc_tables);
-  a.stat = reinterpret_cast<const uint8_t*>(p->tc_static);
-  a.RbT = p->RbT; a.Rb = p->Rb; a.beta = p->beta; a.h = p->h; a.seed = p->seed; a.offset = p->offset;
-  a.x_out = p->x_out; a.rr_out = p->rr_out; a.ratio_out = p->ratio_out;
-  a.stats = reinterpret_cast<unsigned long long*>(p->stats_out);
-  a.head_fix = p->head == CTDD_HEAD_LOGISTIC_FIX;
-  a.head_mu = p->head_mu; a.head_ls = p->head_log_scale; a.head_bs = p->head_batch_stride;
+  tc::Args a = tc::make_args(p);
   if (a.rows >= (1LL << 31)) {      // the producers index rows with 32 bits (2^31 rows would be 2 TB of logits)
     set_error("ctdd_reverse_step: N * D = %lld rows exceed the tensor path's 2^31 - 1", a.rows);
     return 2;

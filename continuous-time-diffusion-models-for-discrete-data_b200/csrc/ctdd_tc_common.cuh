@@ -15,8 +15,7 @@ constexpr int TMEM_COLS = 512;
 constexpr size_t TAB_QH_OFF = 0;                                 // uint32 [256][128]  bf16 pairs of Q^T hi
 constexpr size_t TAB_QM_OFF = TAB_QH_OFF + (size_t)S * 128 * 4;  // uint32 [256][128]  bf16 pairs of Q^T mid
 constexpr size_t TAB_A_OFF = TAB_QM_OFF + (size_t)S * 128 * 4;   // float [x][k]  tauLDR: 1/(Q[k,x]+eps); SDDM: Q[k,x]
-constexpr size_t TAB_G_OFF = TAB_A_OFF + (size_t)S * S * 4;      // float [x][k]  total-rate table (see prep_g_kernel)
-constexpr size_t TAB_BYTES = TAB_G_OFF + (size_t)S * S * 4;
+constexpr size_t TAB_BYTES = TAB_A_OFF + (size_t)S * S * 4;
 // static blob (ctdd_prep_tc_static); the caller places it on a ST_ALIGN boundary, so that "blob + offset" never carries
 // into the upper address word (the epilogue adds 32-bit offsets to a constant upper word)
 constexpr size_t ST_ALIGN = (size_t)2 << 20;
@@ -25,17 +24,14 @@ constexpr size_t ST_RBZ_OFF = (size_t)S * S * 4;                 // float [x][s]
 constexpr size_t ST_RBT_OFF = 2 * (size_t)S * S * 4;             // float [x][s] = Rb[s][x], diagonal kept (rates output)
 constexpr size_t ST_RB_OFF = 3 * (size_t)S * S * 4;              // float [x][s] = Rb[x][s], diagonal kept
 constexpr size_t ST_ZERO_OFF = 4 * (size_t)S * S * 4;            // float [S] zeros: the "row" read for chunks outside the band
-constexpr size_t ST_ROWSUM_OFF = ST_ZERO_OFF + (size_t)S * 4;    // float [x] = sum_s Rbz[x][s]
-constexpr size_t ST_BANDT_OFF = ST_ROWSUM_OFF + (size_t)S * 4;   // int [x] = lo | hi << 8: first / last s with Rbzt[x][s] != 0
+constexpr size_t ST_BANDT_OFF = ST_ZERO_OFF + (size_t)S * 4;     // int [x] = lo | hi << 8: first / last s with Rbzt[x][s] != 0
 constexpr size_t ST_BANDR_OFF = ST_BANDT_OFF + (size_t)S * 4;    // int [x], same for Rbz[x][s]   (empty: lo = 255, hi = 0)
 constexpr size_t ST_BYTES = ST_BANDR_OFF + (size_t)S * 4;
 static_assert(ST_BYTES <= ST_ALIGN, "static blob larger than its alignment");
 
-enum { KM_JUMP = 0, KM_CORR = 1, KM_RATES = 2, KM_DRIFT = 3, KM_EULER = 4, KM_EULER_CORR = 5 };
-// the corrector variants add h * R_t[x,:] to the rates; the Euler variants draw ONE categorical per row over
-// {h * rate_s (s != x), max(0, 1 - h * sum)} (sampling.py:278-293) instead of Poisson jump counts
-__host__ __device__ constexpr bool km_corr(int km) { return km == KM_CORR || km == KM_EULER_CORR; }
-__host__ __device__ constexpr bool km_euler(int km) { return km == KM_EULER || km == KM_EULER_CORR; }
+// step_q_kernel modes (the Euler modes run on step_tc_kernel); the corrector variant adds h * R_t[x,:] to the rates
+enum { KM_JUMP = 0, KM_CORR = 1, KM_RATES = 2, KM_DRIFT = 3 };
+__host__ __device__ constexpr bool km_corr(int km) { return km == KM_CORR; }
 
 struct Args {
   int branch, D, reject_multi;
@@ -46,8 +42,6 @@ struct Args {
   const int* x_base;
   const uint8_t* tab;     // per-time-point blob
   const uint8_t* stat;    // static blob
-  const float* RbT;       // [x][s] = Rb[s][x] (diagonal kept) for rr_out
-  const float* Rb;        // [x][s] diagonal kept
   float beta, h;
   unsigned long long seed, offset;
   int* x_out;
@@ -60,6 +54,24 @@ struct Args {
   const float* head_ls;
   long long head_bs;         // elements between consecutive n
 };
+
+// the kernel arguments of a step; num_tiles depends on the kernel's tile size and is left to the launcher
+inline Args make_args(const ctdd_step_params* p) {
+  Args a;
+  a.branch = p->branch; a.D = p->D; a.reject_multi = p->reject_multi;
+  a.rows = (long long)p->N * p->D; a.row_offset = p->row_offset;
+  a.logits = p->logits; a.ld = p->ld_logits; a.batch_stride = p->batch_stride_logits;
+  a.x_eval = p->x_eval; a.x_base = p->x_base;
+  a.tab = reinterpret_cast<const uint8_t*>(p->tc_tables);
+  a.stat = reinterpret_cast<const uint8_t*>(p->tc_static);
+  a.beta = p->beta; a.h = p->h; a.seed = p->seed; a.offset = p->offset;
+  a.x_out = p->x_out; a.rr_out = p->rr_out; a.ratio_out = p->ratio_out;
+  a.stats = reinterpret_cast<unsigned long long*>(p->stats_out);
+  a.head_fix = p->head == CTDD_HEAD_LOGISTIC_FIX;
+  a.head_mu = p->head_mu; a.head_ls = p->head_log_scale; a.head_bs = p->head_batch_stride;
+  a.num_tiles = 0;
+  return a;
+}
 
 // ---------------------------------------------------------------------------------------------- PTX helpers
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }

@@ -164,12 +164,12 @@ int64_t ctdd_step_workspace_bytes(int64_t rows, int S, int impl);
 int ctdd_reverse_step(const ctdd_step_params* p, void* stream);
 
 /* Derived per-time-point tables for the tcgen05 path (S == 256): bf16 hi/mid splits of Q^T in the
- * order the kernel loads them into tensor memory, the gathered-denominator table 1/(Q[k,x]+eps)
- * (tauLDR; Q[k,x] for the SDDM branch) and the total-rate table G (sum_s lam_s of a row is one dot
- * product with G[x][.]).  T time points at once. */
+ * order the kernel loads them into tensor memory and the gathered-denominator table 1/(Q[k,x]+eps)
+ * (tauLDR; Q[k,x] for the SDDM branch).  T time points at once.  The tables depend on QT, eps and
+ * branch only: Q and Rb are not read (either may be NULL). */
 int64_t ctdd_tc_tables_bytes(int S);
 /* time-independent tables of the tcgen05 path: Rb^T and Rb with zeroed and with kept diagonals (epilogue gathers), a zero
- * row, row sums, the band of non-zero base rates per state.  static_out must be aligned to ctdd_tc_static_align() bytes
+ * row, the band of non-zero base rates per state.  static_out must be aligned to ctdd_tc_static_align() bytes
  * (the epilogue addresses the blob with 32-bit offsets under a constant upper address word). */
 int64_t ctdd_tc_static_bytes(int S);
 int64_t ctdd_tc_static_align(void);

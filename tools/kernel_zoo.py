@@ -64,14 +64,17 @@ def model_for(wname):
 
 def steps():
     # C1 / C2 also at 16 x the configuration's batch (VERDICT r1 #10: the HBM-rate claim of the small-S kernels is made there;
-    # at the configurations' own batch the inputs fit in L2 and back-to-back Python calls time the host)
-    for wname, t, mult in (("C1", 0.5, 1), ("C1", 0.5, 16), ("C2", 0.1, 1), ("C2", 0.1, 16), ("C3", 0.5, 1)):
+    # at the configurations' own batch the inputs fit in L2 and back-to-back Python calls time the host).  The last line
+    # times the Euler kernel at the C4 shape: no configuration samples with Euler at S = 256.
+    for wname, t, mult, mname in (("C1", 0.5, 1, None), ("C1", 0.5, 16, None), ("C2", 0.1, 1, None), ("C2", 0.1, 16, None),
+                                  ("C3", 0.5, 1, None), ("C4", 0.5, 1, "euler")):
         w, model = model_for(wname)
+        mname = mname or w["mode"]
         S, D, B = w["S"], w["D"], w["B"] * mult
         Q, QT, beta = model.qt0_tables([t], dev)
         Rb, RbT = model.base_rate_tables(dev)
         branch = nat.branch_for(w["loss"], None)
-        mode = nat.MODE_EULER if w["mode"] == "euler" else nat.MODE_TAU_LEAP
+        mode = nat.MODE_EULER if mname == "euler" else nat.MODE_TAU_LEAP
         tc = ops.prep_tc_tables(Q, QT, Rb, 1e-9, branch) if S == 256 else None
         tcs = ops.prep_tc_static(Rb) if tc is not None else None
         lg, x0 = bench.synth_logits(B, D, S, 7, dev, None)
@@ -84,8 +87,8 @@ def steps():
                              reject_multi=not w["ordinal"], seed=1, offset=0, tc_tables=(tc[0] if tc is not None else None),
                              tc_static=tcs, workspace=ws)
         ms = timed(run)
-        name = "step_tc_kernel" if S == 256 else f"step_small_kernel<{S}>"
-        report(name, f"{wname}: S={S} D={D} N={B} {w['mode']} t={t}", ms, bytes_=4.0 * B * D * S + 8.0 * B * D,
+        name = f"step_small_kernel<{S}>" if S != 256 else ("step_tc_kernel" if mname == "euler" else "step_q_kernel")
+        report(name, f"{wname}: S={S} D={D} N={B} {mname} t={t}", ms, bytes_=4.0 * B * D * S + 8.0 * B * D,
                flop=2.0 * B * D * S * S if S == 256 else None)
     # CUDA-core block kernel at S = 256 (SDDM direct branch / cross-check path), and the exact-posterior branch sizes
     w, model = model_for("C3")
