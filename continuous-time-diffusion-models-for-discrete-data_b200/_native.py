@@ -9,8 +9,7 @@ from ctypes import c_char_p, c_float, c_int, c_int32, c_int64, c_longlong, c_uin
 import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# CTDD_B200_LIB: diagnostic builds of the same library (tools/variants.py); the product always loads the in-tree file
-LIB_PATH = os.environ.get("CTDD_B200_LIB") or os.path.join(_HERE, "libctdd_b200.so")
+LIB_PATH = os.path.join(_HERE, "libctdd_b200.so")
 
 # enums of include/ctdd.h
 BRANCH_TAULDR, BRANCH_SDDM_DIRECT, BRANCH_SDDM_REVERSE_PROB, BRANCH_SDDM_REVERSE_LOGSCALE = 0, 1, 2, 3

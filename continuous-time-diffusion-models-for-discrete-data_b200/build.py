@@ -24,14 +24,6 @@ NVCC_FLAGS = [
 ]
 
 
-if os.environ.get("CTDD_TRACE"):   # diagnostic build: per-tile clock stamps in step_q_kernel (tools/tcq_trace.py)
-    NVCC_FLAGS.append("-DCTDD_TC_TRACE")
-
-
-for _flag in os.environ.get("CTDD_DEFINES", "").split():   # diagnostic builds, e.g. CTDD_DEFINES="CTDD_EXP_NOPICK"
-    NVCC_FLAGS.append("-D" + _flag)
-
-
 def _sources():
     return sorted(os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith(".cu"))
 

@@ -35,7 +35,6 @@ constexpr int PASSES_PER_TILE = NH / 2;
 constexpr int KBLOCK_BYTES = NH * 128;
 constexpr int SPLIT_BYTES = 4 * KBLOCK_BYTES;
 constexpr int STAGE_BYTES = 2 * SPLIT_BYTES;
-constexpr int TM_QH = 0, TM_QM = 128, TM_ACC = 256;
 constexpr uint32_t IDESC = make_idesc(NT);
 
 struct Smem {
@@ -153,17 +152,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) bgem
 #pragma unroll
         for (int k = 0; k < 16; ++k) v[k] = 0.f;
       }
-      const uint32_t stage_s = smem_u32(sm.stage[st]);
-      const int r = 2 * ps + half;
-      const uint32_t off = (uint32_t)r * 128 + (uint32_t)((((l16 >> 1) ^ (r & 7)) << 4) | ((l16 & 1) << 3));
-#pragma unroll
-      for (int c = 0; c < 4; ++c) {
-        uint32_t h0, m0, h1, m1;
-        split2(v[4 * c], v[4 * c + 1], h0, m0);
-        split2(v[4 * c + 2], v[4 * c + 3], h1, m1);
-        sts64(stage_s + c * KBLOCK_BYTES + off, h0, h1);
-        sts64(stage_s + SPLIT_BYTES + c * KBLOCK_BYTES + off, m0, m1);
-      }
+      store_operand_row<KBLOCK_BYTES, SPLIT_BYTES>(smem_u32(sm.stage[st]), 2 * ps + half, l16, v);
       if (last_in_tile) {
         fence_proxy_async();
         __syncwarp();
@@ -189,29 +178,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) bgem
         mbar_wait_cluster(&sm.full[st], (i / STAGES) & 1);
         mbar_wait(&sm.tmem_empty[b], ((i / ACC) & 1) ^ 1);
         tc_fence_after();
-        const uint32_t d_tmem = tmem + TM_ACC + b * NT;
-        const uint64_t bd0 = make_b_desc(smem_u32(sm.stage[st]));
-        const uint32_t bd_lo = (uint32_t)bd0, bd_hi = (uint32_t)(bd0 >> 32);
-#pragma unroll 1
-        for (int pass = 0; pass < 3; ++pass) {
-          const uint32_t a_tmem = tmem + (pass == 2 ? TM_QM : TM_QH);
-          const uint32_t lo = bd_lo + (pass == 1 ? (uint32_t)(SPLIT_BYTES >> 4) : 0u);
-#pragma unroll
-          for (int k16 = 0; k16 < 16; ++k16) {
-            const uint32_t boff = (uint32_t)((k16 >> 2) * KBLOCK_BYTES + (k16 & 3) * 32) >> 4;
-            umma_ts_pair(d_tmem, a_tmem + k16 * 8, lo + boff, bd_hi, IDESC, (pass | k16) ? 1u : 0u);
-          }
-        }
+        issue_tile<KBLOCK_BYTES, SPLIT_BYTES, IDESC>(tmem, tmem + TM_ACC + b * NT, smem_u32(sm.stage[st]));
         umma_commit_pair(&sm.empty[st]);
         umma_commit_pair(&sm.tmem_full[b]);
       }
     } else if (rank != 0 && lane == 0) {
-      const uint32_t full_addr = mapa(smem_u32(&sm.full[0]), 0);
-      for (int i = 0; i < my_tiles; ++i) {
-        const int st = i % STAGES;
-        mbar_wait(&sm.full_local[st], (i / STAGES) & 1);
-        mbar_arrive_cluster_release(full_addr + (uint32_t)st * 8u);
-      }
+      relay_full<STAGES, POLL_NS>(sm.full_local, sm.full, my_tiles);
     }
     __syncwarp();
   } else {
@@ -273,12 +245,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) bgem
       if ((i + 1 < my_tiles) && ((g + 1) % TPS == 0)) load_matrix(bs + 1);
     }
   }
-  tc_fence_before();
-  cluster_sync_all();
-  if (warp == MMA_WARP) {
-    tc_fence_after();
-    tmem_dealloc(tmem);
-  }
+  pair_teardown(warp == MMA_WARP, tmem);
 }
 
 }  // namespace bgemm
@@ -292,28 +259,16 @@ extern "C" int ctdd_bgemm256_tc(const float* X, const float* M, int B, int D, fl
     set_error("ctdd_bgemm256_tc: X and M must be 16-byte aligned");
     return 2;
   }
-  static int num_sms[64] = {0};
-  static unsigned long long attr_done = 0ull;
-  int dev = 0;
-  cudaGetDevice(&dev);
+  static tc::PairLaunchState launch_state;
+  void (*const kerns[1])(const GemmArgs) = {bgemm_kernel};
   const size_t smem_bytes = sizeof(Smem) + 1024;
-  if (!(dev >= 0 && dev < 64 && ((attr_done >> dev) & 1ull))) {
-    cudaDeviceGetAttribute(&num_sms[dev & 63], cudaDevAttrMultiProcessorCount, dev);
-    if (cudaFuncSetAttribute(bgemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes) != cudaSuccess) {
-      set_error("ctdd_bgemm256_tc: cannot reserve %zu bytes of shared memory", smem_bytes);
-      cudaGetLastError();
-      return 1;
-    }
-    if (dev >= 0 && dev < 64) attr_done |= 1ull << dev;
-  }
   GemmArgs a;
   a.X = X; a.M = M; a.out = out; a.B = B; a.D = D;
   a.tiles_per_sample = (D + NT - 1) / NT;
   a.num_tiles = (long long)B * a.tiles_per_sample;
-  long long pairs = num_sms[dev & 63] / 2;
-  if (pairs > a.num_tiles) pairs = a.num_tiles;
-  if (pairs < 1) pairs = 1;
-  bgemm_kernel<<<(unsigned)(2 * pairs), NUM_THREADS, smem_bytes, (cudaStream_t)stream>>>(a);
+  const int pairs = tc::pair_count(launch_state, "ctdd_bgemm256_tc", kerns, smem_bytes, a.num_tiles);
+  if (!pairs) return 1;
+  bgemm_kernel<<<2 * pairs, NUM_THREADS, smem_bytes, (cudaStream_t)stream>>>(a);
   CTDD_CHECK_LAUNCH("bgemm_kernel");
   return 0;
 }

@@ -118,9 +118,6 @@ __device__ __forceinline__ void flush_stats(const RowStats& st, unsigned long lo
 // (the small-S kernels run tens of thousands of warps per launch onto the same 5 addresses).  Every thread of the CTA
 // must call it.
 __device__ __forceinline__ void flush_stats_cta(const RowStats& st, unsigned long long* stats) {
-#ifdef CTDD_WARP_STATS
-  flush_stats(st, stats);
-#else
   if (!stats) return;            // uniform: a kernel argument
   __shared__ int s_cnt[5];
   if (threadIdx.x < 5) s_cnt[threadIdx.x] = 0;
@@ -135,7 +132,6 @@ __device__ __forceinline__ void flush_stats_cta(const RowStats& st, unsigned lon
   }
   __syncthreads();
   if (threadIdx.x < 5 && s_cnt[threadIdx.x]) atomicAdd(stats + threadIdx.x, (unsigned long long)s_cnt[threadIdx.x]);
-#endif
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -145,16 +141,12 @@ __device__ __forceinline__ void flush_stats_cta(const RowStats& st, unsigned lon
 // The S = 2 lean instantiation is compiled for 8 CTAs of 128 threads per SM (64 registers) and runs as a grid-stride
 // kernel on a capped grid (a CTA pays its table prologue once for several groups of rows): 3.0 -> 3.2 TB/s at 33 M rows.
 // The S = 3 one measured 7 % slower that way (4.4 vs 4.8 TB/s) and keeps one group per thread.
-#ifndef CTDD_SMALL_MINB
-#define CTDD_SMALL_MINB 8
-#endif
-#ifndef CTDD_SMALL_GRIDCAP
-#define CTDD_SMALL_GRIDCAP 64u   // CTAs per SM of the capped grid
-#endif
+constexpr int SMALL_MINB = 8;
+constexpr unsigned SMALL_GRIDCAP = 64u;   // CTAs per SM of the capped grid
 // LEAN: the launch has dense logits and no rr_out / ratio_out (the samplers' call): the strided-row loads and the
 // (predicated, but issued) rate stores drop out as well.
 template <int S, int MODE = -1, int BRANCH = -1, bool LEAN = false>
-__global__ void __launch_bounds__(128, (LEAN && S == 2 && MODE == CTDD_MODE_TAU_LEAP) ? CTDD_SMALL_MINB : 0) step_small_kernel(StepArgs a_in) {
+__global__ void __launch_bounds__(128, (LEAN && S == 2 && MODE == CTDD_MODE_TAU_LEAP) ? SMALL_MINB : 0) step_small_kernel(StepArgs a_in) {
   StepArgs a = a_in;
   if (MODE >= 0) a.mode = MODE;
   if (BRANCH >= 0) a.branch = BRANCH;
@@ -662,7 +654,7 @@ int launch_step_simt(const ctdd_step_params* p, cudaStream_t st) {
       case 2:   // C1: S = 2, tau-leaping on the tauLDR branch
         if (a.mode == CTDD_MODE_TAU_LEAP && a.branch == CTDD_BRANCH_TAULDR && lean)    // grid-stride instantiation
           step_small_kernel<2, CTDD_MODE_TAU_LEAP, CTDD_BRANCH_TAULDR, true>
-              <<<blocks > 148u * CTDD_SMALL_GRIDCAP ? 148u * CTDD_SMALL_GRIDCAP : blocks, threads, 0, st>>>(a);
+              <<<blocks > 148u * SMALL_GRIDCAP ? 148u * SMALL_GRIDCAP : blocks, threads, 0, st>>>(a);
         else if (lean && a.branch == CTDD_BRANCH_TAULDR && a.mode == CTDD_MODE_TAU_LEAP_CORR)   // PCTauL's corrector step
           step_small_kernel<2, CTDD_MODE_TAU_LEAP_CORR, CTDD_BRANCH_TAULDR, true><<<blocks, threads, 0, st>>>(a);
         else if (lean && a.branch == CTDD_BRANCH_TAULDR && a.mode == CTDD_MODE_EULER)

@@ -56,7 +56,6 @@ constexpr int ROWS_PER_SAMPLER = NH / NUM_EPI_WARPS;                 // 4
 constexpr int KBLOCK_BYTES = NH * 128;         // one 64-wide K block of one split: NH rows x 128 B
 constexpr int SPLIT_BYTES = 4 * KBLOCK_BYTES;  // K = 256 -> 4 blocks
 constexpr int STAGE_BYTES = 2 * SPLIT_BYTES;   // hi + mid
-constexpr int TM_QH = 0, TM_QM = 128, TM_ACC = 256;  // TMEM column map (accumulator b at TM_ACC + b * NT)
 constexpr int PREFETCH_TILES = 8;      // HBM -> L2 bulk-prefetch distance (tiles of this pair's sequence)
 constexpr int LRING = 2;               // per-producer-warp ring of raw logits row pairs filled by cp.async.bulk
 constexpr uint32_t IDESC = make_idesc(NT);
@@ -138,26 +137,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem = sm.tmem_base;
-
-  // Q^T half of this CTA -> tensor memory (A operand). Warp q < 4 owns TMEM lanes [32q, 32q+32).
-  if (warp < 4) {
-    const int srow = (int)rank * 128 + warp * 32 + lane;
-#pragma unroll 1
-    for (int split = 0; split < 2; ++split) {
-      const uint4* src = reinterpret_cast<const uint4*>(a.tab + (split ? TAB_QM_OFF : TAB_QH_OFF)) + (size_t)srow * 32;
-#pragma unroll 1
-      for (int c = 0; c < 128; c += 32) {
-        uint32_t r[32];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          const uint4 v = __ldg(src + (c >> 2) + i);
-          r[4 * i] = v.x; r[4 * i + 1] = v.y; r[4 * i + 2] = v.z; r[4 * i + 3] = v.w;
-        }
-        tmem_st32(tmem + ((uint32_t)(warp * 32) << 16) + (split ? TM_QM : TM_QH) + c, r);
-      }
-    }
-    tmem_st_wait();
-  }
+  if (warp < 4) load_qt_half<4>(a.tab, tmem, rank, warp, lane);
   tc_fence_before();
   cluster_sync_all();    // barriers initialised and both A halves resident before any cross-CTA traffic
   tc_fence_after();
@@ -340,17 +320,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
 #pragma unroll
         for (int c = 0; c < 4; ++c) t4[c] = __ldg(reinterpret_cast<const float4*>(tabA + xo + 64 * c));
       }
-      // k = 64c + 4*l16 .. +3 lives in K block c, 16-byte chunk l16/2 (XOR-swizzled by the row), half l16&1
-      const uint32_t off = (uint32_t)r * 128 + (uint32_t)((((l16 >> 1) ^ (r & 7)) << 4) | ((l16 & 1) << 3));
+      // rows past the end (the last tile only) contribute zero operand rows
+      if (!ok) {
 #pragma unroll
-      for (int c = 0; c < 4; ++c) {
-        uint32_t h0, m0, h1, m1;
-        split2(v[4 * c], v[4 * c + 1], h0, m0);
-        split2(v[4 * c + 2], v[4 * c + 3], h1, m1);
-        if (!ok) h0 = m0 = h1 = m1 = 0u;
-        sts64(stage_s + c * KBLOCK_BYTES + off, h0, h1);
-        sts64(stage_s + SPLIT_BYTES + c * KBLOCK_BYTES + off, m0, m1);
+        for (int k = 0; k < 16; ++k) v[k] = 0.f;
       }
+      store_operand_row<KBLOCK_BYTES, SPLIT_BYTES>(stage_s, r, l16, v);
       // this pass's partial sums and row identity travel to the next pass (finish_prev)
       p_sum = sum; p_dot = dot;
       p_x = x_cur; p_r = r; p_slot = slot; p_close = (ps + 1 == PASSES); p_have = true;
@@ -400,32 +375,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
         mbar_wait_cluster(&sm.full[st], (i / STAGES) & 1);
         mbar_wait(&sm.tmem_empty[b], ((i / ACC) & 1) ^ 1);
         tc_fence_after();
-        const uint32_t d_tmem = tmem + TM_ACC + b * NT;
-        // one descriptor per tile; the 48 instructions differ only by compile-time offsets (16-byte units, low word)
-        const uint64_t bd0 = make_b_desc(smem_u32(sm.stage[st]));
-        const uint32_t bd_lo = (uint32_t)bd0, bd_hi = (uint32_t)(bd0 >> 32);
-#pragma unroll 1
-        for (int pass = 0; pass < 3; ++pass) {
-          const uint32_t a_tmem = tmem + (pass == 2 ? TM_QM : TM_QH);
-          const uint32_t lo = bd_lo + (pass == 1 ? (uint32_t)(SPLIT_BYTES >> 4) : 0u);
-#pragma unroll
-          for (int k16 = 0; k16 < 16; ++k16) {
-            const uint32_t boff = (uint32_t)((k16 >> 2) * KBLOCK_BYTES + (k16 & 3) * 32) >> 4;
-            umma_ts_pair(d_tmem, a_tmem + k16 * 8, lo + boff, bd_hi, IDESC, (pass | k16) ? 1u : 0u);
-          }
-        }
+        issue_tile<KBLOCK_BYTES, SPLIT_BYTES, IDESC>(tmem, tmem + TM_ACC + b * NT, smem_u32(sm.stage[st]));
         umma_commit_pair(&sm.empty[st]);
         umma_commit_pair(&sm.tmem_full[b]);
       }
     } else if (rank != 0 && lane == 0) {
-      // partner CTA: relay "my 8 producer warps have filled stage st" to the leader as ONE cluster-scope arrival
-      // (this thread has no memory traffic of its own, so its release costs nothing)
-      const uint32_t full_addr = mapa(smem_u32(&sm.full[0]), 0);
-      for (int i = 0; i < my_tiles; ++i) {
-        const int st = i % STAGES;
-        mbar_wait(&sm.full_local[st], (i / STAGES) & 1);
-        mbar_arrive_cluster_release(full_addr + (uint32_t)st * 8u);
-      }
+      relay_full<STAGES, POLL_NS>(sm.full_local, sm.full, my_tiles);
     }
     __syncwarp();
   } else {
@@ -621,12 +576,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
       }
     }
   }
-  tc_fence_before();
-  cluster_sync_all();     // no CTA of the pair may exit (or free tensor memory) while the other can still reach it
-  if (warp == MMA_WARP) {
-    tc_fence_after();
-    tmem_dealloc(tmem);
-  }
+  pair_teardown(warp == MMA_WARP, tmem);
 }
 
 // ---------------------------------------------------------------------------------------------- table prep
@@ -710,37 +660,20 @@ long long tc_workspace_bytes(long long rows, int S) {
 // launch_step_tcq.
 int launch_step_tc(const ctdd_step_params* p, cudaStream_t st) {
   using namespace tc;
-  // per-device one-time setup (function attributes live in the device's context): a bit per device ordinal
-  static int num_sms[64] = {0};
-  static unsigned long long attr_done = 0ull;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  const bool attr_set = dev >= 0 && dev < 64 && ((attr_done >> dev) & 1ull);
+  static PairLaunchState launch_state;
   const size_t smem_bytes = sizeof(Smem) + 1024;
   typedef void (*kern_t)(const Args);
-#define CTDD_TC_ROW(T, H) {step_tc_kernel<T, false, H>, step_tc_kernel<T, true, H>}
-  static const kern_t kerns[4][2] = {CTDD_TC_ROW(false, false), CTDD_TC_ROW(true, false), CTDD_TC_ROW(false, true),
+#define CTDD_TC_ROW(T, H) step_tc_kernel<T, false, H>, step_tc_kernel<T, true, H>
+  static const kern_t kerns[8] = {CTDD_TC_ROW(false, false), CTDD_TC_ROW(true, false), CTDD_TC_ROW(false, true),
                                      CTDD_TC_ROW(true, true)};
 #undef CTDD_TC_ROW
-  if (!attr_set) {
-    cudaDeviceGetAttribute(&num_sms[dev & 63], cudaDevAttrMultiProcessorCount, dev);
-    for (int i = 0; i < 4; ++i)
-      for (int j = 0; j < 2; ++j)
-        if (cudaFuncSetAttribute(kerns[i][j], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes) != cudaSuccess) {
-          set_error("ctdd_reverse_step: cannot reserve %zu bytes of shared memory for the tcgen05 kernel", smem_bytes);
-          cudaGetLastError();
-          return 1;
-        }
-    if (dev >= 0 && dev < 64) attr_done |= 1ull << dev;
-  }
   Args a = make_args(p);
   a.num_tiles = (int)((a.rows + NT - 1) / NT);
-  int pairs = num_sms[dev & 63] / 2;                 // one CTA pair (cluster of 2) per TPC
-  if (pairs > a.num_tiles) pairs = a.num_tiles;
-  if (pairs < 1) pairs = 1;
+  const int pairs = pair_count(launch_state, "ctdd_reverse_step", kerns, smem_bytes, a.num_tiles);
+  if (!pairs) return 1;
   const int ki = ((p->branch == CTDD_BRANCH_TAULDR) ? 1 : 0) + (p->head != CTDD_HEAD_LOGITS ? 2 : 0);
   const int kj = (p->mode == CTDD_MODE_EULER_CORR) ? 1 : 0;
-  kerns[ki][kj]<<<2 * pairs, NUM_THREADS, smem_bytes, st>>>(a);
+  kerns[2 * ki + kj]<<<2 * pairs, NUM_THREADS, smem_bytes, st>>>(a);
   CTDD_CHECK_LAUNCH("step_tc_kernel");
   return 0;
 }

@@ -47,10 +47,7 @@ constexpr int ACC = 2;                 // TMEM accumulator buffers (NT columns e
 constexpr int CBUF = 2;                // contribution buffers (epilogue -> finalizer)
 constexpr int RING = 7;                // per-tile row-scalar ring (> STAGES + ACC + CBUF)
 constexpr int NUM_EPI_WARPS = 8;       // epilogue warp e: TMEM quadrant e&3, column half e>>2 (= CTA that owns those rows)
-#ifndef CTDD_TCQ_NPW
-#define CTDD_TCQ_NPW 12
-#endif
-constexpr int NPW = CTDD_TCQ_NPW;      // producer warps (a multiple of 4: register budgets are per 4-warp group)
+constexpr int NPW = 12;                // producer warps (a multiple of 4: register budgets are per 4-warp group)
 constexpr int FIRST_PROD_WARP = NUM_EPI_WARPS;
 constexpr int FIRST_EPI_WARP = 0;
 constexpr int MMA_WARP = NUM_EPI_WARPS + NPW;   // light group: MMA issue / relay, idle, 2 finalizer warps
@@ -58,43 +55,26 @@ constexpr int FIN_WARP0 = MMA_WARP + 2;
 constexpr int NUM_THREADS = (NUM_EPI_WARPS + NPW + 4) * 32;
 // setmaxnreg targets.  The registers handed out by .inc are the ones the CTA's own warps released with .dec:
 // 8 * EPI + NPW * PROD + 4 * LIGHT must not exceed (12 + NPW) * (launch allocation), or the .inc never returns.
-constexpr int REGS_LAUNCH = (65536 / NUM_THREADS) & ~7;          // what __launch_bounds__ gives every thread
+constexpr int REGS_LAUNCH = (65536 / NUM_THREADS) & ~7;          // what __launch_bounds__ gives every thread (80)
 constexpr int REGS_LIGHT = 48;
-constexpr int REGS_PROD = NPW == 16 ? 64 : (NPW == 12 ? 80 : 96);
-constexpr int REGS_EPI = NPW == 8 ? 112 : 96;
+constexpr int REGS_PROD = REGS_LAUNCH;                           // producers keep the launch allocation
+constexpr int REGS_EPI = 96;
 static_assert(NUM_EPI_WARPS * REGS_EPI + NPW * REGS_PROD + 4 * REGS_LIGHT <= (NUM_EPI_WARPS + NPW + 4) * REGS_LAUNCH,
               "setmaxnreg budget exceeds the launch allocation");
 constexpr int PASSES_PER_TILE = NH / 2;                          // 32 two-row passes per tile and CTA
 constexpr int KBLOCK_BYTES = NH * 128;         // one 64-wide K block of one split: NH rows x 128 B
 constexpr int SPLIT_BYTES = 4 * KBLOCK_BYTES;  // K = 256 -> 4 blocks
 constexpr int STAGE_BYTES = 2 * SPLIT_BYTES;   // hi + mid
-constexpr int TM_QH = 0, TM_QM = 128, TM_ACC = 256;  // TMEM column map (accumulator b at TM_ACC + b * NT)
-#ifndef CTDD_LRING
-#define CTDD_LRING 2
-#endif
 // The logits ring is refilled per GROUP of 4 producer warps 4g .. 4g+3 (one per SM sub-partition, the same rank in each
 // scheduler's priority order, so they advance together): their 4 consecutive passes are 8 consecutive rows of one tile = one
 // 8 KB bulk copy per group and round.
-#ifndef CTDD_GSZ
-#define CTDD_GSZ 4
-#endif
-constexpr int GSZ = CTDD_GSZ, NSUB = CTDD_TCQ_NPW / GSZ;   // (GSZ = 1, 2, 4: passes of a group never cross a tile boundary)
-#ifndef CTDD_PREFETCH_ROUNDS
-#define CTDD_PREFETCH_ROUNDS 0
-#endif
-constexpr int PREFETCH_ROUNDS = CTDD_PREFETCH_ROUNDS;   // HBM -> L2 prefetch of the round that many rounds ahead (measured: no gain)
-#ifndef CTDD_REGPICK_MAX
-#define CTDD_REGPICK_MAX 3
-#endif
-constexpr int REGPICK_MAX = CTDD_REGPICK_MAX;   // largest per-(row, chunk) jump count of a batch that is resolved from registers (3, 7 or 11)
-constexpr int LRING = CTDD_LRING;      // per-producer-warp slots of raw logits row pairs filled by cp.async.bulk: refilled for the
+constexpr int GSZ = 4, NSUB = NPW / GSZ;   // (4 divides 32: passes of a group never cross a tile boundary)
+constexpr int REGPICK_MAX = 3;         // largest per-(row, chunk) jump count of a batch that is resolved from registers
+constexpr int LRING = 2;               // per-producer-warp slots of raw logits row pairs filled by cp.async.bulk: refilled for the
                                        // warp's next pass as soon as this pass has its values in registers (rows are L2 hits)
 constexpr int SCR_LD = 34;             // floats per row of an epilogue warp's transposing scratch (conflict-free 64-bit reads; 32 states + the jump-sum column)
 constexpr uint32_t IDESC = make_idesc(NT);
-#ifndef CTDD_POLL_LONG
-#define CTDD_POLL_LONG 512
-#endif
-constexpr uint32_t POLL_LONG = CTDD_POLL_LONG;   // ns between polls of the roles that wait for a whole tile (producers on a free stage, finalizers)
+constexpr uint32_t POLL_LONG = 512;    // ns between polls of the roles that wait for a whole tile (producers on a free stage, finalizers)
 constexpr int NCHUNK = S / JUMP_CHUNK;                           // 8 chunks of 32 states per row
 constexpr uint32_t SCAL_TX_BYTES = NH * 12;                      // row scalars the partner sends per tile
 constexpr uint32_t CONTRIB_TX_BYTES = (NUM_EPI_WARPS / 2) * 2 * 32 * 4;   // records the partner's 4 warps send per tile
@@ -104,11 +84,7 @@ struct Smem {
   alignas(16) float lring[LRING][NPW][2][S];   // raw fp32 logits rows, LRING passes of every producer warp ahead of their use
   alignas(16) float2 scal_c[RING][NT];         // (c1, c0) of the tile's rows: rows 0..63 from CTA 0, 64..127 from CTA 1
   uint32_t scal_x[RING][NT];                   // chunk mask of the band (bits 0-7) | valid << 8 | x << 10 (= table-row byte offset)
-#ifdef CTDD_EXP_NOEPI
-  alignas(16) float scratch[NUM_EPI_WARPS][2][SCR_LD];    // (diagnostic build: the epilogue does not transpose)
-#else
-  alignas(16) float scratch[NUM_EPI_WARPS][32][SCR_LD];
-#endif   // per epilogue warp: lam[row][state of the chunk] (lane = state -> lane = row)
+  alignas(16) float scratch[NUM_EPI_WARPS][32][SCR_LD];   // per epilogue warp: lam[row][state of the chunk] (lane = state -> lane = row)
   alignas(16) int contrib[CBUF][NCHUNK][NH];   // per (chunk, row of THIS CTA): sum of jumps << 2 | min(jump count, 3), or the drift's float bits
   uint8_t band[S];                             // per state x: which of the 8 chunks hold a non-zero base rate (this launch's branch / mode)
   alignas(8) uint64_t full[STAGES];            // leader CTA: its NPW producer warps + 1 relayed arrival for the partner's
@@ -125,35 +101,6 @@ struct Smem {
   uint64_t contrib_free_remote[CBUF];          // the 2 finalizer warps of the PARTNER are done with the partner's buffer
   uint32_t tmem_base;
 };
-
-#ifdef CTDD_TC_TRACE
-// diagnostic build only (CTDD_TRACE=1 python build.py): per-tile clock stamps of the first CTA pair's roles, read back with
-// ctdd_debug_trace_read_q; never compiled into the product library
-constexpr int TRACE_TILES = 512, TRACE_EVENTS = 8, TRACE_ROLES = 7;   // 5: epilogue detail (q = 0, h = 0, batch 0), 6: producer pass detail
-__device__ long long g_trace[2][TRACE_ROLES][TRACE_TILES][TRACE_EVENTS];
-#define TRACEQ(role, tile, ev)                                                                      \
-  do {                                                                                              \
-    if (blockIdx.x < 2 && (tile) < TRACE_TILES) g_trace[blockIdx.x][role][tile][ev] = clock64();    \
-  } while (0)
-// stamp taken once `dep` (a register) is available: the and.b32 consumes it, zero is a run-time 0 the compiler cannot fold
-#define TRACEQ_DEP(role, tile, ev, dep, zero)                                                       \
-  do {                                                                                              \
-    if (blockIdx.x < 2 && (tile) < TRACE_TILES) {                                                   \
-      long long c_;                                                                                 \
-      asm volatile("{ .reg .b32 t; .reg .b64 t2, c; and.b32 t, %1, %2; cvt.u64.u32 t2, t; mov.u64 c, %%clock64; add.u64 %0, c, t2; }" \
-                   : "=l"(c_) : "r"(dep), "r"(zero));                                               \
-      g_trace[blockIdx.x][role][tile][ev] = c_;                                                     \
-    }                                                                                               \
-  } while (0)
-#define TRACEQ_ADD(role, tile, ev, val)                                                             \
-  do {                                                                                              \
-    if (blockIdx.x < 2 && (tile) < TRACE_TILES) g_trace[blockIdx.x][role][tile][ev] += (val);       \
-  } while (0)
-#else
-#define TRACEQ(role, tile, ev) do { } while (0)
-#define TRACEQ_ADD(role, tile, ev, val) do { } while (0)
-#define TRACEQ_DEP(role, tile, ev, dep, zero) do { } while (0)
-#endif
 
 static_assert(sizeof(Smem) + 1024 <= 232448, "shared memory budget of one CTA (227 KB) exceeded");
 static_assert(NPW <= PASSES_PER_TILE, "every producer warp must own a pass in every tile");
@@ -212,34 +159,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem = sm.tmem_base;
-
-  // Q^T half of this CTA -> tensor memory (A operand).  A warp reaches the TMEM lanes [32q, 32q+32) of its quadrant
-  // q = warp & 3; the quadrant's 8 pieces of 32 columns (4 per bf16 split) are dealt to all the warps of that quadrant, so
-  // that the whole 128 KB is requested at once instead of in eight dependent round trips of four warps.
-  {
-    const int q = warp & 3;
-    const int srow = (int)rank * 128 + q * 32 + lane;
-    constexpr int WPQ = NUM_THREADS / 128;           // warps per quadrant
-    for (int piece = warp >> 2; piece < 8; piece += WPQ) {
-      const int split = piece >> 2, c = (piece & 3) * 32;
-      const uint4* src = reinterpret_cast<const uint4*>(a.tab + (split ? TAB_QM_OFF : TAB_QH_OFF)) + (size_t)srow * 32;
-      uint32_t r[32];
-#pragma unroll
-      for (int i = 0; i < 8; ++i) {
-        const uint4 v = __ldg(src + (c >> 2) + i);
-        r[4 * i] = v.x; r[4 * i + 1] = v.y; r[4 * i + 2] = v.z; r[4 * i + 3] = v.w;
-      }
-      tmem_st32(tmem + ((uint32_t)(q * 32) << 16) + (split ? TM_QM : TM_QH) + c, r);
-    }
-    tmem_st_wait();
-  }
+  load_qt_half<NUM_THREADS / 32>(a.tab, tmem, rank, warp, lane);
   tc_fence_before();
   cluster_sync_all();    // barriers initialised and both A halves resident before any cross-CTA traffic
   tc_fence_after();
 
   if (warp >= FIRST_PROD_WARP && warp < FIRST_PROD_WARP + NPW) {
-    if constexpr (REGS_PROD > REGS_LAUNCH) asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(REGS_PROD));
-    else if constexpr (REGS_PROD < REGS_LAUNCH) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(REGS_PROD));
     // ======================================================================== producers: 16 lanes per row, 2 rows per pass
     const int pw = warp - FIRST_PROD_WARP;
     const int half = lane >> 4, l16 = lane & 15;
@@ -309,18 +234,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
       const bool ok = x_cur >= 0;
       const int x = ok ? x_cur : 0;
       const bool last_in_tile = ps + NPW >= PASSES_PER_TILE;     // this warp's next pass belongs to another tile
-#ifdef CTDD_TC_TRACE
-      const long long tq0 = clock64();
-      const bool ptr_on = (pw == 0 && lane == 0 && tl != last_tl);
-      const uint32_t pzero = (uint32_t)a.head_fix >> 8;
-      if (ptr_on) TRACEQ(6, tl, 0);
-#endif
       const int rslot = ring_n % LRING;
       mbar_wait(&sm.lring_full_g[rslot][pw / GSZ], (uint32_t)((ring_n / LRING) & 1));
-#ifdef CTDD_TC_TRACE
-      if (pw == 0 && lane == 0) TRACEQ_ADD(0, tl, 3, clock64() - tq0);
-      if (ptr_on) TRACEQ(6, tl, 1);
-#endif
       const int r = 2 * ps + half;
       float v[16];
       float ml = 0.f;
@@ -346,14 +261,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
           v[4 * c] = q4.x; v[4 * c + 1] = q4.y; v[4 * c + 2] = q4.z; v[4 * c + 3] = q4.w;
         }
         ++ring_n;
-#ifdef CTDD_TC_TRACE
-        if (ptr_on) TRACEQ_DEP(6, tl, 2, __float_as_uint(v[15]), pzero);
-#endif
         __syncwarp();            // every lane has its values: the group's slots may be refilled once its 4 warps say so
         if (lane == 0) mbar_arrive(&sm.lring_free_g[rslot][pw / GSZ]);
-#ifdef CTDD_TC_TRACE
-        if (ptr_on) TRACEQ(6, tl, 3);
-#endif
         float m4[4];
 #pragma unroll
         for (int c = 0; c < 4; ++c) m4[c] = fmaxf(fmaxf(v[4 * c], v[4 * c + 1]), fmaxf(v[4 * c + 2], v[4 * c + 3]));
@@ -366,24 +275,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
         }
         ml = -m * 1.4426950408889634f;
       }
-#ifdef CTDD_TC_TRACE
-      if (ptr_on) TRACEQ_DEP(6, tl, 4, __float_as_uint(ml), pzero);
-#endif
       finish_prev();
-#ifdef CTDD_TC_TRACE
-      if (ptr_on) TRACEQ(6, tl, 5);
-#endif
       if (tl != last_tl) {       // first pass of this warp in a new tile: the tile's operand stage must be free
-        if (pw == 0 && lane == 0) TRACEQ(0, tl, 0);
         mbar_wait<POLL_LONG>(&sm.empty[st], (uint32_t)(((tl / STAGES) & 1) ^ 1));
-        if (pw == 0 && lane == 0) TRACEQ(0, tl, 1);
         last_tl = tl;
       }
       const uint32_t stage_s = smem_u32(sm.stage[st]);
-#ifdef CTDD_EXP_NOPRODUCE    // diagnostic build: producers only run the barrier protocol (isolates MMA + epilogue)
-      (void)stage_s; (void)ml; (void)r;
-      const float sum = 1.f, dot = 0.f;
-#else
       // four independent accumulation chains of packed pairs
       float2 sum2[4], dot2[4];
       const float2 l2e2 = make_float2(1.4426950408889634f, 1.4426950408889634f), ml2 = make_float2(ml, ml);
@@ -411,9 +308,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
         const float2 d01 = fadd2(dot2[0], dot2[1]), d23 = fadd2(dot2[2], dot2[3]), dall = fadd2(d01, d23);
         dot = dall.x + dall.y;
       }
-#ifdef CTDD_TC_TRACE
-      if (ptr_on) TRACEQ_DEP(6, tl, 6, __float_as_uint(sum), pzero);
-#endif
       // the table row of the NEXT pass is requested as soon as this pass's has been consumed
       {
         const size_t xo = (size_t)(x_n1 < 0 ? 0 : x_n1) << 8;
@@ -427,22 +321,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
           for (int k = 0; k < 16; ++k) v[k] = 0.f;
         }
       }
-      // k = 64c + 4*l16 .. +3 lives in K block c, 16-byte chunk l16/2 (XOR-swizzled by the row), half l16&1
-      const uint32_t off = (uint32_t)r * 128 + (uint32_t)((((l16 >> 1) ^ (r & 7)) << 4) | ((l16 & 1) << 3));
-#pragma unroll
-      for (int c = 0; c < 4; ++c) {
-        uint32_t h0, m0, h1, m1;
-        split2(v[4 * c], v[4 * c + 1], h0, m0);
-        split2(v[4 * c + 2], v[4 * c + 3], h1, m1);
-        {
-          sts64(stage_s + c * KBLOCK_BYTES + off, h0, h1);
-          sts64(stage_s + SPLIT_BYTES + c * KBLOCK_BYTES + off, m0, m1);
-        }
-      }
-#endif
-#ifdef CTDD_TC_TRACE
-      if (ptr_on) TRACEQ(6, tl, 7);
-#endif
+      store_operand_row<KBLOCK_BYTES, SPLIT_BYTES>(stage_s, r, l16, v);
       // this pass's partial sums and row identity travel to the next pass (finish_prev)
       p_sum = sum; p_dot = dot;
       p_x = x; p_ok = ok; p_idx = slot * NT + (int)rank * NH + r; p_slot = slot; p_last = last_in_tile; p_have = true;
@@ -450,7 +329,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
         fence_proxy_async();
         __syncwarp();
         if (lane == 0) mbar_arrive(full_bar + st);
-        if (pw == 0 && lane == 0) TRACEQ(0, tl, 2);
       }
       x_cur = x_n1;
       x_n1 = fetch(P + 2 * NPW);
@@ -550,14 +428,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
           } else {               // strided logits: one copy per row
             for (long long rr = 0; rr < nA; ++rr) bulk_g2s(dA + rr * S, row_ptr(rA + rr), S * 4, gbar);
           }
-          if (contiguous && PREFETCH_ROUNDS > 0) {      // the rows of a later round from HBM into L2
-            const int Q0 = P0 + PREFETCH_ROUNDS * NPW;
-            if (Q0 < total) {
-              const long long qA = row00 + (long long)(Q0 >> 5) * tile_rows + 2 * (Q0 & 31);
-              const long long mA = seg_rows(qA);
-              if (mA > 0) l2_prefetch_bulk(a.logits + qA * S, (uint32_t)mA * S * 4);
-            }
-          }
           ++grp;
           did = true;
         }
@@ -616,16 +486,13 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
       for (int i = 0; i < my_tiles; ++i) {
         const int tile = pair + i * npairs, slot = i % RING, cb = i % CBUF;
         const long long g = (long long)tile * NT + (long long)rank * NH + r;
-        if (r == 0) TRACEQ(4, i, 0);
         mbar_wait<POLL_LONG>(&sm.scal_full[slot], (i / RING) & 1);
-        if (r == 0) TRACEQ(4, i, 1);
         const uint32_t sx = sm.scal_x[slot][rank * NH + r];
         const int x = (int)((sx >> 10) & 255u);
         const bool valid = (sx >> 8) & 1u;
         int xb = x;
         if (a.x_base && valid) xb = __ldg(a.x_base + g);
         mbar_wait<POLL_LONG>(&sm.contrib_full[cb], (i / CBUF) & 1);
-        if (r == 0) TRACEQ(4, i, 2);
         int jump = 0, cnt = 0;
         float drift = 0.f;
 #pragma unroll
@@ -653,7 +520,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
           mbar_arrive(&sm.contrib_free_local[cb]);
           mbar_arrive_cluster_relaxed(cfree_remote + (uint32_t)cb * 8u);
         }
-        if (r == 0) TRACEQ(4, i, 3);
       }
       if (a.stats) {
         const int v[5] = {stt.changed_base, stt.nonzero, stt.changed_eval, stt.jumped, stt.multi};
@@ -670,43 +536,19 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
     if (rank == 0 && lane == 0) {
       for (int i = 0; i < my_tiles; ++i) {
         const int st = i % STAGES, b = i % ACC;
-        TRACEQ(1, i, 0);
         mbar_wait_cluster(&sm.full[st], (i / STAGES) & 1);
-        TRACEQ(1, i, 1);
         mbar_wait(&sm.tmem_empty[b], ((i / ACC) & 1) ^ 1);
-        TRACEQ(1, i, 2);
         tc_fence_after();
-        const uint32_t d_tmem = tmem + TM_ACC + b * NT;
-        // one descriptor per tile; the 48 instructions differ only by compile-time offsets (16-byte units, low word)
-        const uint64_t bd0 = make_b_desc(smem_u32(sm.stage[st]));
-        const uint32_t bd_lo = (uint32_t)bd0, bd_hi = (uint32_t)(bd0 >> 32);
-#pragma unroll 1
-        for (int pass = 0; pass < 3; ++pass) {
-          const uint32_t a_tmem = tmem + (pass == 2 ? TM_QM : TM_QH);
-          const uint32_t lo = bd_lo + (pass == 1 ? (uint32_t)(SPLIT_BYTES >> 4) : 0u);
-#pragma unroll
-          for (int k16 = 0; k16 < 16; ++k16) {
-            const uint32_t boff = (uint32_t)((k16 >> 2) * KBLOCK_BYTES + (k16 & 3) * 32) >> 4;
-            umma_ts_pair(d_tmem, a_tmem + k16 * 8, lo + boff, bd_hi, IDESC, (pass | k16) ? 1u : 0u);
-          }
-        }
+        issue_tile<KBLOCK_BYTES, SPLIT_BYTES, IDESC>(tmem, tmem + TM_ACC + b * NT, smem_u32(sm.stage[st]));
         umma_commit_pair(&sm.empty[st]);
         umma_commit_pair(&sm.tmem_full[b]);
-        TRACEQ(1, i, 3);
       }
     } else if (rank != 0 && lane == 0) {
-      // partner CTA: relay "my producers have filled stage st" to the leader as ONE cluster-scope arrival
-      // (this thread has no memory traffic of its own, so its release costs nothing)
-      const uint32_t full_addr = mapa(smem_u32(&sm.full[0]), 0);
-      for (int i = 0; i < my_tiles; ++i) {
-        const int st = i % STAGES;
-        mbar_wait<POLL_LONG>(&sm.full_local[st], (i / STAGES) & 1);
-        mbar_arrive_cluster_release(full_addr + (uint32_t)st * 8u);
-      }
+      relay_full<STAGES, POLL_LONG>(sm.full_local, sm.full, my_tiles);
     }
     __syncwarp();
   } else {
-    if constexpr (REGS_EPI > REGS_LAUNCH) asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(REGS_EPI));
+    asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(REGS_EPI));
     // ======================================================================== epilogue: lane = state
     const int ew = warp - FIRST_EPI_WARP;         // (FIRST_EPI_WARP is a multiple of 4: ew & 3 is the warp's TMEM quadrant)
     const int q = ew & 3;                         // TMEM quadrant -> states rank*128 + 32q + lane = one chunk of the map
@@ -734,16 +576,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
     for (int i = 0; i < my_tiles; ++i) {
       const int tile = pair + i * npairs;
       const int slot = i % RING, b = i % ACC, cb = i % CBUF;
-      const int trole = 2 + (ew >> 2);
-      const bool tr_on = (q == 0 && lane == 0);
-      if (tr_on) TRACEQ(trole, i, 0);
       mbar_wait(&sm.scal_full[slot], (i / RING) & 1);
-      if (tr_on) TRACEQ(trole, i, 1);
       mbar_wait(&sm.tmem_full[b], (i / ACC) & 1);
       tc_fence_after();
-      if (tr_on) TRACEQ(trole, i, 2);
       if (SAMPLES) mbar_wait(cfree_wait + cb, ((i / CBUF) & 1) ^ 1);
-      if (tr_on) TRACEQ(trole, i, 3);
 #pragma unroll 1
       for (int bb = 0; bb < 2; ++bb) {
         const int col = (int)h * NH + 32 * bb;                         // tile column (= tile row) of this batch's row 0
@@ -798,21 +634,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
           Philox4 p0 = {{0u, 0u, 0u, 0u}};
           if constexpr (KM == KM_JUMP || KM == KM_CORR) p0 = philox_rowjump(grow, cbase, a.offset, a.seed);
           tmem_ld_wait();
-          if (tr_on) TRACEQ(trole, i, 4 + 2 * bb);
           if (bb == 1) {           // the accumulator has been read: hand the buffer back to the MMA warp
             tc_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive_cluster_relaxed(tempty_dst + (uint32_t)b * 8u);
           }
-#ifdef CTDD_EXP_NOEPI        // diagnostic build: the epilogue only drains the accumulator (isolates producers + MMA)
-          {
-            const uint32_t roff = (uint32_t)cb * (NCHUNK * NH * 4) + (uint32_t)(32 * bb + lane) * 4u;
-            const uint32_t z = (__float_as_uint(R[lane & 1]) ^ acc[lane & 3]) == 0x7fc12345u;
-            if (h == rank) asm volatile("st.shared.b32 [%0], %1;" ::"r"(contrib_dst + roff), "r"(z) : "memory");
-            else st_async_cluster_b32(contrib_dst + roff, z, cfull_dst + (uint32_t)cb * 8u);
-          }
-          continue;
-#endif
           // transpose through the warp's scratch: lane = state -> lane = row (row `lane` of the batch, the chunk's 32 states)
           __syncwarp();          // the previous batch's reads of the scratch are done
 #pragma unroll
@@ -823,14 +649,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
           for (int c = 0; c < 16; ++c) {
             asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(p[2 * c]), "=f"(p[2 * c + 1]) : "r"(scr_p + (uint32_t)(lane * SCR_LD + 2 * c) * 4u));
           }
-#ifdef CTDD_TC_TRACE
-          const uint32_t tzero = (uint32_t)a.head_fix >> 8;
-          if (tr_on && h == 0 && bb == 0) {
-            TRACEQ(5, i, 0);
-            TRACEQ_DEP(5, i, 1, __float_as_uint(p[31]), tzero);    // transposed values have arrived
-            TRACEQ_DEP(5, i, 2, __float_as_uint(p[0]), tzero);
-          }
-#endif
           // lam[s, row] (zero at s == x through the zero-diagonal tables).  tauLDR without corrector: the row's scale c1
           // is applied to the chunk total only (the picks are scale-invariant); otherwise per element.
           float sc1 = 0.f, sc0 = 0.f;
@@ -870,24 +688,15 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
             }
             float tot = p[31];
             if constexpr (UNSCALED) tot *= sc1;
-#ifdef CTDD_TC_TRACE
-            if (tr_on && h == 0 && bb == 0) TRACEQ_DEP(5, i, 3, __float_as_uint(tot), tzero);   // prefix chain done
-#endif
             int K = poisson_from_unit(tot, u32_to_unit(p0.w[0]));
             K = K > JUMP_PICK_CAP ? JUMP_PICK_CAP : K;
             rec.y = K;
-#ifdef CTDD_EXP_NOPICK       // diagnostic build: counts are drawn, picks are not resolved
-            K = 0;
-#endif
             // Picks: first state whose prefix sum exceeds v * total.  The picks of the batch's 32 rows are dealt to the
             // 32 lanes (a row with K picks would otherwise keep 31 lanes idle for K rounds): lane = row parks its prefix
             // sums in its scratch row, a warp scan of K numbers the picks, and lane i resolves pick base + i of whatever
             // row it belongs to (row found by a 5-shuffle search over the scan, uniforms fetched from the row's lane).
             int jump = 0;
             const uint32_t any = __ballot_sync(0xffffffffu, K > 0);
-#ifdef CTDD_TC_TRACE
-            if (tr_on && h == 0 && bb == 0) { TRACEQ_DEP(5, i, 4, any, tzero); TRACEQ_ADD(5, i, 6, (long long)__popc(any)); }   // counts drawn
-#endif
             // Few picks per row (the common case once the schedule has left its first tenth): every lane resolves the
             // picks of ITS row from the prefix sums it holds in registers - the pick is the number of prefix sums <= the
             // target, 31 independent compares, no shared memory, no shuffles; one round per pick, uniforms of call 0.
@@ -895,13 +704,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
             if (any) maxK = __reduce_max_sync(0xffffffffu, K);
             if (any && maxK <= REGPICK_MAX) {
               const float ptot = p[31];
-              Philox4 pc1 = {{0u, 0u, 0u, 0u}}, pc2 = {{0u, 0u, 0u, 0u}};
-              if (REGPICK_MAX > 3 && maxK > 3) pc1 = philox_rowjump(grow, cbase + 1u, a.offset, a.seed);     // picks 3..6
-              if (REGPICK_MAX > 7 && maxK > 7) pc2 = philox_rowjump(grow, cbase + 2u, a.offset, a.seed);     // picks 7..10
 #pragma unroll
               for (int j = 0; j < REGPICK_MAX; ++j) {
                 if (j < maxK) {
-                  const uint32_t w = j < 3 ? p0.w[1 + j] : (j < 7 ? pc1.w[j - 3] : pc2.w[j - 7]);
+                  const uint32_t w = p0.w[1 + j];   // the three pick uniforms of the row's Philox call
                   float T = fminf(u32_to_unit(w), 0.99999994f) * ptot;
                   // the product can round up to the total itself: then the pick is the last state with a positive rate
                   if (T >= ptot) T = __uint_as_float(__float_as_uint(ptot) - 1u);
@@ -971,9 +777,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
               asm volatile("ld.shared.s32 %0, [%1];" : "=r"(jump) : "r"(scr_p + (uint32_t)(lane * SCR_LD + 32) * 4u));
             }
             rec.x = jump;
-#ifdef CTDD_TC_TRACE
-            if (tr_on && h == 0 && bb == 0) TRACEQ_DEP(5, i, 5, (uint32_t)jump, tzero);   // picks resolved
-#endif
           }
           // the record of (row `lane`, this chunk) goes to the CTA that produced the row
           const uint32_t roff = (uint32_t)cb * (NCHUNK * NH * 4) + (uint32_t)(32 * bb + lane) * 4u;
@@ -983,7 +786,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
           } else {
             st_async_cluster_b32(contrib_dst + roff, word, cfull_dst + (uint32_t)cb * 8u);
           }
-          if (tr_on) TRACEQ(trole, i, 5 + 2 * bb);
         }
       }
       if (SAMPLES && h == rank) {
@@ -996,43 +798,22 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
       }
     }
   }
-  tc_fence_before();
-  cluster_sync_all();     // no CTA of the pair may exit (or free tensor memory) while the other can still reach it
-  if (warp == MMA_WARP) {
-    tc_fence_after();
-    tmem_dealloc(tmem);
-  }
+  pair_teardown(warp == MMA_WARP, tmem);
 }
 
 }  // namespace tcq
 
 int launch_step_tcq(const ctdd_step_params* p, cudaStream_t st) {
   using namespace tcq;
-  // per-device one-time setup (function attributes live in the device's context): a bit per device ordinal
-  static int num_sms[64] = {0};
-  static unsigned long long attr_done = 0ull;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  const bool attr_set = dev >= 0 && dev < 64 && ((attr_done >> dev) & 1ull);
+  static tc::PairLaunchState launch_state;
   const size_t smem_bytes = sizeof(Smem) + 1024;
   typedef void (*kern_t)(const tc::Args);
 #define CTDD_TCQ_ROW(T, H)                                                                                        \
-  {step_q_kernel<T, tc::KM_JUMP, H>, step_q_kernel<T, tc::KM_CORR, H>, step_q_kernel<T, tc::KM_RATES, H>,       \
-   step_q_kernel<T, tc::KM_DRIFT, H>}
-  static const kern_t kerns[4][4] = {CTDD_TCQ_ROW(false, false), CTDD_TCQ_ROW(true, false), CTDD_TCQ_ROW(false, true),
+  step_q_kernel<T, tc::KM_JUMP, H>, step_q_kernel<T, tc::KM_CORR, H>, step_q_kernel<T, tc::KM_RATES, H>,        \
+      step_q_kernel<T, tc::KM_DRIFT, H>
+  static const kern_t kerns[16] = {CTDD_TCQ_ROW(false, false), CTDD_TCQ_ROW(true, false), CTDD_TCQ_ROW(false, true),
                                      CTDD_TCQ_ROW(true, true)};
 #undef CTDD_TCQ_ROW
-  if (!attr_set) {
-    cudaDeviceGetAttribute(&num_sms[dev & 63], cudaDevAttrMultiProcessorCount, dev);
-    for (int i = 0; i < 4; ++i)
-      for (int j = 0; j < 4; ++j)
-        if (cudaFuncSetAttribute(kerns[i][j], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes) != cudaSuccess) {
-          set_error("ctdd_reverse_step: cannot reserve %zu bytes of shared memory for the tcgen05 kernel", smem_bytes);
-          cudaGetLastError();
-          return 1;
-        }
-    if (dev >= 0 && dev < 64) attr_done |= 1ull << dev;
-  }
   if (reinterpret_cast<uintptr_t>(p->tc_static) % tc::ST_ALIGN) {
     set_error("ctdd_reverse_step: tc_static must be aligned to ctdd_tc_static_align() = %zu bytes", tc::ST_ALIGN);
     return 2;
@@ -1043,29 +824,16 @@ int launch_step_tcq(const ctdd_step_params* p, cudaStream_t st) {
     return 2;
   }
   a.num_tiles = (int)((a.rows + NT - 1) / NT);
-  int pairs = num_sms[dev & 63] / 2;                 // one CTA pair (cluster of 2) per TPC
-  if (pairs > a.num_tiles) pairs = a.num_tiles;
-  if (pairs < 1) pairs = 1;
+  const int pairs = tc::pair_count(launch_state, "ctdd_reverse_step", kerns, smem_bytes, a.num_tiles);
+  if (!pairs) return 1;
   const int ki = ((p->branch == CTDD_BRANCH_TAULDR) ? 1 : 0) + (p->head != CTDD_HEAD_LOGITS ? 2 : 0);
   int kj = 0;
   if (p->mode == CTDD_MODE_RATES_ONLY) kj = 2;
   else if (p->mode == CTDD_MODE_TAU_LEAP_CORR) kj = 1;
   else if (p->mode == CTDD_MODE_MIDPOINT_DRIFT) kj = 3;
-  kerns[ki][kj]<<<2 * pairs, NUM_THREADS, smem_bytes, st>>>(a);
+  kerns[4 * ki + kj]<<<2 * pairs, NUM_THREADS, smem_bytes, st>>>(a);
   CTDD_CHECK_LAUNCH("step_q_kernel");
   return 0;
 }
-
-
-#ifdef CTDD_TC_TRACE
-extern "C" int ctdd_debug_trace_read_q(void* host, long long bytes) {
-  return (int)cudaMemcpyFromSymbol(host, ctdd::tcq::g_trace, (size_t)bytes);
-}
-extern "C" int ctdd_debug_trace_clear_q() {
-  void* p = nullptr;
-  cudaGetSymbolAddress(&p, ctdd::tcq::g_trace);
-  return (int)cudaMemset(p, 0, sizeof(ctdd::tcq::g_trace));
-}
-#endif
 
 }  // namespace ctdd

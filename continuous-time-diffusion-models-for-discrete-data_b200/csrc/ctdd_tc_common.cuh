@@ -1,6 +1,8 @@
-// Shared pieces of the tcgen05 reverse-step kernels (ctdd_step_tc.cu: Euler modes, ctdd_step_tcq.cu: every other mode):
-// table-blob layout, kernel arguments, PTX wrappers (mbarrier, tcgen05, bulk copies, packed fp32 pairs), the bf16
-// hi/mid split and the softmax numerators of the truncated-logistic head.
+// Shared pieces of the three tcgen05 kernels: the reverse-step kernels (ctdd_step_tc.cu: Euler modes, ctdd_step_tcq.cu:
+// every other mode) and the per-sample contraction of the losses (ctdd_bgemm_tc.cu).  Table-blob layout and kernel
+// arguments of the step kernels, PTX wrappers (mbarrier, tcgen05, bulk copies, packed fp32 pairs), the bf16 hi/mid split,
+// the CTA-pair plumbing all three share (operand rows, MMA issue, relay, teardown, launch geometry) and the softmax
+// numerators of the truncated-logistic head.
 #pragma once
 #include "ctdd_common.cuh"
 #include <cuda_bf16.h>
@@ -10,6 +12,7 @@ namespace tc {
 
 constexpr int S = 256;
 constexpr int TMEM_COLS = 512;
+constexpr int TM_QH = 0, TM_QM = 128, TM_ACC = 256;  // TMEM column map: A operand hi / mid, accumulator b at TM_ACC + b * NT
 
 // per-time-point table blob (ctdd_prep_tc_tables)
 constexpr size_t TAB_QH_OFF = 0;                                 // uint32 [256][128]  bf16 pairs of Q^T hi
@@ -109,10 +112,8 @@ __device__ __forceinline__ void mbar_arrive_cluster_relaxed(uint32_t cluster_add
 // sleep / try_wait loop - a warp that has to wait longer must not eat issue slots of the warps it is waiting for.
 // SLEEP_NS: pause between polls; roles whose waits are long (a whole tile) and whose wake-up is not on the critical path
 // use a longer one.
-#ifndef CTDD_POLL_NS
-#define CTDD_POLL_NS 96
-#endif
-template <uint32_t SLEEP_NS = CTDD_POLL_NS>
+constexpr uint32_t POLL_NS = 96;
+template <uint32_t SLEEP_NS = POLL_NS>
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
   asm volatile(
       "{\n"
@@ -344,6 +345,123 @@ __device__ __forceinline__ void split2(float a0, float a1, uint32_t& hi, uint32_
   __nv_bfloat162 m = __floats2bfloat162_rn(r0, r1);
 #endif
   mid = *reinterpret_cast<uint32_t*>(&m);
+}
+
+// ---------------------------------------------------------------------------------------------- CTA-pair plumbing
+// Each kernel runs on CTA pairs (cluster of 2, cta_group::2).  The A operand, one CTA's 128-row half of a 256 x 256 matrix
+// split into bf16 hi and mid, stays in tensor memory at TM_QH / TM_QM.  The B operand is a smem stage of the CTA's rows
+// of a tile, K-major and 128B-swizzled: the hi split, then the mid split (SPLIT_BYTES each), each 4 K blocks of
+// KBLOCK_BYTES = rows x 128 B.
+
+// One operand row of a producer half-warp: lane l16 holds k = 64c + 4*l16 .. +3 (c = 0..3) of row r, which lives in
+// K block c, 16-byte chunk l16/2 (XOR-swizzled by the row), half l16&1 (the layout make_b_desc describes).
+template <int KBLOCK_BYTES, int SPLIT_BYTES>
+__device__ __forceinline__ void store_operand_row(uint32_t stage, int r, int l16, const float (&v)[16]) {
+  const uint32_t off = (uint32_t)r * 128 + (uint32_t)((((l16 >> 1) ^ (r & 7)) << 4) | ((l16 & 1) << 3));
+#pragma unroll
+  for (int c = 0; c < 4; ++c) {
+    uint32_t h0, m0, h1, m1;
+    split2(v[4 * c], v[4 * c + 1], h0, m0);
+    split2(v[4 * c + 2], v[4 * c + 3], h1, m1);
+    sts64(stage + c * KBLOCK_BYTES + off, h0, h1);
+    sts64(stage + SPLIT_BYTES + c * KBLOCK_BYTES + off, m0, m1);
+  }
+}
+
+// The 48 tcgen05.mma of one tile: 3 passes Qh*ah + Qh*am + Qm*ah of 16 K steps into the accumulator at d_tmem.  One
+// descriptor per tile; the 48 instructions differ only by compile-time offsets (16-byte units, low word).
+template <int KBLOCK_BYTES, int SPLIT_BYTES, uint32_t IDESC>
+__device__ __forceinline__ void issue_tile(uint32_t tmem, uint32_t d_tmem, uint32_t stage) {
+  const uint64_t bd0 = make_b_desc(stage);
+  const uint32_t bd_lo = (uint32_t)bd0, bd_hi = (uint32_t)(bd0 >> 32);
+#pragma unroll 1
+  for (int pass = 0; pass < 3; ++pass) {
+    const uint32_t a_tmem = tmem + (pass == 2 ? TM_QM : TM_QH);
+    const uint32_t lo = bd_lo + (pass == 1 ? (uint32_t)(SPLIT_BYTES >> 4) : 0u);
+#pragma unroll
+    for (int k16 = 0; k16 < 16; ++k16) {
+      const uint32_t boff = (uint32_t)((k16 >> 2) * KBLOCK_BYTES + (k16 & 3) * 32) >> 4;
+      umma_ts_pair(d_tmem, a_tmem + k16 * 8, lo + boff, bd_hi, IDESC, (pass | k16) ? 1u : 0u);
+    }
+  }
+}
+
+// Partner CTA: relay "my producer warps have filled stage st" (full_local) to the leader's full barrier as ONE
+// cluster-scope arrival per tile (this thread has no memory traffic of its own, so its release costs nothing).
+template <int STAGES, uint32_t SLEEP_NS>
+__device__ __forceinline__ void relay_full(uint64_t* full_local, uint64_t* full, int my_tiles) {
+  const uint32_t full_addr = mapa(smem_u32(full), 0);
+  for (int i = 0; i < my_tiles; ++i) {
+    const int st = i % STAGES;
+    mbar_wait<SLEEP_NS>(&full_local[st], (i / STAGES) & 1);
+    mbar_arrive_cluster_release(full_addr + (uint32_t)st * 8u);
+  }
+}
+
+// The step kernels' A operand: this CTA's 128-state half of Q^T (bf16 hi + mid pairs of the table blob) -> tensor
+// memory, loaded by warps 0 .. LOAD_WARPS - 1 (a multiple of 4).  A warp reaches the TMEM lanes [32q, 32q+32) of its
+// quadrant q = warp & 3; the quadrant's 8 pieces of 32 columns (4 per bf16 split) are dealt to the loading warps of that
+// quadrant.  step_q_kernel lets all its warps load, so that the whole 128 KB is requested at once.  step_tc_kernel keeps
+// its four loading warps (each loads its quadrant's 8 pieces): dealt to all 20 of its warps, its Euler step at the C4
+// shape (tools/kernel_zoo.py) took 1.747-1.750 ms instead of 1.724-1.736 ms (three alternated runs each, one B200 with
+// a 1000 W power limit).
+template <int LOAD_WARPS>
+__device__ __forceinline__ void load_qt_half(const uint8_t* tab, uint32_t tmem, uint32_t rank, int warp, int lane) {
+  const int q = warp & 3;
+  const int srow = (int)rank * 128 + q * 32 + lane;
+  constexpr int WPQ = LOAD_WARPS / 4;              // loading warps per quadrant
+#pragma unroll 1
+  for (int piece = warp >> 2; piece < 8; piece += WPQ) {
+    const int split = piece >> 2, c = (piece & 3) * 32;
+    const uint4* src = reinterpret_cast<const uint4*>(tab + (split ? TAB_QM_OFF : TAB_QH_OFF)) + (size_t)srow * 32;
+    uint32_t r[32];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      const uint4 v = __ldg(src + (c >> 2) + i);
+      r[4 * i] = v.x; r[4 * i + 1] = v.y; r[4 * i + 2] = v.z; r[4 * i + 3] = v.w;
+    }
+    tmem_st32(tmem + ((uint32_t)(q * 32) << 16) + (split ? TM_QM : TM_QH) + c, r);
+  }
+  tmem_st_wait();
+}
+
+// End of a pair kernel: no CTA of the pair may exit (or free tensor memory) while the other can still reach it.
+// `alloc_warp`: the warp that allocated the tensor memory frees it.
+__device__ __forceinline__ void pair_teardown(bool alloc_warp, uint32_t tmem) {
+  tc_fence_before();
+  cluster_sync_all();
+  if (alloc_warp) {
+    tc_fence_after();
+    tmem_dealloc(tmem);
+  }
+}
+
+// Host side of a pair-kernel launcher.  Function attributes live in the device's context, so each launcher reserves its
+// kernels' dynamic shared memory once per device ordinal (a bit of `attr_done`) and reads the SM count then.
+struct PairLaunchState {
+  int num_sms[64] = {0};
+  unsigned long long attr_done = 0ull;
+};
+// Makes that reservation for every kernel of `kerns` on the current device if it has not been made, and returns the number
+// of CTA pairs of the grid for num_tiles tiles: one pair per TPC, at most one per tile, at least one.  Returns 0 with the
+// error set (in the name of `who`) when the reservation fails.
+template <typename Kernel, size_t N>
+inline int pair_count(PairLaunchState& ls, const char* who, const Kernel (&kerns)[N], size_t smem_bytes, long long num_tiles) {
+  int dev = 0;
+  cudaGetDevice(&dev);
+  if (!(dev >= 0 && dev < 64 && ((ls.attr_done >> dev) & 1ull))) {
+    cudaDeviceGetAttribute(&ls.num_sms[dev & 63], cudaDevAttrMultiProcessorCount, dev);
+    for (size_t i = 0; i < N; ++i)
+      if (cudaFuncSetAttribute(kerns[i], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes) != cudaSuccess) {
+        set_error("%s: cannot reserve %zu bytes of shared memory for the tcgen05 kernel", who, smem_bytes);
+        cudaGetLastError();
+        return 0;
+      }
+    if (dev >= 0 && dev < 64) ls.attr_done |= 1ull << dev;
+  }
+  long long pairs = ls.num_sms[dev & 63] / 2;
+  if (pairs > num_tiles) pairs = num_tiles;
+  return pairs < 1 ? 1 : (int)pairs;
 }
 
 __device__ __forceinline__ int warp_sum_int(int v) {
