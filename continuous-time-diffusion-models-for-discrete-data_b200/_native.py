@@ -16,6 +16,7 @@ BRANCH_TAULDR, BRANCH_SDDM_DIRECT, BRANCH_SDDM_REVERSE_PROB, BRANCH_SDDM_REVERSE
 MODE_TAU_LEAP, MODE_TAU_LEAP_CORR, MODE_MIDPOINT_DRIFT, MODE_MIDPOINT_JUMP, MODE_EULER, MODE_EULER_CORR, MODE_RATES_ONLY, MODE_EXACT = range(8)
 IMPL_AUTO, IMPL_SIMT, IMPL_TC = 0, 1, 2
 HEAD_LOGITS, HEAD_LOGISTIC, HEAD_LOGISTIC_FIX = 0, 1, 2
+DTYPE_F32, DTYPE_BF16 = 0, 1
 STAT_CHANGED_BASE, STAT_NONZERO_JUMP, STAT_CHANGED_EVAL, STAT_ROWS_JUMPED, STAT_ROWS_MULTI = 0, 1, 2, 3, 4
 STAT_COUNT = 8
 LOSS_CTELBO, LOSS_CRM, LOSS_SDDM = 0, 1, 2
@@ -49,7 +50,13 @@ class StepParams(ctypes.Structure):
         ("x_out", c_void_p), ("rr_out", c_void_p), ("ratio_out", c_void_p),
         ("stats_out", c_void_p), ("workspace", c_void_p),
         ("head", c_int32), ("head_mu", c_void_p), ("head_log_scale", c_void_p), ("head_batch_stride", c_int64),
+        ("logits_dtype", c_int32),
     ]
+
+
+def logits_dtype_of(t) -> int:
+    """ctdd_step_params.logits_dtype of a logits tensor the step kernels read as they are (fp32, bf16)."""
+    return DTYPE_BF16 if t.dtype == torch.bfloat16 else DTYPE_F32
 
 
 class LossParams(ctypes.Structure):

@@ -41,6 +41,10 @@ extern "C" int ctdd_reverse_step(const ctdd_step_params* p, void* stream) {
   if (p->mode < CTDD_MODE_TAU_LEAP || p->mode > CTDD_MODE_EXACT) { set_error("ctdd_reverse_step: unknown mode %d", p->mode); return 2; }
   if (p->branch < CTDD_BRANCH_TAULDR || p->branch > CTDD_BRANCH_SDDM_REVERSE_LOGSCALE) { set_error("ctdd_reverse_step: unknown branch %d", p->branch); return 2; }
   if (p->head < CTDD_HEAD_LOGITS || p->head > CTDD_HEAD_LOGISTIC_FIX) { set_error("ctdd_reverse_step: unknown head %d", p->head); return 2; }
+  if (p->head == CTDD_HEAD_LOGITS && p->logits_dtype != CTDD_DTYPE_F32 && p->logits_dtype != CTDD_DTYPE_BF16) {
+    set_error("ctdd_reverse_step: unknown logits_dtype %d (CTDD_DTYPE_F32 = 0, CTDD_DTYPE_BF16 = 1)", p->logits_dtype);
+    return 2;
+  }
   if (p->head == CTDD_HEAD_LOGITS ? !p->logits : (!p->head_mu || !p->head_log_scale || p->head_batch_stride < p->D)) {
     set_error("ctdd_reverse_step: null logits (or head_mu / head_log_scale / head_batch_stride < D for a logistic head)");
     return 2;

@@ -2,6 +2,7 @@
 // The arithmetic here is restated op-for-op (fp32) in oracle/rng.py; keep the two in sync.
 #pragma once
 #include <cuda_runtime.h>
+#include <cuda_bf16.h>
 #include <stdint.h>
 #include <math.h>
 #include "../../include/ctdd.h"
@@ -87,6 +88,19 @@ __device__ __forceinline__ Philox4 philox_keyed(uint32_t c0, uint32_t c1, uint32
   }
   Philox4 o; o.w[0] = c0; o.w[1] = c1; o.w[2] = c2; o.w[3] = c3;
   return o;
+}
+
+// Logits of the reverse step are fp32 or bf16 (ctdd_step_params::logits_dtype).  Widening bf16 to fp32 is exact (the 16
+// bits are the upper half of the fp32 pattern), so a kernel that widens on load and then runs its fp32 code returns the
+// results of the same call on the widened logits bit for bit.
+__device__ __forceinline__ float ld_logit(const float* p) { return __ldg(p); }
+__device__ __forceinline__ float ld_logit(const __nv_bfloat16* p) {
+  return __uint_as_float((uint32_t)__ldg(reinterpret_cast<const unsigned short*>(p)) << 16);
+}
+// 4 consecutive bf16 (element 0 in the low half of w.x) -> fp32
+__device__ __forceinline__ void widen_bf16x4(uint2 w, float& v0, float& v1, float& v2, float& v3) {
+  v0 = __uint_as_float(w.x << 16); v1 = __uint_as_float(w.x & 0xFFFF0000u);
+  v2 = __uint_as_float(w.y << 16); v3 = __uint_as_float(w.y & 0xFFFF0000u);
 }
 #endif
 

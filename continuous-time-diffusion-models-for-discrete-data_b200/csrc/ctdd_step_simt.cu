@@ -28,7 +28,7 @@ struct StepArgs {
   int mode, branch, D, S, reject_multi;
   long long rows;        // N*D
   long long row_offset;  // multiple of 8
-  const float* logits;
+  const void* logits;    // fp32 or bf16 (the kernel's logits-type template argument)
   long long ld, batch_stride;
   const int* x_eval;
   const int* x_base;
@@ -97,9 +97,10 @@ __device__ __noinline__ int2 tau_leap_small(LamVec<S> lam, float tot, float v0, 
   return make_int2(jump, K);
 }
 
-__device__ __forceinline__ const float* logits_row(const StepArgs& a, long long r) {
+template <typename LT>
+__device__ __forceinline__ const LT* logits_row(const StepArgs& a, long long r) {
   const long long n = r / a.D, d = r - n * a.D;
-  return a.logits + n * a.batch_stride + d * a.ld;
+  return static_cast<const LT*>(a.logits) + n * a.batch_stride + d * a.ld;
 }
 
 __device__ __forceinline__ void flush_stats(const RowStats& st, unsigned long long* stats) {
@@ -145,7 +146,8 @@ constexpr int SMALL_MINB = 8;
 constexpr unsigned SMALL_GRIDCAP = 64u;   // CTAs per SM of the capped grid
 // LEAN: the launch has dense logits and no rr_out / ratio_out (the samplers' call): the strided-row loads and the
 // (predicated, but issued) rate stores drop out as well.
-template <int S, int MODE = -1, int BRANCH = -1, bool LEAN = false>
+// LT: element type of the logits, float or __nv_bfloat16 (widened on load; everything after the load is the fp32 code).
+template <int S, int MODE = -1, int BRANCH = -1, bool LEAN = false, typename LT = float>
 __global__ void __launch_bounds__(128, (LEAN && S == 2 && MODE == CTDD_MODE_TAU_LEAP) ? SMALL_MINB : 0) step_small_kernel(StepArgs a_in) {
   StepArgs a = a_in;
   if (MODE >= 0) a.mode = MODE;
@@ -191,23 +193,42 @@ __global__ void __launch_bounds__(128, (LEAN && S == 2 && MODE == CTDD_MODE_TAU_
     g += (long long)gridDim.x * blockDim.x;
     const int nr = (a.rows - r0) < 8 ? (int)(a.rows - r0) : 8;
     float lg[8][S];
-    const bool contiguous = (a.ld == S) && (a.batch_stride == (long long)a.D * S) && nr == 8;
+    // (bf16: the 16-byte loads also need a 16-byte aligned tensor; r0 * S * 2 is a multiple of 16)
+    const bool contiguous = (a.ld == S) && (a.batch_stride == (long long)a.D * S) && nr == 8 &&
+                            (sizeof(LT) == 4 || (reinterpret_cast<uintptr_t>(a.logits) & 15) == 0);
     if (contiguous) {
-      const float4* p = reinterpret_cast<const float4*>(a.logits + r0 * S);
-      float4 buf[2 * S];
+      if constexpr (sizeof(LT) == 2) {     // 8 rows of S bf16: S 16-byte loads
+        const uint4* p = reinterpret_cast<const uint4*>(static_cast<const LT*>(a.logits) + r0 * S);
+        uint4 buf[S];
 #pragma unroll
-      for (int i = 0; i < 2 * S; ++i) buf[i] = __ldg(p + i);
-      const float* f = reinterpret_cast<const float*>(buf);
+        for (int i = 0; i < S; ++i) buf[i] = __ldg(p + i);
+        float f[8 * S];
 #pragma unroll
-      for (int r = 0; r < 8; ++r)
+        for (int i = 0; i < S; ++i) {
+          widen_bf16x4(make_uint2(buf[i].x, buf[i].y), f[8 * i], f[8 * i + 1], f[8 * i + 2], f[8 * i + 3]);
+          widen_bf16x4(make_uint2(buf[i].z, buf[i].w), f[8 * i + 4], f[8 * i + 5], f[8 * i + 6], f[8 * i + 7]);
+        }
 #pragma unroll
-        for (int s = 0; s < S; ++s) lg[r][s] = f[r * S + s];
+        for (int r = 0; r < 8; ++r)
+#pragma unroll
+          for (int s = 0; s < S; ++s) lg[r][s] = f[r * S + s];
+      } else {
+        const float4* p = reinterpret_cast<const float4*>(static_cast<const LT*>(a.logits) + r0 * S);
+        float4 buf[2 * S];
+#pragma unroll
+        for (int i = 0; i < 2 * S; ++i) buf[i] = __ldg(p + i);
+        const float* f = reinterpret_cast<const float*>(buf);
+#pragma unroll
+        for (int r = 0; r < 8; ++r)
+#pragma unroll
+          for (int s = 0; s < S; ++s) lg[r][s] = f[r * S + s];
+      }
     } else {
 #pragma unroll
       for (int r = 0; r < 8; ++r) {
-        const float* p = LEAN ? a.logits + (r0 + (r < nr ? r : 0)) * S : logits_row(a, r0 + (r < nr ? r : 0));
+        const LT* p = LEAN ? static_cast<const LT*>(a.logits) + (r0 + (r < nr ? r : 0)) * S : logits_row<LT>(a, r0 + (r < nr ? r : 0));
 #pragma unroll
-        for (int s = 0; s < S; ++s) lg[r][s] = __ldg(p + s);
+        for (int s = 0; s < S; ++s) lg[r][s] = ld_logit(p + s);
       }
     }
     int xe[8], xb[8];
@@ -468,6 +489,8 @@ __global__ void __launch_bounds__(128, (LEAN && S == 2 && MODE == CTDD_MODE_TAU_
 // terms), small per-row scalars.
 constexpr int BLK_ROWS = 8;
 
+// LT: element type of the logits, float or __nv_bfloat16 (every logits load goes through ld_logit)
+template <typename LT = float>
 __global__ void __launch_bounds__(256) step_block_kernel(StepArgs a) {
   extern __shared__ float smem[];
   const int S = a.S;
@@ -487,21 +510,21 @@ __global__ void __launch_bounds__(256) step_block_kernel(StepArgs a) {
   __syncthreads();
   // 1. softmax statistics and operand rows: warp w handles rows w, w+nwarp, ...
   for (int r = warp; r < BLK_ROWS; r += nwarp) {
-    const float* lp = logits_row(a, r0 + (r < nr ? r : 0));
+    const LT* lp = logits_row<LT>(a, r0 + (r < nr ? r : 0));
     const int x = s_xe[r];
     float m = -INFINITY;
-    for (int k = lane; k < S; k += 32) m = fmaxf(m, __ldg(lp + k));
+    for (int k = lane; k < S; k += 32) m = fmaxf(m, ld_logit(lp + k));
     m = warp_max(m);
     float sum = 0.f;
-    for (int k = lane; k < S; k += 32) sum += expf(__ldg(lp + k) - m);
+    for (int k = lane; k < S; k += 32) sum += expf(ld_logit(lp + k) - m);
     sum = warp_sum(sum);
     if (lane == 0) s_lse[r] = m + logf(sum);
     for (int k = lane; k < S; k += 32) {
-      const float p = expf(__ldg(lp + k) - m) / sum;
+      const float p = expf(ld_logit(lp + k) - m) / sum;
       float v;
       if (a.mode == CTDD_MODE_EXACT) v = p;
       else if (a.branch == CTDD_BRANCH_TAULDR) v = p / (a.QT[(size_t)x * S + k] + a.eps);
-      else if (a.branch == CTDD_BRANCH_SDDM_REVERSE_LOGSCALE) v = __ldg(lp + k) - (m + logf(sum));  // log p
+      else if (a.branch == CTDD_BRANCH_SDDM_REVERSE_LOGSCALE) v = ld_logit(lp + k) - (m + logf(sum));  // log p
       else v = p;
       sA[r * S + k] = v;
     }
@@ -546,7 +569,7 @@ __global__ void __launch_bounds__(256) step_block_kernel(StepArgs a) {
     for (int r = 0; r < BLK_ROWS; ++r) {
       float v = acc[r];
       if (a.branch == CTDD_BRANCH_SDDM_REVERSE_PROB) v = logf(v + 1e-35f);
-      else if (a.branch == CTDD_BRANCH_SDDM_DIRECT) v = __ldg(logits_row(a, r0 + (r < nr ? r : 0)) + s) - s_lse[r];
+      else if (a.branch == CTDD_BRANCH_SDDM_DIRECT) v = ld_logit(logits_row<LT>(a, r0 + (r < nr ? r : 0)) + s) - s_lse[r];
       sT[r * S + s] = v;  // tauLDR: ratio; SDDM: ll
       if (a.branch != CTDD_BRANCH_TAULDR && s == s_xe[r]) s_llx[r] = v;
     }
@@ -634,6 +657,43 @@ __global__ void __launch_bounds__(256) step_block_kernel(StepArgs a) {
   flush_stats(st, a.stats);
 }
 
+// The small-S dispatch table, the same for both logits types.
+template <typename LT>
+void launch_step_small(const StepArgs& a, int S, bool lean, unsigned blocks, int threads, cudaStream_t st) {
+  switch (S) {
+    case 2:   // C1: S = 2, tau-leaping on the tauLDR branch
+      if (a.mode == CTDD_MODE_TAU_LEAP && a.branch == CTDD_BRANCH_TAULDR && lean)    // grid-stride instantiation
+        step_small_kernel<2, CTDD_MODE_TAU_LEAP, CTDD_BRANCH_TAULDR, true, LT>
+            <<<blocks > 148u * SMALL_GRIDCAP ? 148u * SMALL_GRIDCAP : blocks, threads, 0, st>>>(a);
+      else if (lean && a.branch == CTDD_BRANCH_TAULDR && a.mode == CTDD_MODE_TAU_LEAP_CORR)   // PCTauL's corrector step
+        step_small_kernel<2, CTDD_MODE_TAU_LEAP_CORR, CTDD_BRANCH_TAULDR, true, LT><<<blocks, threads, 0, st>>>(a);
+      else if (lean && a.branch == CTDD_BRANCH_TAULDR && a.mode == CTDD_MODE_EULER)
+        step_small_kernel<2, CTDD_MODE_EULER, CTDD_BRANCH_TAULDR, true, LT><<<blocks, threads, 0, st>>>(a);
+      else if (lean && a.branch == CTDD_BRANCH_TAULDR && a.mode == CTDD_MODE_EULER_CORR)
+        step_small_kernel<2, CTDD_MODE_EULER_CORR, CTDD_BRANCH_TAULDR, true, LT><<<blocks, threads, 0, st>>>(a);
+      else
+        step_small_kernel<2, -1, -1, false, LT><<<blocks, threads, 0, st>>>(a);
+      break;
+    case 3:   // C2: S = 3, Euler (LBJF) on the tauLDR branch
+      if (a.mode == CTDD_MODE_EULER && a.branch == CTDD_BRANCH_TAULDR && lean)
+        step_small_kernel<3, CTDD_MODE_EULER, CTDD_BRANCH_TAULDR, true, LT><<<blocks, threads, 0, st>>>(a);
+      else if (lean && a.branch == CTDD_BRANCH_TAULDR && a.mode == CTDD_MODE_EULER_CORR)      // LBJF's corrector step
+        step_small_kernel<3, CTDD_MODE_EULER_CORR, CTDD_BRANCH_TAULDR, true, LT><<<blocks, threads, 0, st>>>(a);
+      else if (lean && a.branch == CTDD_BRANCH_TAULDR && a.mode == CTDD_MODE_TAU_LEAP)
+        step_small_kernel<3, CTDD_MODE_TAU_LEAP, CTDD_BRANCH_TAULDR, true, LT><<<blocks, threads, 0, st>>>(a);
+      else if (lean && a.branch == CTDD_BRANCH_TAULDR && a.mode == CTDD_MODE_TAU_LEAP_CORR)
+        step_small_kernel<3, CTDD_MODE_TAU_LEAP_CORR, CTDD_BRANCH_TAULDR, true, LT><<<blocks, threads, 0, st>>>(a);
+      else
+        step_small_kernel<3, -1, -1, false, LT><<<blocks, threads, 0, st>>>(a);
+      break;
+    case 4: step_small_kernel<4, -1, -1, false, LT><<<blocks, threads, 0, st>>>(a); break;
+    case 5: step_small_kernel<5, -1, -1, false, LT><<<blocks, threads, 0, st>>>(a); break;
+    case 6: step_small_kernel<6, -1, -1, false, LT><<<blocks, threads, 0, st>>>(a); break;
+    case 7: step_small_kernel<7, -1, -1, false, LT><<<blocks, threads, 0, st>>>(a); break;
+    default: step_small_kernel<8, -1, -1, false, LT><<<blocks, threads, 0, st>>>(a); break;
+  }
+}
+
 int launch_step_simt(const ctdd_step_params* p, cudaStream_t st) {
   StepArgs a;
   a.mode = p->mode; a.branch = p->branch; a.D = p->D; a.S = p->S; a.reject_multi = p->reject_multi;
@@ -644,44 +704,15 @@ int launch_step_simt(const ctdd_step_params* p, cudaStream_t st) {
   a.x_out = p->x_out; a.rr_out = p->rr_out; a.ratio_out = p->ratio_out;
   a.stats = reinterpret_cast<unsigned long long*>(p->stats_out);
   philox_key_schedule(p->seed, a.pk);
+  const bool bf16 = p->logits_dtype == CTDD_DTYPE_BF16;
   const int S = p->S;
   if (S <= 8 && S >= 2) {
     const long long groups = (a.rows + 7) / 8;
     const int threads = 128;
     unsigned blocks = (unsigned)((groups + threads - 1) / threads);
     const bool lean = !a.rr_out && !a.ratio_out && a.ld == S && a.batch_stride == (long long)a.D * S;
-    switch (S) {
-      case 2:   // C1: S = 2, tau-leaping on the tauLDR branch
-        if (a.mode == CTDD_MODE_TAU_LEAP && a.branch == CTDD_BRANCH_TAULDR && lean)    // grid-stride instantiation
-          step_small_kernel<2, CTDD_MODE_TAU_LEAP, CTDD_BRANCH_TAULDR, true>
-              <<<blocks > 148u * SMALL_GRIDCAP ? 148u * SMALL_GRIDCAP : blocks, threads, 0, st>>>(a);
-        else if (lean && a.branch == CTDD_BRANCH_TAULDR && a.mode == CTDD_MODE_TAU_LEAP_CORR)   // PCTauL's corrector step
-          step_small_kernel<2, CTDD_MODE_TAU_LEAP_CORR, CTDD_BRANCH_TAULDR, true><<<blocks, threads, 0, st>>>(a);
-        else if (lean && a.branch == CTDD_BRANCH_TAULDR && a.mode == CTDD_MODE_EULER)
-          step_small_kernel<2, CTDD_MODE_EULER, CTDD_BRANCH_TAULDR, true><<<blocks, threads, 0, st>>>(a);
-        else if (lean && a.branch == CTDD_BRANCH_TAULDR && a.mode == CTDD_MODE_EULER_CORR)
-          step_small_kernel<2, CTDD_MODE_EULER_CORR, CTDD_BRANCH_TAULDR, true><<<blocks, threads, 0, st>>>(a);
-        else
-          step_small_kernel<2><<<blocks, threads, 0, st>>>(a);
-        break;
-      case 3:   // C2: S = 3, Euler (LBJF) on the tauLDR branch
-        if (a.mode == CTDD_MODE_EULER && a.branch == CTDD_BRANCH_TAULDR && lean)
-          step_small_kernel<3, CTDD_MODE_EULER, CTDD_BRANCH_TAULDR, true><<<blocks, threads, 0, st>>>(a);
-        else if (lean && a.branch == CTDD_BRANCH_TAULDR && a.mode == CTDD_MODE_EULER_CORR)      // LBJF's corrector step
-          step_small_kernel<3, CTDD_MODE_EULER_CORR, CTDD_BRANCH_TAULDR, true><<<blocks, threads, 0, st>>>(a);
-        else if (lean && a.branch == CTDD_BRANCH_TAULDR && a.mode == CTDD_MODE_TAU_LEAP)
-          step_small_kernel<3, CTDD_MODE_TAU_LEAP, CTDD_BRANCH_TAULDR, true><<<blocks, threads, 0, st>>>(a);
-        else if (lean && a.branch == CTDD_BRANCH_TAULDR && a.mode == CTDD_MODE_TAU_LEAP_CORR)
-          step_small_kernel<3, CTDD_MODE_TAU_LEAP_CORR, CTDD_BRANCH_TAULDR, true><<<blocks, threads, 0, st>>>(a);
-        else
-          step_small_kernel<3><<<blocks, threads, 0, st>>>(a);
-        break;
-      case 4: step_small_kernel<4><<<blocks, threads, 0, st>>>(a); break;
-      case 5: step_small_kernel<5><<<blocks, threads, 0, st>>>(a); break;
-      case 6: step_small_kernel<6><<<blocks, threads, 0, st>>>(a); break;
-      case 7: step_small_kernel<7><<<blocks, threads, 0, st>>>(a); break;
-      default: step_small_kernel<8><<<blocks, threads, 0, st>>>(a); break;
-    }
+    if (bf16) launch_step_small<__nv_bfloat16>(a, S, lean, blocks, threads, st);
+    else launch_step_small<float>(a, S, lean, blocks, threads, st);
     CTDD_CHECK_LAUNCH("step_small_kernel");
     return 0;
   }
@@ -691,14 +722,16 @@ int launch_step_simt(const ctdd_step_params* p, cudaStream_t st) {
   int dev = 0;
   cudaGetDevice(&dev);
   if (dev < 0 || dev >= 64 || !((attr_done >> dev) & 1ull)) {
-    cudaFuncSetAttribute(step_block_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    cudaFuncSetAttribute(step_block_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    cudaFuncSetAttribute(step_block_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
     if (dev >= 0 && dev < 64) attr_done |= 1ull << dev;
   }
   int threads = ((S + 31) / 32) * 32;
   if (threads > 256) threads = 256;
   if (threads < 64) threads = 64;
   const unsigned blocks = (unsigned)((a.rows + BLK_ROWS - 1) / BLK_ROWS);
-  step_block_kernel<<<blocks, threads, smem, st>>>(a);
+  if (bf16) step_block_kernel<__nv_bfloat16><<<blocks, threads, smem, st>>>(a);
+  else step_block_kernel<float><<<blocks, threads, smem, st>>>(a);
   CTDD_CHECK_LAUNCH("step_block_kernel");
   return 0;
 }

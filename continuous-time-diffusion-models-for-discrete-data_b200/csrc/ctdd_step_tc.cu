@@ -9,7 +9,7 @@
 //   * M side = state s. Each CTA keeps ITS 128-state half of Q^T (bf16 hi + mid split, 2 x 128 TMEM columns)
 //     resident in tensor memory as the A operand (TS form) for the whole kernel; 4 accumulators of 64 columns.
 //   * N side = data rows. Each CTA's 8 producer warps build 32 of the tile's 64 rows, two rows per pass with 16 lanes
-//     per row: raw fp32 logits arrive through a per-warp smem ring filled by cp.async.bulk (HBM -> L2 prefetch eight
+//     per row: raw fp32 or bf16 logits arrive through a per-warp smem ring filled by cp.async.bulk (HBM -> L2 prefetch eight
 //     tiles ahead), row softmax by half-warp butterflies, gathered reciprocal denominators 1/(Q[k,x]+eps), bf16 hi/mid
 //     split, K-major 128B-swizzled smem stage.  Every row is produced exactly once.
 //   * Count warp (lane = row): the row's Euler uniform (Philox, STREAM_ROW).
@@ -67,7 +67,8 @@ struct Smem {
   alignas(1024) uint8_t stage[STAGES][STAGE_BYTES];
   alignas(16) float gather[GBUF][NH][S];   // [row owned by this CTA][state]: accumulator values, then prefix sums
   Side side[RING][NH];
-  alignas(16) float lring[NUM_PROD_WARPS][LRING][2][S];   // raw fp32 logits rows, one pass ahead of their use
+  alignas(16) float lring[NUM_PROD_WARPS][LRING][2][S];   // raw logits rows, one pass ahead of their use (bf16: the
+                                                          // row pair packed into the first half of the slot)
   alignas(8) uint64_t full[STAGES];  // leader CTA: its 8 producer warps + 1 relayed arrival for the partner's 8
   uint64_t full_local[STAGES];       // partner CTA: its 8 producer warps; the partner's idle MMA warp relays the phase
   uint64_t empty[STAGES];            // multicast tcgen05.commit
@@ -102,9 +103,13 @@ __device__ __forceinline__ int prefix_search(uint32_t P, float T) {
 
 // ---------------------------------------------------------------------------------------------- the kernel
 // TAULDR: tauLDR rates (else SDDM reverse_prob); CORR: the corrector variant adds h * R_t[x,:] to the rates;
-// HEAD: the rows' softmax numerators come from the truncated-logistic head (mu, log_scale per row) instead of logits
-template <bool TAULDR, bool CORR, bool HEAD>
+// HEAD: the rows' softmax numerators come from the truncated-logistic head (mu, log_scale per row) instead of logits;
+// LT: element type of the logits, float or __nv_bfloat16 (a bf16 row pair travels packed, 2*S bytes per row, and is
+// widened on the producers' shared-memory load; the arithmetic after that load is the fp32 kernel's)
+template <bool TAULDR, bool CORR, bool HEAD, typename LT = float>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step_tc_kernel(const Args a) {
+  static_assert(!HEAD || sizeof(LT) == 4, "the head kernels read no logits");
+  constexpr uint32_t ROW_BYTES = S * sizeof(LT);
   extern __shared__ uint8_t smem_raw[];
   // aligned by offsetting the shared array itself (not through an integer): the compiler keeps `sm` a shared-space
   // pointer, so its accesses are 32-bit LDS/STS and no 64-bit generic base stays live (that base was spilled at 96 registers)
@@ -158,10 +163,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
     constexpr int PASSES = ROWS_PER_PROD / 2;                    // passes per tile; warp pw builds rows ROWS_PER_PROD*pw ..
     const int npass = my_tiles * PASSES;
 
-    auto row_ptr = [&](long long g) -> const float* {
-      if (contiguous) return a.logits + g * S;
+    const LT* const logits = static_cast<const LT*>(a.logits);
+    auto row_ptr = [&](long long g) -> const LT* {
+      if (contiguous) return logits + g * S;
       const uint32_t n = (uint32_t)g / (uint32_t)a.D, d = (uint32_t)g - n * (uint32_t)a.D;
-      return a.logits + (long long)n * a.batch_stride + (long long)d * a.ld;
+      return logits + (long long)n * a.batch_stride + (long long)d * a.ld;
     };
     // Running state of the fetch stream (two passes ahead of the compute stream): first row of the pair, pass-in-tile,
     // ring slot.  Everything advances by additions only - no index arithmetic on the warp's critical path.
@@ -188,21 +194,22 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
           }
         } else if (lane == 0) {
           uint64_t* bar = &sm.lring_full[pw][f_slot];
-          mbar_arrive_expect_tx(bar, 2 * S * 4);
+          mbar_arrive_expect_tx(bar, 2 * ROW_BYTES);
+          uint8_t* const dst = reinterpret_cast<uint8_t*>(&sm.lring[pw][f_slot][0][0]);   // row hf of the pair at hf * ROW_BYTES
           if (contiguous && gf + 1 < a.rows) {
-            bulk_g2s(&sm.lring[pw][f_slot][0][0], a.logits + gf * S, 2 * S * 4, bar);
+            bulk_g2s(dst, logits + gf * S, 2 * ROW_BYTES, bar);
           } else {
 #pragma unroll
             for (int hf = 0; hf < 2; ++hf) {
               const long long gg = (gf + hf < a.rows) ? gf + hf : 0;
-              bulk_g2s(&sm.lring[pw][f_slot][hf][0], row_ptr(gg), S * 4, bar);
+              bulk_g2s(dst + hf * ROW_BYTES, row_ptr(gg), ROW_BYTES, bar);
             }
           }
         }
         if (gf + half < a.rows) xv = __ldg(a.x_eval + gf + half);
         if (!HEAD && contiguous && f_ps == 0 && lane == 0) {   // pull this warp's 4 rows of a later tile from HBM into L2
           const long long r0 = gf + (long long)PREFETCH_TILES * npairs * NT;
-          if (r0 + ROWS_PER_PROD <= a.rows) l2_prefetch_bulk(a.logits + r0 * S, ROWS_PER_PROD * S * 4);
+          if (r0 + ROWS_PER_PROD <= a.rows) l2_prefetch_bulk(logits + r0 * S, ROWS_PER_PROD * ROW_BYTES);
         }
         --f_left;
         f_slot = (f_slot + 1 == LRING) ? 0 : f_slot + 1;
@@ -268,11 +275,18 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
         }
         head_numerators(mu_cur, ls_cur, a.head_fix != 0, l16, v);
       } else {
-        const uint32_t src = smem_u32(&sm.lring[pw][rslot][half][4 * l16]);
+        if constexpr (sizeof(LT) == 2) {
+          // lane l16 widens the same elements 64c + 4*l16 .. +3 as in the fp32 kernel, one 64-bit load each
+          const uint32_t src = smem_u32(&sm.lring[pw][rslot][0][0]) + half * ROW_BYTES + 8 * l16;
 #pragma unroll
-        for (int c = 0; c < 4; ++c) {
-          const float4 q4 = lds128(src + 256 * c);
-          v[4 * c] = q4.x; v[4 * c + 1] = q4.y; v[4 * c + 2] = q4.z; v[4 * c + 3] = q4.w;
+          for (int c = 0; c < 4; ++c) widen_bf16x4(lds64(src + 128 * c), v[4 * c], v[4 * c + 1], v[4 * c + 2], v[4 * c + 3]);
+        } else {
+          const uint32_t src = smem_u32(&sm.lring[pw][rslot][half][4 * l16]);
+#pragma unroll
+          for (int c = 0; c < 4; ++c) {
+            const float4 q4 = lds128(src + 256 * c);
+            v[4 * c] = q4.x; v[4 * c + 1] = q4.y; v[4 * c + 2] = q4.z; v[4 * c + 3] = q4.w;
+          }
         }
         float m4[4];
 #pragma unroll
@@ -642,8 +656,10 @@ bool tc_supports(const ctdd_step_params* p) {
         p->mode == CTDD_MODE_RATES_ONLY))
     return false;
   if (!p->tc_tables || !p->tc_static) return false;
+  // rows are bulk-copied: 16-byte aligned (4 fp32 or 8 bf16 elements)
+  const int64_t row_align = p->logits_dtype == CTDD_DTYPE_BF16 ? 7 : 3;
   if (p->head == CTDD_HEAD_LOGITS &&
-      ((p->ld_logits & 3) || (p->batch_stride_logits & 3) || (reinterpret_cast<uintptr_t>(p->logits) & 15)))
+      ((p->ld_logits & row_align) || (p->batch_stride_logits & row_align) || (reinterpret_cast<uintptr_t>(p->logits) & 15)))
     return false;
   if (p->mode == CTDD_MODE_RATES_ONLY &&
       ((reinterpret_cast<uintptr_t>(p->rr_out) & 15) || (reinterpret_cast<uintptr_t>(p->ratio_out) & 15)))
@@ -663,15 +679,18 @@ int launch_step_tc(const ctdd_step_params* p, cudaStream_t st) {
   static PairLaunchState launch_state;
   const size_t smem_bytes = sizeof(Smem) + 1024;
   typedef void (*kern_t)(const Args);
-#define CTDD_TC_ROW(T, H) step_tc_kernel<T, false, H>, step_tc_kernel<T, true, H>
-  static const kern_t kerns[8] = {CTDD_TC_ROW(false, false), CTDD_TC_ROW(true, false), CTDD_TC_ROW(false, true),
-                                     CTDD_TC_ROW(true, true)};
+#define CTDD_TC_ROW(T, H, LT) step_tc_kernel<T, false, H, LT>, step_tc_kernel<T, true, H, LT>
+  static const kern_t kerns[12] = {CTDD_TC_ROW(false, false, float), CTDD_TC_ROW(true, false, float),
+                                     CTDD_TC_ROW(false, true, float), CTDD_TC_ROW(true, true, float),
+                                     CTDD_TC_ROW(false, false, __nv_bfloat16), CTDD_TC_ROW(true, false, __nv_bfloat16)};
 #undef CTDD_TC_ROW
   Args a = make_args(p);
   a.num_tiles = (int)((a.rows + NT - 1) / NT);
   const int pairs = pair_count(launch_state, "ctdd_reverse_step", kerns, smem_bytes, a.num_tiles);
   if (!pairs) return 1;
-  const int ki = ((p->branch == CTDD_BRANCH_TAULDR) ? 1 : 0) + (p->head != CTDD_HEAD_LOGITS ? 2 : 0);
+  // rows of kerns: fp32 logits, fused head, bf16 logits
+  const int ki = ((p->branch == CTDD_BRANCH_TAULDR) ? 1 : 0) +
+                 (p->head != CTDD_HEAD_LOGITS ? 2 : (p->logits_dtype == CTDD_DTYPE_BF16 ? 4 : 0));
   const int kj = (p->mode == CTDD_MODE_EULER_CORR) ? 1 : 0;
   kerns[2 * ki + kj]<<<2 * pairs, NUM_THREADS, smem_bytes, st>>>(a);
   CTDD_CHECK_LAUNCH("step_tc_kernel");

@@ -9,7 +9,7 @@
 //     in tensor memory as the A operand (TS form) for the whole kernel; 2 accumulators of 128 columns.  With N = 128
 //     an instruction sits on the 64-cycle floor of the TS form (the A slice is read from tensor memory at 64 B/cycle).
 //   * N side = data rows; each CTA produces 64 rows of a tile.  Producer warps work on two rows per pass, 16 lanes per
-//     row: raw fp32 logits from a per-warp ring of two 2 KB slots, row softmax by half-warp butterflies, gathered reciprocal
+//     row: raw fp32 or bf16 logits from a per-warp ring of two 2 KB slots, row softmax by half-warp butterflies, gathered reciprocal
 //     denominators 1/(Q[k,x]+eps), bf16 hi/mid split, K-major 128B-swizzled smem stage.  The passes of a tile are dealt
 //     round-robin to the producer warps; one pass counter per warp, every position derives from it.
 //   * A loader warp issues what the producers would otherwise stall on: per GROUP of 4 producer warps (one per SM
@@ -81,7 +81,8 @@ constexpr uint32_t CONTRIB_TX_BYTES = (NUM_EPI_WARPS / 2) * 2 * 32 * 4;   // rec
 
 struct Smem {
   alignas(1024) uint8_t stage[STAGES][STAGE_BYTES];
-  alignas(16) float lring[LRING][NPW][2][S];   // raw fp32 logits rows, LRING passes of every producer warp ahead of their use
+  alignas(16) float lring[LRING][NPW][2][S];   // raw logits rows, LRING passes of every producer warp ahead of their use
+                                               // (bf16: a round's 8 rows packed into the first half of its group's slots)
   alignas(16) float2 scal_c[RING][NT];         // (c1, c0) of the tile's rows: rows 0..63 from CTA 0, 64..127 from CTA 1
   uint32_t scal_x[RING][NT];                   // chunk mask of the band (bits 0-7) | valid << 8 | x << 10 (= table-row byte offset)
   alignas(16) float scratch[NUM_EPI_WARPS][32][SCR_LD];   // per epilogue warp: lam[row][state of the chunk] (lane = state -> lane = row)
@@ -107,9 +108,13 @@ static_assert(NPW <= PASSES_PER_TILE, "every producer warp must own a pass in ev
 static_assert(RING > STAGES + ACC + CBUF, "row-scalar ring shorter than the pipeline");
 
 // TAULDR: tauLDR rates (else SDDM reverse_prob); KM: KM_JUMP / KM_CORR / KM_RATES / KM_DRIFT;
-// HEAD: the rows' softmax numerators come from the truncated-logistic head (mu, log_scale per row) instead of logits
-template <bool TAULDR, int KM, bool HEAD>
+// HEAD: the rows' softmax numerators come from the truncated-logistic head (mu, log_scale per row) instead of logits;
+// LT: element type of the logits, float or __nv_bfloat16 (bf16 rows travel packed, 2*S bytes each, and are widened on
+// the producers' shared-memory load; the arithmetic after that load is the fp32 kernel's)
+template <bool TAULDR, int KM, bool HEAD, typename LT = float>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step_q_kernel(const Args a) {
+  static_assert(!HEAD || sizeof(LT) == 4, "the head kernels read no logits");
+  constexpr uint32_t ROW_BYTES = S * sizeof(LT);
   extern __shared__ uint8_t smem_raw[];
   Smem& sm = *reinterpret_cast<Smem*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -254,11 +259,20 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
         const HeadRec hr = {h0.x, h0.y, h0.z, h0.w, h1.x, h1.y, h1.z, h1.w};
         head_numerators_rec(hr, a.head_fix != 0, l16, v);
       } else {
-        const uint32_t src = smem_u32(&sm.lring[rslot][pw][half][4 * l16]);
+        if constexpr (sizeof(LT) == 2) {
+          // the round's 8 bf16 rows lie packed from the group's first slot: this half's row is number 2 * (pw % GSZ) + half;
+          // lane l16 widens the same elements 64c + 4*l16 .. +3 as in the fp32 kernel, one 64-bit load each
+          const uint32_t src = smem_u32(&sm.lring[rslot][pw - pw % GSZ][0][0]) + (uint32_t)(2 * (pw % GSZ) + half) * ROW_BYTES +
+                               8 * l16;
 #pragma unroll
-        for (int c = 0; c < 4; ++c) {
-          const float4 q4 = lds128(src + 256 * c);
-          v[4 * c] = q4.x; v[4 * c + 1] = q4.y; v[4 * c + 2] = q4.z; v[4 * c + 3] = q4.w;
+          for (int c = 0; c < 4; ++c) widen_bf16x4(lds64(src + 128 * c), v[4 * c], v[4 * c + 1], v[4 * c + 2], v[4 * c + 3]);
+        } else {
+          const uint32_t src = smem_u32(&sm.lring[rslot][pw][half][4 * l16]);
+#pragma unroll
+          for (int c = 0; c < 4; ++c) {
+            const float4 q4 = lds128(src + 256 * c);
+            v[4 * c] = q4.x; v[4 * c + 1] = q4.y; v[4 * c + 2] = q4.z; v[4 * c + 3] = q4.w;
+          }
         }
         ++ring_n;
         __syncwarp();            // every lane has its values: the group's slots may be refilled once its 4 warps say so
@@ -350,10 +364,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
     // two DSMEM bulk copies.  Nobody blocks: the warp polls, every lane acts on what is ready.
     {
       const bool contiguous = (a.ld == S) && (a.batch_stride == (long long)a.D * S);
-      auto row_ptr = [&](long long g) -> const float* {
-        if (contiguous) return a.logits + g * S;
+      const LT* const logits = static_cast<const LT*>(a.logits);
+      auto row_ptr = [&](long long g) -> const LT* {
+        if (contiguous) return logits + g * S;
         const uint32_t n = (uint32_t)g / (uint32_t)a.D, d = (uint32_t)g - n * (uint32_t)a.D;
-        return a.logits + (long long)n * a.batch_stride + (long long)d * a.ld;
+        return logits + (long long)n * a.batch_stride + (long long)d * a.ld;
       };
       const uint32_t scal_c_p = smem_u32(&sm.scal_c[0][rank * NH]), scal_x_p = smem_u32(&sm.scal_x[0][rank * NH]);
       const uint32_t scal_c_remote = mapa(scal_c_p, rank ^ 1u), scal_x_remote = mapa(scal_x_p, rank ^ 1u);
@@ -421,12 +436,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
           const long long rA = row00 + (long long)(P0 >> 5) * tile_rows + 2 * (P0 & 31);
           const long long nA = seg_rows(rA);
           uint64_t* gbar = &sm.lring_full_g[gslot][lane];
-          mbar_arrive_expect_tx(gbar, (uint32_t)nA * S * 4);
-          float* dA = &sm.lring[gslot][GSZ * lane][0][0];
+          mbar_arrive_expect_tx(gbar, (uint32_t)nA * ROW_BYTES);
+          uint8_t* dA = reinterpret_cast<uint8_t*>(&sm.lring[gslot][GSZ * lane][0][0]);   // row rr of the round at rr * ROW_BYTES
           if (contiguous) {
-            if (nA > 0) bulk_g2s(dA, a.logits + rA * S, (uint32_t)nA * S * 4, gbar);
+            if (nA > 0) bulk_g2s(dA, logits + rA * S, (uint32_t)nA * ROW_BYTES, gbar);
           } else {               // strided logits: one copy per row
-            for (long long rr = 0; rr < nA; ++rr) bulk_g2s(dA + rr * S, row_ptr(rA + rr), S * 4, gbar);
+            for (long long rr = 0; rr < nA; ++rr) bulk_g2s(dA + rr * ROW_BYTES, row_ptr(rA + rr), ROW_BYTES, gbar);
           }
           ++grp;
           did = true;
@@ -808,11 +823,12 @@ int launch_step_tcq(const ctdd_step_params* p, cudaStream_t st) {
   static tc::PairLaunchState launch_state;
   const size_t smem_bytes = sizeof(Smem) + 1024;
   typedef void (*kern_t)(const tc::Args);
-#define CTDD_TCQ_ROW(T, H)                                                                                        \
-  step_q_kernel<T, tc::KM_JUMP, H>, step_q_kernel<T, tc::KM_CORR, H>, step_q_kernel<T, tc::KM_RATES, H>,        \
-      step_q_kernel<T, tc::KM_DRIFT, H>
-  static const kern_t kerns[16] = {CTDD_TCQ_ROW(false, false), CTDD_TCQ_ROW(true, false), CTDD_TCQ_ROW(false, true),
-                                     CTDD_TCQ_ROW(true, true)};
+#define CTDD_TCQ_ROW(T, H, LT)                                                                                            \
+  step_q_kernel<T, tc::KM_JUMP, H, LT>, step_q_kernel<T, tc::KM_CORR, H, LT>, step_q_kernel<T, tc::KM_RATES, H, LT>,    \
+      step_q_kernel<T, tc::KM_DRIFT, H, LT>
+  static const kern_t kerns[24] = {CTDD_TCQ_ROW(false, false, float), CTDD_TCQ_ROW(true, false, float),
+                                     CTDD_TCQ_ROW(false, true, float), CTDD_TCQ_ROW(true, true, float),
+                                     CTDD_TCQ_ROW(false, false, __nv_bfloat16), CTDD_TCQ_ROW(true, false, __nv_bfloat16)};
 #undef CTDD_TCQ_ROW
   if (reinterpret_cast<uintptr_t>(p->tc_static) % tc::ST_ALIGN) {
     set_error("ctdd_reverse_step: tc_static must be aligned to ctdd_tc_static_align() = %zu bytes", tc::ST_ALIGN);
@@ -826,7 +842,9 @@ int launch_step_tcq(const ctdd_step_params* p, cudaStream_t st) {
   a.num_tiles = (int)((a.rows + NT - 1) / NT);
   const int pairs = tc::pair_count(launch_state, "ctdd_reverse_step", kerns, smem_bytes, a.num_tiles);
   if (!pairs) return 1;
-  const int ki = ((p->branch == CTDD_BRANCH_TAULDR) ? 1 : 0) + (p->head != CTDD_HEAD_LOGITS ? 2 : 0);
+  // rows of kerns: fp32 logits, fused head, bf16 logits
+  const int ki = ((p->branch == CTDD_BRANCH_TAULDR) ? 1 : 0) +
+                 (p->head != CTDD_HEAD_LOGITS ? 2 : (p->logits_dtype == CTDD_DTYPE_BF16 ? 4 : 0));
   int kj = 0;
   if (p->mode == CTDD_MODE_RATES_ONLY) kj = 2;
   else if (p->mode == CTDD_MODE_TAU_LEAP_CORR) kj = 1;

@@ -39,7 +39,7 @@ __host__ __device__ constexpr bool km_corr(int km) { return km == KM_CORR; }
 struct Args {
   int branch, D, reject_multi;
   long long rows, row_offset;
-  const float* logits;
+  const void* logits;        // fp32 or bf16 (the kernel's logits-type template argument)
   long long ld, batch_stride;
   const int* x_eval;
   const int* x_base;
@@ -235,6 +235,11 @@ __device__ __forceinline__ void ldg256_pred(const uint8_t* p, float* v, bool on)
 __device__ __forceinline__ float4 lds128(uint32_t addr) {
   float4 v;
   asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(addr));
+  return v;
+}
+__device__ __forceinline__ uint2 lds64(uint32_t addr) {
+  uint2 v;
+  asm volatile("ld.shared.v2.b32 {%0, %1}, [%2];" : "=r"(v.x), "=r"(v.y) : "r"(addr));
   return v;
 }
 __device__ __forceinline__ float lds32(uint32_t addr) {

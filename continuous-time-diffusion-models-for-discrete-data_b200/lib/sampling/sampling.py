@@ -96,7 +96,7 @@ class StepEngine:
         return self._t_all[tidx]
 
     def _fast_step(self, mode, logits, x_eval, tidx, h, reject_multi, x_base, row):
-        """The common case of step(): dense contiguous fp32 logits or an un-materialised head, state update only."""
+        """The common case of step(): dense contiguous fp32 / bf16 logits or an un-materialised head, state update only."""
         N, D, S = self.N, self.D, self.S
         p = self._p
         if isinstance(logits, ops.LogisticHead):
@@ -107,6 +107,8 @@ class StepEngine:
         else:
             p.head, p.head_mu, p.head_log_scale, p.head_batch_stride = nat.HEAD_LOGITS, None, None, 0
             p.logits = logits.data_ptr()
+            # the struct is reused across calls, whose logits may alternate between fp32 and bf16
+            p.logits_dtype = nat.logits_dtype_of(logits)
         xe = x_eval.data_ptr()
         xb = x_base.data_ptr() if x_base is not None else 0
         k = 0
@@ -146,7 +148,8 @@ class StepEngine:
                 and (x_base is None or (x_base.dtype == torch.int32 and x_base.is_contiguous()))
                 and torch.cuda.current_device() == (self.device.index or 0)
                 and ((head is not None and self.tc_tables is not None)
-                     or (head is None and logits.dtype == torch.float32 and logits.is_contiguous() and logits.is_cuda)))
+                     or (head is None and logits.dtype in (torch.float32, torch.bfloat16) and logits.is_contiguous()
+                         and logits.is_cuda)))
         if fast:
             x_out = self._fast_step(mode, ops.LogisticHead(*head) if head is not None else logits, x_eval, tidx, h,
                                     reject_multi, x_base, row)
@@ -199,7 +202,7 @@ def _dense(logits, S):
 
 def _final_argmax(model, x, min_t, N, device):
     out = model(x.long(), min_t * torch.ones((N,), device=device))
-    p_0gt = F.softmax(_dense(out, getattr(model, "S", None)), dim=2)
+    p_0gt = F.softmax(_dense(out, getattr(model, "S", None)), dim=2, dtype=torch.float32)   # bf16 logits: fp32 ties as for fp32
     return torch.max(p_0gt, dim=2)[1]
 
 
@@ -465,7 +468,7 @@ class ConditionalTauLeaping(_SamplerBase):
                 full = model(torch.concat((conditioner, x.long()), dim=1), eng.t_ones(idx))
                 x, _ = eng.step(nat.MODE_TAU_LEAP, full, x, idx, h, False, logits_view=(full, condition_dim))
             full = model(torch.concat((conditioner, x.long()), dim=1), scfg.min_t * torch.ones((N,), device=device))
-            x_0max = torch.max(F.softmax(_dense(full, S), dim=2)[:, condition_dim:, :], dim=2)[1]
+            x_0max = torch.max(F.softmax(_dense(full, S), dim=2, dtype=torch.float32)[:, condition_dim:, :], dim=2)[1]
             output = torch.concat((conditioner, x_0max), dim=1)
             return output.detach().cpu().numpy().astype(int)
 
@@ -492,7 +495,7 @@ class ConditionalPCTauLeaping(_SamplerBase):
                             reject=bool(scfg.reject_multiple_jumps), init_std=init_std, seed=self.seed,
                             row_offset=self.row_offset, impl=self.impl)
             full = model(torch.concat((conditioner, x.long()), dim=1), scfg.min_t * torch.ones((N,), device=device))
-            x_0max = torch.max(F.softmax(_dense(full, S), dim=2)[:, condition_dim:, :], dim=2)[1]
+            x_0max = torch.max(F.softmax(_dense(full, S), dim=2, dtype=torch.float32)[:, condition_dim:, :], dim=2)[1]
             output = torch.concat((conditioner, x_0max), dim=1)
             return output.detach().cpu().numpy().astype(int)
 

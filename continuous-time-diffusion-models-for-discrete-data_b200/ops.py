@@ -75,7 +75,7 @@ def reverse_step(mode, branch, logits, x_eval, Q, QT, Rb, RbT, beta, h, eps, *, 
         else:
             logits = logistic_logits(mu, ls, S, fix)
     if logits is not None:
-        if logits.dtype != torch.float32:
+        if logits.dtype not in (torch.float32, torch.bfloat16):     # bf16 is read as it is (widened on load, exactly)
             logits = logits.float()
         logits = logits.contiguous()
     if mode == nat.MODE_RATES_ONLY:
@@ -91,7 +91,7 @@ def reverse_step(mode, branch, logits, x_eval, Q, QT, Rb, RbT, beta, h, eps, *, 
         workspace = torch.empty((ws,), dtype=torch.uint8, device=dev) if ws > 0 else None
     p = nat.StepParams(
         mode=mode, branch=branch, impl=impl, N=N, D=D, S=S, row_offset=int(row_offset),
-        logits=(nat.ptr(logits) + 4 * int(logits_offset_elems)) if logits is not None else None, ld_logits=S,
+        logits=(nat.ptr(logits) + logits.element_size() * int(logits_offset_elems)) if logits is not None else None, ld_logits=S,
         batch_stride_logits=(int(batch_stride) if batch_stride is not None else D * S),
         x_eval=nat.ptr(x_eval), x_base=nat.ptr(x_base),
         Q=nat.ptr(Q), QT=nat.ptr(QT), Rb=nat.ptr(Rb), RbT=nat.ptr(RbT), tc_tables=nat.ptr(tc_tables), tc_static=nat.ptr(tc_static),
@@ -100,7 +100,8 @@ def reverse_step(mode, branch, logits, x_eval, Q, QT, Rb, RbT, beta, h, eps, *, 
         x_out=nat.ptr(x_out), rr_out=nat.ptr(rr), ratio_out=nat.ptr(ratio),
         stats_out=(stats.data_ptr() if stats is not None else None), workspace=nat.ptr(workspace),
         head=head_kind, head_mu=(head_mu.data_ptr() if head_mu is not None else None),
-        head_log_scale=(head_ls.data_ptr() if head_ls is not None else None), head_batch_stride=int(head_bs))
+        head_log_scale=(head_ls.data_ptr() if head_ls is not None else None), head_batch_stride=int(head_bs),
+        logits_dtype=(nat.logits_dtype_of(logits) if logits is not None else nat.DTYPE_F32))
     nat.check(nat.lib().ctdd_reverse_step(p, nat.stream()), "ctdd_reverse_step")
     return {"x": x_out, "rr": rr, "ratio": ratio}
 

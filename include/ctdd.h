@@ -109,9 +109,9 @@ typedef struct ctdd_step_params {
   int32_t impl;          /* CTDD_IMPL_* */
   int32_t N, D, S;
   int64_t row_offset;    /* global index of row 0 (batch sharding across GPUs) */
-  const float* logits;   /* [N*D rows][S], row r at logits + r*ld_logits (elements) */
-  int64_t ld_logits;     /* >= S; lets a caller pass model output sliced as [:, cond:, :] */
-  int64_t batch_stride_logits; /* elements between consecutive n (= D_total*ld_logits for a sliced view, else D*ld_logits) */
+  const void* logits;    /* [N*D rows][S] of logits_dtype, row r at logits + r*ld_logits (elements) */
+  int64_t ld_logits;     /* >= S, in elements of logits_dtype; lets a caller pass model output sliced as [:, cond:, :] */
+  int64_t batch_stride_logits; /* elements of logits_dtype between consecutive n (= D_total*ld_logits for a sliced view, else D*ld_logits) */
   const int32_t* x_eval; /* [N*D] state the logits/rates were evaluated at */
   const int32_t* x_base; /* [N*D] state the jump is added to; NULL -> x_eval (only MIDPOINT_JUMP differs) */
   const float* Q;        /* [S,S] q_{t|0} at this step's time */
@@ -140,7 +140,20 @@ typedef struct ctdd_step_params {
   const float* head_mu;         /* row (n,d) at head_mu[n*head_batch_stride + d] */
   const float* head_log_scale;  /* same addressing */
   int64_t head_batch_stride;    /* elements between consecutive n (2*D for the two halves of a torch.chunk'ed (B,2C,H,W)) */
+  /* Element type of `logits` (appended field; zero-initialised = fp32).  CTDD_DTYPE_BF16 takes the logits a network run
+   * under torch.autocast(dtype=torch.bfloat16) emits without a widening copy: the kernels widen on load (exact) and then
+   * run the fp32 arithmetic, so the states, counters, rr_out and ratio_out equal those of the same call on the widened
+   * logits bit for bit.  The outputs stay fp32 / int32.  The tcgen05 path (S == 256) needs 16-byte aligned rows:
+   * logits 16-byte aligned, ld_logits and batch_stride_logits multiples of 8 bf16 elements (4 fp32 ones); a view that is
+   * not goes to the CUDA-core path under CTDD_IMPL_AUTO and is refused under CTDD_IMPL_TC.  Ignored unless
+   * head == CTDD_HEAD_LOGITS. */
+  int32_t logits_dtype;         /* CTDD_DTYPE_* */
 } ctdd_step_params;
+
+enum {
+  CTDD_DTYPE_F32 = 0,          /* float32 logits */
+  CTDD_DTYPE_BF16 = 1          /* bfloat16 logits */
+};
 
 enum {
   CTDD_HEAD_LOGITS = 0,        /* dense logits */

@@ -64,10 +64,12 @@ def model_for(wname):
 
 def steps():
     # C1 / C2 also at 16 x the configuration's batch (VERDICT r1 #10: the HBM-rate claim of the small-S kernels is made there;
-    # at the configurations' own batch the inputs fit in L2 and back-to-back Python calls time the host).  The last line
-    # times the Euler kernel at the C4 shape: no configuration samples with Euler at S = 256.
+    # at the configurations' own batch the inputs fit in L2 and back-to-back Python calls time the host).  The C4 Euler line
+    # times the Euler kernel at the C4 shape: no configuration samples with Euler at S = 256.  Every line has a bf16 twin
+    # (the logits a network run under torch.autocast(dtype=torch.bfloat16) emits), and the C4 tau-leap step is also timed
+    # through the route bf16 logits took before the kernels read them: a .float() copy, then the fp32 step.
     for wname, t, mult, mname in (("C1", 0.5, 1, None), ("C1", 0.5, 16, None), ("C2", 0.1, 1, None), ("C2", 0.1, 16, None),
-                                  ("C3", 0.5, 1, None), ("C4", 0.5, 1, "euler")):
+                                  ("C3", 0.5, 1, None), ("C4", 0.5, 1, None), ("C4", 0.5, 1, "euler")):
         w, model = model_for(wname)
         mname = mname or w["mode"]
         S, D, B = w["S"], w["D"], w["B"] * mult
@@ -82,14 +84,22 @@ def steps():
         ws = torch.empty((max(1, int(nat.lib().ctdd_step_workspace_bytes(B * D, S, 0))),), dtype=torch.uint8, device=dev)
         h = (w["max_t"] - w["min_t"]) / w["num_steps"]
 
-        def run():
-            ops.reverse_step(mode, branch, lg, x, Q[0], QT[0], Rb, RbT, beta[0], h, 1e-9, N=B, D=D, S=S,
+        def run(logits):
+            ops.reverse_step(mode, branch, logits, x, Q[0], QT[0], Rb, RbT, beta[0], h, 1e-9, N=B, D=D, S=S,
                              reject_multi=not w["ordinal"], seed=1, offset=0, tc_tables=(tc[0] if tc is not None else None),
                              tc_static=tcs, workspace=ws)
-        ms = timed(run)
         name = f"step_small_kernel<{S}>" if S != 256 else ("step_tc_kernel" if mname == "euler" else "step_q_kernel")
-        report(name, f"{wname}: S={S} D={D} N={B} {mname} t={t}", ms, bytes_=4.0 * B * D * S + 8.0 * B * D,
+        what = f"{wname}: S={S} D={D} N={B} {mname} t={t}"
+        report(name, what, timed(lambda: run(lg)), bytes_=4.0 * B * D * S + 8.0 * B * D,
                flop=2.0 * B * D * S * S if S == 256 else None)
+        lgb = lg.to(torch.bfloat16)
+        del lg
+        report(name, what + " bf16 logits", timed(lambda: run(lgb)), bytes_=2.0 * B * D * S + 8.0 * B * D,
+               flop=2.0 * B * D * S * S if S == 256 else None)
+        if wname == "C4" and mname == "tau_leap":
+            report("widening copy + " + name, what + " bf16 logits through .float() and the fp32 step", timed(lambda: run(lgb.float())),
+                   bytes_=2.0 * B * D * S + 8.0 * B * D, note="the copy reads 2 and writes 4 bytes per logit on top of the step")
+        del lgb
     # CUDA-core block kernel at S = 256 (SDDM direct branch / cross-check path), and the exact-posterior branch sizes
     w, model = model_for("C3")
     S, D, B = 256, 784, 64
@@ -98,11 +108,12 @@ def steps():
     lg, x0 = bench.synth_logits(B, D, S, 8, dev, None)
     x = x0.to(torch.int32)
 
-    def run_block():
-        ops.reverse_step(nat.MODE_TAU_LEAP, nat.BRANCH_TAULDR, lg, x, Q[0], QT[0], Rb, RbT, beta[0], 1e-3, 1e-9, N=B, D=D, S=S,
+    def run_block(logits):
+        ops.reverse_step(nat.MODE_TAU_LEAP, nat.BRANCH_TAULDR, logits, x, Q[0], QT[0], Rb, RbT, beta[0], 1e-3, 1e-9, N=B, D=D, S=S,
                          seed=1, offset=0, impl=nat.IMPL_SIMT)
-    report("step_block_kernel", f"S=256 D=784 N={B} tau_leap (CUDA-core path)", timed(run_block), bytes_=4.0 * B * D * S + 8.0 * B * D,
-           flop=2.0 * B * D * S * S)
+    for logits, esz, tag in ((lg, 4, ""), (lg.to(torch.bfloat16), 2, " bf16 logits")):
+        report("step_block_kernel", f"S=256 D=784 N={B} tau_leap (CUDA-core path){tag}", timed(lambda: run_block(logits)),
+               bytes_=esz * B * D * S + 8.0 * B * D, flop=2.0 * B * D * S * S)
 
 
 def forward_process():
