@@ -55,7 +55,8 @@ class StepParams(ctypes.Structure):
 
 
 def logits_dtype_of(t) -> int:
-    """ctdd_step_params.logits_dtype of a logits tensor the step kernels read as they are (fp32, bf16)."""
+    """ctdd_step_params.logits_dtype / ctdd_loss_params.logits_dtype of a logits tensor the kernels read as they are
+    (fp32, bf16)."""
     return DTYPE_BF16 if t.dtype == torch.bfloat16 else DTYPE_F32
 
 
@@ -69,6 +70,7 @@ class LossParams(ctypes.Structure):
         ("out_a", c_void_p), ("out_b", c_void_p), ("out_c", c_void_p), ("out_d", c_void_p), ("out_nll", c_void_p),
         ("ga", c_void_p), ("gb", c_void_p), ("gd", c_void_p), ("gn", c_void_p),
         ("grad_logits", c_void_p), ("workspace", c_void_p), ("tc_scratch", c_void_p),
+        ("logits_dtype", c_int32),
     ]
 
 

@@ -10,6 +10,10 @@
 // Q once per 8 rows and was L2-bandwidth bound at ~15 TFLOP/s); other S keep ROWS = 8.  The k order of every dot
 // product is the same in both forms, so the results are bit-identical.
 // Per-sample reductions are returned as [B] vectors; the final means / weights are combined by the Python classes.
+// Logits and their gradient are fp32 or bf16 (ctdd_loss_params::logits_dtype; template argument LT of every kernel that
+// touches them).  bf16 is widened on load, which is exact, and the fp32 code runs unchanged; the gradient is rounded once
+// (round-to-nearest-even) when it is stored.  A bf16 call therefore returns the per-sample terms of the same call on the
+// widened logits (bit for bit up to the order of the cross-CTA atomicAdds) and that call's gradient rounded to bf16.
 #include "ctdd_common.cuh"
 
 namespace ctdd {
@@ -18,7 +22,7 @@ namespace loss {
 
 struct Args {
   int kind, logit_type, crm_type, B, D, S;
-  const float* logits;
+  const void* logits;  // [B][D][S] of LT
   const float* Q;
   const float* QT;
   const float* Rb;
@@ -33,7 +37,7 @@ struct Args {
   float eps;
   float* out_a; float* out_b; float* out_c; float* out_d; float* out_nll;
   const float* ga; const float* gb; const float* gd; const float* gn;
-  float* grad;
+  void* grad;          // [B][D][S] of LT
   float* bufA;         // tensor-core path (S == 256): [B][D][S] GEMM operand p, later the cotangent V
   float* bufU;         // tensor-core path: [B][D][S] u = p Q (kept from forward to backward), later dp = V Q^T
   float* lse;          // tensor-core path: [B][D] log-sum-exp of every logits row (kept from forward to backward)
@@ -192,7 +196,18 @@ __device__ __forceinline__ void rows_times_matrix(const float* __restrict__ in, 
   }
 }
 
-template <bool BWD, int ROWS>
+// One logits element as fp32.  fp32 keeps a plain load (ld_logit's __ldg would change the fp32 kernels' code); bf16 is
+// widened by ld_logit.
+template <typename LT>
+__device__ __forceinline__ float logit_at(const LT* p) {
+  if constexpr (sizeof(LT) == 4) return *p;
+  else return ld_logit(p);
+}
+// One gradient element: fp32 stored as it is, bf16 rounded to nearest even.
+__device__ __forceinline__ void st_grad(float* p, float v) { *p = v; }
+__device__ __forceinline__ void st_grad(__nv_bfloat16* p, float v) { *p = __float2bfloat16_rn(v); }
+
+template <bool BWD, int ROWS, typename LT = float>
 __global__ void __launch_bounds__(256, ROWS == 32 ? 2 : 1) loss_kernel(const Args a) {
   extern __shared__ __align__(16) float smem[];
   const int S = a.S;
@@ -224,19 +239,19 @@ __global__ void __launch_bounds__(256, ROWS == 32 ? 2 : 1) loss_kernel(const Arg
   __syncthreads();
   // 1. softmax, GEMM operand
   for (int r = warp; r < ROWS; r += nwarp) {
-    const float* lp = a.logits + ((size_t)b * a.D + d0 + (r < nr ? r : 0)) * S;
+    const LT* lp = static_cast<const LT*>(a.logits) + ((size_t)b * a.D + d0 + (r < nr ? r : 0)) * S;
     float m = -INFINITY;
-    for (int k = lane; k < S; k += 32) m = fmaxf(m, lp[k]);
+    for (int k = lane; k < S; k += 32) m = fmaxf(m, logit_at(lp + k));
     m = warp_max(m);
     float sum = 0.f;
     for (int k = lane; k < S; k += 32) {      // one exp per element: the numerators are parked in sP
-      const float e = expf(lp[k] - m);
+      const float e = expf(logit_at(lp + k) - m);
       sP[r * S + k] = e;
       sum += e;
     }
     sum = warp_sum(sum);
     const float lse = m + logf(sum);
-    if (lane == 0) { s_lse[r] = lse; s_row_n[r] = lse - lp[s_x0[r]]; }
+    if (lane == 0) { s_lse[r] = lse; s_row_n[r] = lse - logit_at(lp + s_x0[r]); }
     const int xt = s_xt[r];
     const float rsum = 1.f / sum;
     for (int k = lane; k < S; k += 32) {
@@ -253,7 +268,7 @@ __global__ void __launch_bounds__(256, ROWS == 32 ? 2 : 1) loss_kernel(const Arg
     for (int s = tid; s < S; s += nth)
 #pragma unroll
       for (int r = 0; r < ROWS; ++r)
-        sU[r * S + s] = a.logits[((size_t)b * a.D + d0 + (r < nr ? r : 0)) * S + s] - s_lse[r];  // ll directly
+        sU[r * S + s] = logit_at(static_cast<const LT*>(a.logits) + ((size_t)b * a.D + d0 + (r < nr ? r : 0)) * S + s) - s_lse[r];  // ll directly
   }
   __syncthreads();
   // SDDM / CRM: ll[s] and ll at the evaluation state
@@ -383,13 +398,13 @@ __global__ void __launch_bounds__(256, ROWS == 32 ? 2 : 1) loss_kernel(const Arg
       for (int k = lane; k < S; k += 32) dot += sP[r * S + k] * sA[r * S + k];
     }
     dot = warp_sum(dot);
-    float* gp = a.grad + ((size_t)b * a.D + d0 + r) * S;
+    LT* gp = static_cast<LT*>(a.grad) + ((size_t)b * a.D + d0 + r) * S;
     const int x0 = s_x0[r];
     for (int k = lane; k < S; k += 32) {
       const float p = sP[r * S + k];
       float g = direct ? (sU[r * S + k] - p * dot) : p * (sA[r * S + k] - dot);
       g += gn * (p - (k == x0 ? 1.f : 0.f));
-      gp[k] = g;
+      st_grad(gp + k, g);
     }
   }
 }
@@ -403,7 +418,9 @@ __global__ void __launch_bounds__(256, ROWS == 32 ? 2 : 1) loss_kernel(const Arg
 //   tc_terms_kernel u from bufU: the per-(row, s) terms and their per-sample sums            (forward)
 //                   or the cotangent V = dL/du -> bufA                                        (backward)
 //   tc_post_kernel  dp = V Q^T from bufU: softmax Jacobian + cross-entropy gradient -> grad   (backward)
-// The arithmetic per element is loss_kernel's (phases 1, 3 and 5).
+// The arithmetic per element is loss_kernel's (phases 1, 3 and 5).  With bf16 logits (LT) tc_pre_kernel and
+// tc_post_kernel read a row as two 8-byte loads per lane and tc_post_kernel stores the gradient as two 8-byte stores of
+// packed bf16; lanes own the same states, and the scratch (bufA, bufU, lse, fix) stays fp32.
 constexpr int TC_S = 256;
 constexpr int TC_ROWS = 32;      // rows of ONE sample per CTA (8 warps x 4 rows): one atomicAdd per CTA and output
 
@@ -415,6 +432,20 @@ __device__ __forceinline__ Row8 load_row8(const float* p, int lane) {
 __device__ __forceinline__ void store_row8(float* p, int lane, const float (&v)[8]) {
   reinterpret_cast<float4*>(p)[lane] = make_float4(v[0], v[1], v[2], v[3]);
   reinterpret_cast<float4*>(p + 128)[lane] = make_float4(v[4], v[5], v[6], v[7]);
+}
+__device__ __forceinline__ Row8 load_row8(const __nv_bfloat16* p, int lane) {
+  const uint2 a = __ldg(reinterpret_cast<const uint2*>(p) + lane), b = __ldg(reinterpret_cast<const uint2*>(p + 128) + lane);
+  Row8 r;
+  widen_bf16x4(a, r.v[0], r.v[1], r.v[2], r.v[3]);
+  widen_bf16x4(b, r.v[4], r.v[5], r.v[6], r.v[7]);
+  return r;
+}
+__device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {     // lo -> low half, round-to-nearest-even
+  return (uint32_t)__bfloat16_as_ushort(__float2bfloat16_rn(lo)) | ((uint32_t)__bfloat16_as_ushort(__float2bfloat16_rn(hi)) << 16);
+}
+__device__ __forceinline__ void store_row8(__nv_bfloat16* p, int lane, const float (&v)[8]) {
+  reinterpret_cast<uint2*>(p)[lane] = make_uint2(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]));
+  reinterpret_cast<uint2*>(p + 128)[lane] = make_uint2(pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
 }
 __device__ __forceinline__ int state_of(int lane, int e) { return (e < 4 ? 0 : 128) + 4 * lane + (e & 3); }
 // value of element `s` of a row held as Row8 across the warp
@@ -439,6 +470,7 @@ __device__ __forceinline__ void block_accumulate(float (&acc)[5], float* const (
   }
 }
 
+template <typename LT = float>
 __global__ void __launch_bounds__(256) tc_pre_kernel(const Args a) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, b = blockIdx.y;
   float nll = 0.f;
@@ -446,7 +478,7 @@ __global__ void __launch_bounds__(256) tc_pre_kernel(const Args a) {
     const int d = blockIdx.x * TC_ROWS + r;
     if (d >= a.D) break;
     const size_t row = (size_t)b * a.D + d;
-    const Row8 l = load_row8(a.logits + row * TC_S, lane);
+    const Row8 l = load_row8(static_cast<const LT*>(a.logits) + row * TC_S, lane);
     float m = l.v[0];
 #pragma unroll
     for (int e = 1; e < 8; ++e) m = fmaxf(m, l.v[e]);
@@ -561,6 +593,7 @@ __global__ void __launch_bounds__(256) tc_terms_kernel(const Args a) {
   }
 }
 
+template <typename LT = float>
 __global__ void __launch_bounds__(256) tc_post_kernel(const Args a) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, b = blockIdx.y;
   const float gn = a.gn[b];
@@ -568,7 +601,7 @@ __global__ void __launch_bounds__(256) tc_post_kernel(const Args a) {
     const int d = blockIdx.x * TC_ROWS + r;
     if (d >= a.D) break;
     const size_t row = (size_t)b * a.D + d;
-    const Row8 l = load_row8(a.logits + row * TC_S, lane);
+    const Row8 l = load_row8(static_cast<const LT*>(a.logits) + row * TC_S, lane);
     Row8 dp = load_row8(a.bufU + row * TC_S, lane);
     const float lse = a.lse[row], fix = a.fix[row];
     const int x0 = a.x0[row];
@@ -584,7 +617,7 @@ __global__ void __launch_bounds__(256) tc_post_kernel(const Args a) {
     float g[8];
 #pragma unroll
     for (int e = 0; e < 8; ++e) g[e] = p[e] * (dp.v[e] - dot) + gn * (p[e] - (state_of(lane, e) == x0 ? 1.f : 0.f));
-    store_row8(a.grad + row * TC_S, lane, g);
+    store_row8(static_cast<LT*>(a.grad) + row * TC_S, lane, g);
   }
 }
 
@@ -598,6 +631,10 @@ int run_loss(const ctdd_loss_params* p, void* stream, bool bwd) {
   if (!p) { set_error("ctdd_loss: null params"); return 2; }
   if (p->B <= 0 || p->D <= 0 || p->S < 2) { set_error("ctdd_loss: bad sizes"); return 2; }
   if (p->kind < CTDD_LOSS_CTELBO || p->kind > CTDD_LOSS_SDDM) { set_error("ctdd_loss: unknown kind %d", p->kind); return 2; }
+  if (p->logits_dtype != CTDD_DTYPE_F32 && p->logits_dtype != CTDD_DTYPE_BF16) {
+    set_error("ctdd_loss: unknown logits_dtype %d (CTDD_DTYPE_F32 = 0, CTDD_DTYPE_BF16 = 1)", p->logits_dtype);
+    return 2;
+  }
   if (!p->logits || !p->Q || !p->QT || !p->Rb || !p->beta || !p->x0 || !p->xt) { set_error("ctdd_loss: null input"); return 2; }
   if (p->kind != CTDD_LOSS_CTELBO && !(p->logit_type == CTDD_BRANCH_SDDM_DIRECT || p->logit_type == CTDD_BRANCH_SDDM_REVERSE_PROB ||
                                        p->logit_type == CTDD_BRANCH_SDDM_REVERSE_LOGSCALE)) {
@@ -607,6 +644,14 @@ int run_loss(const ctdd_loss_params* p, void* stream, bool bwd) {
   if (p->kind == CTDD_LOSS_CTELBO && !p->x_tilde) { set_error("ctdd_loss: x_tilde required"); return 2; }
   if (bwd && (!p->ga || !p->gb || !p->gd || !p->gn || !p->grad_logits)) { set_error("ctdd_loss_backward: null gradient pointer"); return 2; }
   if (!bwd && (!p->out_a || !p->out_b || !p->out_c || !p->out_d || !p->out_nll)) { set_error("ctdd_loss_forward: null output pointer"); return 2; }
+  // S == 256, SDDM / CRM kinds with a scratch buffer: the tensor-core path (below).  Its streaming kernels read the logits
+  // and write the gradient in 16-byte (fp32) / 8-byte (bf16) pieces per lane: both must be 16-byte aligned.
+  const bool bf16 = p->logits_dtype == CTDD_DTYPE_BF16;
+  const bool tc_path = p->S == 256 && p->tc_scratch && p->kind != CTDD_LOSS_CTELBO && p->logit_type != CTDD_BRANCH_SDDM_DIRECT;
+  if (tc_path && ((reinterpret_cast<uintptr_t>(p->logits) | (bwd ? reinterpret_cast<uintptr_t>(p->grad_logits) : 0)) & 15)) {
+    set_error("ctdd_loss: logits and grad_logits must be 16-byte aligned on the tensor-core path (S = 256, tc_scratch)");
+    return 2;
+  }
   cudaStream_t st = (cudaStream_t)stream;
   const int S = p->S;
   const int ROWS = (S == 256) ? 32 : 8;
@@ -620,6 +665,10 @@ int run_loss(const ctdd_loss_params* p, void* stream, bool bwd) {
     cudaFuncSetAttribute(loss_kernel<true, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
     cudaFuncSetAttribute(loss_kernel<false, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
     cudaFuncSetAttribute(loss_kernel<true, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    cudaFuncSetAttribute(loss_kernel<false, 8, __nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    cudaFuncSetAttribute(loss_kernel<true, 8, __nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    cudaFuncSetAttribute(loss_kernel<false, 32, __nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    cudaFuncSetAttribute(loss_kernel<true, 32, __nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
     if (dev >= 0 && dev < 64) attr_done |= 1ull << dev;
   }
   Args a;
@@ -653,8 +702,7 @@ int run_loss(const ctdd_loss_params* p, void* stream, bool bwd) {
   // streaming kernels.  u = p Q and the rows' log-sum-exp are kept in the scratch from the forward to the backward call.
   // (CT-ELBO stays on the fp32 CUDA-core contraction: its operand p / (Q[k,x~] + eps) spans 9 decades and the softmax
   // Jacobian cancels to ~1e-4 of its terms, which takes the 3 x BF16 product error past the gradient parity bar.)
-  const bool direct_branch = p->logit_type == CTDD_BRANCH_SDDM_DIRECT;
-  if (S == 256 && p->tc_scratch && p->kind != CTDD_LOSS_CTELBO && !direct_branch) {
+  if (tc_path) {
     if (reinterpret_cast<uintptr_t>(p->tc_scratch) & 15) { set_error("ctdd_loss: tc_scratch must be 16-byte aligned"); return 2; }
     const size_t n = (size_t)p->B * p->D * S;
     a.bufA = reinterpret_cast<float*>(p->tc_scratch);
@@ -663,7 +711,8 @@ int run_loss(const ctdd_loss_params* p, void* stream, bool bwd) {
     a.fix = a.lse + (size_t)p->B * p->D;
     dim3 tgrid((p->D + TC_ROWS - 1) / TC_ROWS, p->B);
     if (!bwd) {
-      tc_pre_kernel<<<tgrid, 256, 0, st>>>(a);
+      if (bf16) tc_pre_kernel<__nv_bfloat16><<<tgrid, 256, 0, st>>>(a);
+      else tc_pre_kernel<<<tgrid, 256, 0, st>>>(a);
       CTDD_CHECK_LAUNCH("tc_pre_kernel");
       if (int rc = ctdd_bgemm256_tc(a.bufA, p->QT, p->B, p->D, a.bufU, stream)) return rc;      // u[s] = sum_k p[k] Q[k][s]
       tc_terms_kernel<false><<<tgrid, 256, 0, st>>>(a);
@@ -676,7 +725,8 @@ int run_loss(const ctdd_loss_params* p, void* stream, bool bwd) {
       } else {
         if (int rc = ctdd_bgemm256_tc(a.bufA, p->Q, p->B, p->D, a.bufU, stream)) return rc;     // dp[k] = sum_s V[s] Q[k][s]
       }
-      tc_post_kernel<<<tgrid, 256, 0, st>>>(a);
+      if (bf16) tc_post_kernel<__nv_bfloat16><<<tgrid, 256, 0, st>>>(a);
+      else tc_post_kernel<<<tgrid, 256, 0, st>>>(a);
       CTDD_CHECK_LAUNCH("tc_post_kernel");
     }
     return 0;
@@ -687,11 +737,21 @@ int run_loss(const ctdd_loss_params* p, void* stream, bool bwd) {
   if (threads < 64) threads = 64;
   dim3 grid((p->D + ROWS - 1) / ROWS, p->B);
   if (ROWS == 32) {
-    if (bwd) loss_kernel<true, 32><<<grid, threads, smem, st>>>(a);
-    else loss_kernel<false, 32><<<grid, threads, smem, st>>>(a);
+    if (bf16) {
+      if (bwd) loss_kernel<true, 32, __nv_bfloat16><<<grid, threads, smem, st>>>(a);
+      else loss_kernel<false, 32, __nv_bfloat16><<<grid, threads, smem, st>>>(a);
+    } else {
+      if (bwd) loss_kernel<true, 32><<<grid, threads, smem, st>>>(a);
+      else loss_kernel<false, 32><<<grid, threads, smem, st>>>(a);
+    }
   } else {
-    if (bwd) loss_kernel<true, 8><<<grid, threads, smem, st>>>(a);
-    else loss_kernel<false, 8><<<grid, threads, smem, st>>>(a);
+    if (bf16) {
+      if (bwd) loss_kernel<true, 8, __nv_bfloat16><<<grid, threads, smem, st>>>(a);
+      else loss_kernel<false, 8, __nv_bfloat16><<<grid, threads, smem, st>>>(a);
+    } else {
+      if (bwd) loss_kernel<true, 8><<<grid, threads, smem, st>>>(a);
+      else loss_kernel<false, 8><<<grid, threads, smem, st>>>(a);
+    }
   }
   CTDD_CHECK_LAUNCH("loss_kernel");
   return 0;

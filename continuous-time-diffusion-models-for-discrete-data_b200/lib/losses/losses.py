@@ -6,7 +6,8 @@ Same registered names, config keys and `calc_loss` signatures (BOTH argument ord
   * q_{t|0} for the B distinct times: `ctdd_build_qt0` (one matrix per sample, lib/losses/losses.py:39);
   * forward noising x_t ~ q_{t|0}(.|x_0) and the one-jump proposal x~ (losses.py:46-101): `ctdd_noise_xt`;
   * every (B,D,S)-sized term of CT-ELBO / SDDM-ELBO / ratio matching, forward and backward w.r.t. the logits:
-    `ctdd_loss_forward` / `ctdd_loss_backward` behind one autograd.Function (ops.loss_terms);
+    `ctdd_loss_forward` / `ctdd_loss_backward` behind one autograd.Function (ops.loss_terms), on the logits as the
+    network emits them (fp32, or bf16 under torch.autocast(dtype=torch.bfloat16), with a bf16 gradient back);
   * the final O(B) combination (means, nll weights, lambda mixing) is torch arithmetic on (B,) vectors.
 `reverse_logscale` materialises (B,D,S,S) in the reference (infeasible at S=256); here it is the same fused kernel as
 `reverse_prob`: the log-sum-exp over k of log p_k + log q[k,s] IS log(sum_k p_k q[k,s]) without the 1e-35 guard, and

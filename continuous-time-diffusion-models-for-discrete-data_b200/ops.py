@@ -374,7 +374,11 @@ def bgemm256(X, M, out=None):
 
 class _LossTerms(torch.autograd.Function):
     """Per-sample loss terms (out_a, out_b, out_c, out_d, out_nll), each (B,), differentiable w.r.t. `logits`
-    through the fused backward kernel (include/ctdd.h: ctdd_loss_forward / ctdd_loss_backward)."""
+    through the fused backward kernel (include/ctdd.h: ctdd_loss_forward / ctdd_loss_backward).
+
+    fp32 and bf16 logits are read as they are; bf16 ones (a network under torch.autocast(dtype=torch.bfloat16)) get a
+    bf16 gradient, equal to the fp32 gradient of their widening rounded to bf16.  Other dtypes are widened to an fp32
+    copy and autograd casts the gradient back."""
     #: S == 256: run the two contractions on tcgen05 (set False to force the CUDA-core kernel, e.g. as a cross-check)
     use_tc = True
 
@@ -382,7 +386,12 @@ class _LossTerms(torch.autograd.Function):
     def forward(ctx, logits, kind, logit_branch, crm_type, Q, QT, Rb, beta, x0, xt, x_tilde, eps):
         B, D, S = logits.shape
         dev = logits.device
-        logits = logits.contiguous().float()
+        if logits.dtype == torch.bfloat16:
+            logits = logits.contiguous()
+            if logits.data_ptr() % 16:          # e.g. a contiguous view at an odd storage offset: 16-byte rows needed
+                logits = logits.clone()
+        else:
+            logits = logits.contiguous().float()
         outs = torch.zeros((5, B), dtype=torch.float32, device=dev)
         nbytes = int(nat.lib().ctdd_loss_workspace_bytes(kind, B, S))
         ws = torch.empty((max(nbytes, 4),), dtype=torch.uint8, device=dev)
@@ -395,7 +404,7 @@ class _LossTerms(torch.autograd.Function):
                            x0=nat.ptr(x0), xt=nat.ptr(xt), x_tilde=nat.ptr(x_tilde), eps=float(eps),
                            out_a=outs[0].data_ptr(), out_b=outs[1].data_ptr(), out_c=outs[2].data_ptr(),
                            out_d=outs[3].data_ptr(), out_nll=outs[4].data_ptr(), workspace=nat.ptr(ws),
-                           tc_scratch=nat.ptr(scr))
+                           tc_scratch=nat.ptr(scr), logits_dtype=nat.logits_dtype_of(logits))
         nat.check(nat.lib().ctdd_loss_forward(p, nat.stream()), "ctdd_loss_forward")
         ctx.scr = scr
         ctx.save_for_backward(logits, Q, QT, Rb, beta, x0, xt, x_tilde if x_tilde is not None else xt, ws)
@@ -414,12 +423,12 @@ class _LossTerms(torch.autograd.Function):
         B, D, S = logits.shape
         z = lambda g: (g if g is not None else torch.zeros((B,), device=logits.device)).contiguous().float()
         ga, gb, gd, gn = z(ga), z(gb), z(gd), z(gn)
-        grad = torch.empty_like(logits)
+        grad = torch.empty_like(logits)             # the logits' dtype: bf16 logits get a bf16 gradient
         p = nat.LossParams(kind=kind, logit_type=logit_branch, crm_type=crm_type, B=B, D=D, S=S,
                            logits=nat.ptr(logits), Q=nat.ptr(Q), QT=nat.ptr(QT), Rb=nat.ptr(Rb), beta=nat.ptr(beta),
                            x0=nat.ptr(x0), xt=nat.ptr(xt), x_tilde=(nat.ptr(x_tilde) if has_tilde else None), eps=eps,
                            ga=nat.ptr(ga), gb=nat.ptr(gb), gd=nat.ptr(gd), gn=nat.ptr(gn), grad_logits=nat.ptr(grad),
-                           workspace=nat.ptr(ws), tc_scratch=nat.ptr(ctx.scr))
+                           workspace=nat.ptr(ws), tc_scratch=nat.ptr(ctx.scr), logits_dtype=nat.logits_dtype_of(logits))
         nat.check(nat.lib().ctdd_loss_backward(p, nat.stream()), "ctdd_loss_backward")
         return (grad,) + (None,) * 11
 

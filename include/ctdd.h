@@ -241,7 +241,7 @@ typedef struct ctdd_loss_params {
   int32_t logit_type;    /* CTDD_BRANCH_SDDM_* (CRM / SDDM kinds) */
   int32_t crm_type;      /* 0 rm, 1 mle, 2 elbo (loss.loss_type, losses.py:794-836) */
   int32_t B, D, S;
-  const float* logits;   /* [B,D,S] */
+  const void* logits;    /* [B,D,S] of logits_dtype */
   const float* Q;        /* [B,S,S] */
   const float* QT;       /* [B,S,S] */
   const float* Rb;       /* [S,S] */
@@ -258,13 +258,22 @@ typedef struct ctdd_loss_params {
   float* out_nll;        /* sum_d CrossEntropy(logits[b,d,:], x0[b,d])                            */
   /* backward: grad_logits[b] = ga[b]*d out_a + gb[b]*d out_b + gd[b]*d out_d + gn[b]*d out_nll */
   const float* ga; const float* gb; const float* gd; const float* gn;
-  float* grad_logits;    /* [B,D,S] */
+  void* grad_logits;     /* [B,D,S] of logits_dtype (bf16 logits get a bf16 gradient) */
   void* workspace;       /* >= ctdd_loss_workspace_bytes(kind, B, S); written by forward, read by backward */
   /* appended field (zero-initialised = CUDA-core contractions).  S == 256, kinds SDDM and CRM with reverse_prob /
    * reverse_logscale: >= ctdd_loss_tc_scratch_bytes(B, D, S) bytes, 16-byte aligned; the two (B*D x S)(S x S) contractions
    * then run on tcgen05 (ctdd_bgemm256_tc).  Written by forward, read AND overwritten by backward: pass the same buffer to
    * both calls, untouched in between.  Ignored for CT-ELBO and the `direct` logit type. */
   void* tc_scratch;
+  /* Element type of `logits` and `grad_logits` (appended field; zero-initialised = fp32): CTDD_DTYPE_F32 or
+   * CTDD_DTYPE_BF16, as in ctdd_step_params.  bf16 takes the logits a network run under
+   * torch.autocast(dtype=torch.bfloat16) emits without a widening copy: the kernels widen on load (exact), run the fp32
+   * arithmetic, and round the gradient once (to nearest even) when they store it.  The per-sample outputs equal those of
+   * the same call on the widened logits up to the order of the per-CTA atomicAdds, and grad_logits equals that call's
+   * fp32 gradient rounded to bf16, bit for bit.  The outputs, ga..gn, workspace and tc_scratch stay fp32.  On the
+   * tensor-core path (tc_scratch at S == 256) logits and grad_logits must be 16-byte aligned for either type; other
+   * pointers are refused with status 2 before any launch. */
+  int32_t logits_dtype;  /* CTDD_DTYPE_* */
 } ctdd_loss_params;
 
 enum {

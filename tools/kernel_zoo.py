@@ -42,8 +42,10 @@ def timed(fn, reps=10, warm=3):
     return a.elapsed_time(b) / reps
 
 
-def report(name, what, ms, bytes_=None, flop=None, note=""):
+def report(name, what, ms, bytes_=None, flop=None, note="", peak=None):
     rec = {"kernel": name, "workload": what, "ms": round(ms, 5)}
+    if peak is not None:
+        rec["peak_fwd_bwd_MB"] = round(peak / 2 ** 20, 1)
     if bytes_ is not None:
         rec["alg_bytes"] = int(bytes_)
         rec["GB/s"] = round(bytes_ / ms / 1e6, 1)
@@ -141,6 +143,10 @@ def forward_process():
 
 
 def losses():
+    # Each line has a bf16 twin (the logits a network run under torch.autocast(dtype=torch.bfloat16) emits, read as they
+    # are, with a bf16 gradient) and a line for the route bf16 logits took before the kernels read them: a .float() copy
+    # before ops.loss_terms, the fp32 gradient cast back to bf16 by autograd.  The three run alternately, and each reports
+    # the peak device memory of one forward + backward over what was allocated before it.
     w, model = model_for("C4")
     S = 256
     Rb, _ = model.base_rate_tables(dev)
@@ -151,22 +157,36 @@ def losses():
         beta = model._rate_scalar(ts).float().contiguous()
         x0 = torch.randint(0, S, (B, D), device=dev, dtype=torch.int32)
         xt, xtil = ops.noise_xt(Q, Rb, beta, x0, 1, 0)
-        logits = (torch.randn(B, D, S, device=dev) - (torch.arange(S, device=dev).view(1, 1, S) - x0.unsqueeze(-1)) ** 2 / 128.0)
-        logits.requires_grad_(True)
+        lf32 = (torch.randn(B, D, S, device=dev) - (torch.arange(S, device=dev).view(1, 1, S) - x0.unsqueeze(-1)) ** 2 / 128.0)
+        lb16 = lf32.to(torch.bfloat16)
 
-        def fwd():
+        def fwd(logits):
             return ops.loss_terms(logits, kind, Q=Q, QT=QT, Rb=Rb, beta=beta, x0=x0, xt=xtil if kind != nat.LOSS_CRM else xt,
                                   x_tilde=xtil if kind == nat.LOSS_CTELBO else None, eps=1e-9)
 
-        def fwd_bwd():
-            sum(o.sum() for o in fwd()).backward()
-            logits.grad = None
-        with torch.no_grad():
-            ms_f = timed(fwd)
-        ms_fb = timed(fwd_bwd)
-        report("loss_kernel<0>", f"{name} forward, B={B} D={D} S=256", ms_f, bytes_=4.0 * B * D * S, flop=2.0 * B * D * S * S)
-        report("loss_kernel<0> + loss_kernel<1>", f"{name} forward + backward (torch autograd glue included)", ms_fb,
-               bytes_=12.0 * B * D * S, flop=6.0 * B * D * S * S)
+        def fwd_bwd(leaf, widen):
+            sum(o.sum() for o in fwd(leaf.float() if widen else leaf)).backward()
+            leaf.grad = None
+
+        def peak(leaf, widen):
+            torch.cuda.synchronize()
+            base = torch.cuda.memory_allocated()
+            torch.cuda.reset_peak_memory_stats()
+            fwd_bwd(leaf, widen)
+            torch.cuda.synchronize()
+            return torch.cuda.max_memory_allocated() - base
+        for tag, leaf, esz, widen in (("", lf32, 4, False), (" bf16 logits", lb16, 2, False),
+                                      (" bf16 logits through .float()", lb16, 2, True)):
+            leaf.requires_grad_(True)
+            with torch.no_grad():
+                ms_f = timed(lambda: fwd(leaf.float() if widen else leaf))
+            ms_fb = timed(lambda: fwd_bwd(leaf, widen))
+            note = "the copy reads 2 and writes 4 bytes per logit, the gradient cast reads 4 and writes 2" if widen else ""
+            report(("widening copy + " if widen else "") + "loss_kernel<0>", f"{name} forward, B={B} D={D} S=256{tag}", ms_f,
+                   bytes_=esz * B * D * S, flop=2.0 * B * D * S * S, note=note)
+            report(("widening copy + " if widen else "") + "loss_kernel<0> + loss_kernel<1>",
+                   f"{name} forward + backward (torch autograd glue included){tag}", ms_fb, bytes_=3.0 * esz * B * D * S,
+                   flop=6.0 * B * D * S * S, note=note, peak=peak(leaf, widen))
 
 
 def head():
