@@ -50,7 +50,7 @@ class StepParams(ctypes.Structure):
         ("x_out", c_void_p), ("rr_out", c_void_p), ("ratio_out", c_void_p),
         ("stats_out", c_void_p), ("workspace", c_void_p),
         ("head", c_int32), ("head_mu", c_void_p), ("head_log_scale", c_void_p), ("head_batch_stride", c_int64),
-        ("logits_dtype", c_int32),
+        ("logits_dtype", c_int32), ("head_dtype", c_int32),
     ]
 
 
@@ -111,6 +111,12 @@ def lib() -> ctypes.CDLL:
     L.ctdd_logistic_logits_backward.argtypes = [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int64, c_int, c_int, c_void_p,
                                                 c_void_p, c_void_p]
     L.ctdd_logistic_logits_backward.restype = c_int
+    L.ctdd_logistic_logits_ex.argtypes = [c_void_p, c_void_p, c_int, c_int, c_int, c_int64, c_int, c_int, c_void_p, c_int,
+                                          c_void_p]
+    L.ctdd_logistic_logits_ex.restype = c_int
+    L.ctdd_logistic_logits_backward_ex.argtypes = [c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int64, c_int,
+                                                   c_int, c_void_p, c_void_p, c_void_p]
+    L.ctdd_logistic_logits_backward_ex.restype = c_int
     L.ctdd_pair_partials.argtypes = [c_int, c_int]
     L.ctdd_pair_partials.restype = c_int64
     L.ctdd_pair_similarity.argtypes = [c_void_p, c_int, c_void_p, c_int, c_int, c_float, c_int, c_void_p, c_void_p]

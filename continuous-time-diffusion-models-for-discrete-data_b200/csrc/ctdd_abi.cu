@@ -45,6 +45,10 @@ extern "C" int ctdd_reverse_step(const ctdd_step_params* p, void* stream) {
     set_error("ctdd_reverse_step: unknown logits_dtype %d (CTDD_DTYPE_F32 = 0, CTDD_DTYPE_BF16 = 1)", p->logits_dtype);
     return 2;
   }
+  if (p->head != CTDD_HEAD_LOGITS && p->head_dtype != CTDD_DTYPE_F32 && p->head_dtype != CTDD_DTYPE_BF16) {
+    set_error("ctdd_reverse_step: unknown head_dtype %d (CTDD_DTYPE_F32 = 0, CTDD_DTYPE_BF16 = 1)", p->head_dtype);
+    return 2;
+  }
   if (p->head == CTDD_HEAD_LOGITS ? !p->logits : (!p->head_mu || !p->head_log_scale || p->head_batch_stride < p->D)) {
     set_error("ctdd_reverse_step: null logits (or head_mu / head_log_scale / head_batch_stride < D for a logistic head)");
     return 2;

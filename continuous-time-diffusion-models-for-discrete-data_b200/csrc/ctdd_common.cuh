@@ -90,9 +90,10 @@ __device__ __forceinline__ Philox4 philox_keyed(uint32_t c0, uint32_t c1, uint32
   return o;
 }
 
-// Logits of the reverse step are fp32 or bf16 (ctdd_step_params::logits_dtype).  Widening bf16 to fp32 is exact (the 16
-// bits are the upper half of the fp32 pattern), so a kernel that widens on load and then runs its fp32 code returns the
-// results of the same call on the widened logits bit for bit.
+// Logits of the reverse step are fp32 or bf16 (ctdd_step_params::logits_dtype), and so are the truncated-logistic head's
+// (mu, log_scale) and incoming gradient.  Widening bf16 to fp32 is exact (the 16 bits are the upper half of the fp32
+// pattern), so a kernel that widens on load and then runs its fp32 code returns the results of the same call on the
+// widened inputs bit for bit.
 __device__ __forceinline__ float ld_logit(const float* p) { return __ldg(p); }
 __device__ __forceinline__ float ld_logit(const __nv_bfloat16* p) {
   return __uint_as_float((uint32_t)__ldg(reinterpret_cast<const unsigned short*>(p)) << 16);

@@ -101,14 +101,18 @@ __device__ __forceinline__ int prefix_search(uint32_t P, float T) {
   return 32 * c1 + 4 * c2 + c3;
 }
 
+// (mu, log_scale) of the fused head as the producers carry them: fp32, or the raw bits of a bf16 value (exact widening)
+__device__ __forceinline__ float widen_head(float v) { return v; }
+__device__ __forceinline__ float widen_head(unsigned short v) { return __uint_as_float((uint32_t)v << 16); }
+
 // ---------------------------------------------------------------------------------------------- the kernel
 // TAULDR: tauLDR rates (else SDDM reverse_prob); CORR: the corrector variant adds h * R_t[x,:] to the rates;
 // HEAD: the rows' softmax numerators come from the truncated-logistic head (mu, log_scale per row) instead of logits;
 // LT: element type of the logits, float or __nv_bfloat16 (a bf16 row pair travels packed, 2*S bytes per row, and is
-// widened on the producers' shared-memory load; the arithmetic after that load is the fp32 kernel's)
+// widened on the producers' shared-memory load; the arithmetic after that load is the fp32 kernel's).  A HEAD kernel reads
+// no logits: LT is then the type of (mu, log_scale), widened on the producers' load
 template <bool TAULDR, bool CORR, bool HEAD, typename LT = float>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step_tc_kernel(const Args a) {
-  static_assert(!HEAD || sizeof(LT) == 4, "the head kernels read no logits");
   constexpr uint32_t ROW_BYTES = S * sizeof(LT);
   extern __shared__ uint8_t smem_raw[];
   // aligned by offsetting the shared array itself (not through an integer): the compiler keeps `sm` a shared-space
@@ -176,7 +180,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
     int f_left = npass, f_ps = 0, f_slot = 0;
     // lane 0 starts the bulk copy of the next row pair (rows past the end are replaced by row 0: never used; adjacent
     // rows of a contiguous logits tensor travel as one 2 KB copy); every lane fetches the state of its half's row
-    float f_mu = 0.f, f_ls = 0.f;        // HEAD: head parameters of the row fetch() just visited
+    // HEAD: head parameters of the row fetch() just visited.  They reach their use two passes later in their stored type
+    // (bf16 as its raw 16 bits) and are widened only there: a widening at the load would wait for the load right away and
+    // put its latency on the warp's critical path
+    using HeadRaw = typename std::conditional<sizeof(LT) == 2, unsigned short, float>::type;
+    HeadRaw f_mu = 0, f_ls = 0;
     auto fetch = [&]() -> int {
       int xv = -1;
       if (f_left > 0) {
@@ -189,8 +197,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
               const long long n = (a.rows <= 0xFFFFFFFFLL) ? (long long)((uint32_t)g / (uint32_t)a.D) : g / a.D;
               src = n * a.head_bs + (g - n * a.D);
             }
-            f_mu = __ldg(a.head_mu + src);
-            f_ls = __ldg(a.head_ls + src);
+            f_mu = __ldg(static_cast<const HeadRaw*>(a.head_mu) + src);
+            f_ls = __ldg(static_cast<const HeadRaw*>(a.head_ls) + src);
           }
         } else if (lane == 0) {
           uint64_t* bar = &sm.lring_full[pw][f_slot];
@@ -219,9 +227,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
     };
 
     int x_cur = fetch();
-    float mu_cur = f_mu, ls_cur = f_ls;
+    HeadRaw mu_cur = f_mu, ls_cur = f_ls;
     int x_n1 = fetch();
-    float mu_n1 = f_mu, ls_n1 = f_ls;
+    HeadRaw mu_n1 = f_mu, ls_n1 = f_ls;
     float4 t4[4];
     {
       const size_t xo = (size_t)(x_cur < 0 ? 0 : x_cur) << 8;
@@ -273,7 +281,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
           p_sum += __shfl_xor_sync(0xffffffffu, p_sum, o);
           if (!TAULDR) p_dot += __shfl_xor_sync(0xffffffffu, p_dot, o);
         }
-        head_numerators(mu_cur, ls_cur, a.head_fix != 0, l16, v);
+        head_numerators(widen_head(mu_cur), widen_head(ls_cur), a.head_fix != 0, l16, v);
       } else {
         if constexpr (sizeof(LT) == 2) {
           // lane l16 widens the same elements 64c + 4*l16 .. +3 as in the fp32 kernel, one 64-bit load each
@@ -680,17 +688,18 @@ int launch_step_tc(const ctdd_step_params* p, cudaStream_t st) {
   const size_t smem_bytes = sizeof(Smem) + 1024;
   typedef void (*kern_t)(const Args);
 #define CTDD_TC_ROW(T, H, LT) step_tc_kernel<T, false, H, LT>, step_tc_kernel<T, true, H, LT>
-  static const kern_t kerns[12] = {CTDD_TC_ROW(false, false, float), CTDD_TC_ROW(true, false, float),
+  static const kern_t kerns[16] = {CTDD_TC_ROW(false, false, float), CTDD_TC_ROW(true, false, float),
                                      CTDD_TC_ROW(false, true, float), CTDD_TC_ROW(true, true, float),
-                                     CTDD_TC_ROW(false, false, __nv_bfloat16), CTDD_TC_ROW(true, false, __nv_bfloat16)};
+                                     CTDD_TC_ROW(false, false, __nv_bfloat16), CTDD_TC_ROW(true, false, __nv_bfloat16),
+                                     CTDD_TC_ROW(false, true, __nv_bfloat16), CTDD_TC_ROW(true, true, __nv_bfloat16)};
 #undef CTDD_TC_ROW
   Args a = make_args(p);
   a.num_tiles = (int)((a.rows + NT - 1) / NT);
   const int pairs = pair_count(launch_state, "ctdd_reverse_step", kerns, smem_bytes, a.num_tiles);
   if (!pairs) return 1;
-  // rows of kerns: fp32 logits, fused head, bf16 logits
-  const int ki = ((p->branch == CTDD_BRANCH_TAULDR) ? 1 : 0) +
-                 (p->head != CTDD_HEAD_LOGITS ? 2 : (p->logits_dtype == CTDD_DTYPE_BF16 ? 4 : 0));
+  // rows of kerns: fp32 logits, fused head on fp32 (mu, log_scale), bf16 logits, fused head on bf16 (mu, log_scale)
+  const int ki = ((p->branch == CTDD_BRANCH_TAULDR) ? 1 : 0) + (p->head != CTDD_HEAD_LOGITS ? 2 : 0) +
+                 ((p->head != CTDD_HEAD_LOGITS ? p->head_dtype : p->logits_dtype) == CTDD_DTYPE_BF16 ? 4 : 0);
   const int kj = (p->mode == CTDD_MODE_EULER_CORR) ? 1 : 0;
   kerns[2 * ki + kj]<<<2 * pairs, NUM_THREADS, smem_bytes, st>>>(a);
   CTDD_CHECK_LAUNCH("step_tc_kernel");

@@ -110,10 +110,10 @@ static_assert(RING > STAGES + ACC + CBUF, "row-scalar ring shorter than the pipe
 // TAULDR: tauLDR rates (else SDDM reverse_prob); KM: KM_JUMP / KM_CORR / KM_RATES / KM_DRIFT;
 // HEAD: the rows' softmax numerators come from the truncated-logistic head (mu, log_scale per row) instead of logits;
 // LT: element type of the logits, float or __nv_bfloat16 (bf16 rows travel packed, 2*S bytes each, and are widened on
-// the producers' shared-memory load; the arithmetic after that load is the fp32 kernel's)
+// the producers' shared-memory load; the arithmetic after that load is the fp32 kernel's).  A HEAD kernel reads no logits:
+// LT is then the type of (mu, log_scale), widened on the loader warp's load
 template <bool TAULDR, int KM, bool HEAD, typename LT = float>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step_q_kernel(const Args a) {
-  static_assert(!HEAD || sizeof(LT) == 4, "the head kernels read no logits");
   constexpr uint32_t ROW_BYTES = S * sizeof(LT);
   extern __shared__ uint8_t smem_raw[];
   Smem& sm = *reinterpret_cast<Smem*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
@@ -393,8 +393,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
           const uint32_t n = (uint32_t)g / (uint32_t)a.D;
           src = (long long)n * a.head_bs + ((uint32_t)g - n * (uint32_t)a.D);
         }
-        h_mu = __ldg(a.head_mu + src);
-        h_ls = __ldg(a.head_ls + src);
+        h_mu = ld_logit(static_cast<const LT*>(a.head_mu) + src);
+        h_ls = ld_logit(static_cast<const LT*>(a.head_ls) + src);
       };
       if (HEAD) head_load(0);
       int grp = 0;               // (lanes < NSUB) next round of the lane's group: passes NPW * grp + 4 * lane .. + 3
@@ -826,9 +826,10 @@ int launch_step_tcq(const ctdd_step_params* p, cudaStream_t st) {
 #define CTDD_TCQ_ROW(T, H, LT)                                                                                            \
   step_q_kernel<T, tc::KM_JUMP, H, LT>, step_q_kernel<T, tc::KM_CORR, H, LT>, step_q_kernel<T, tc::KM_RATES, H, LT>,    \
       step_q_kernel<T, tc::KM_DRIFT, H, LT>
-  static const kern_t kerns[24] = {CTDD_TCQ_ROW(false, false, float), CTDD_TCQ_ROW(true, false, float),
+  static const kern_t kerns[32] = {CTDD_TCQ_ROW(false, false, float), CTDD_TCQ_ROW(true, false, float),
                                      CTDD_TCQ_ROW(false, true, float), CTDD_TCQ_ROW(true, true, float),
-                                     CTDD_TCQ_ROW(false, false, __nv_bfloat16), CTDD_TCQ_ROW(true, false, __nv_bfloat16)};
+                                     CTDD_TCQ_ROW(false, false, __nv_bfloat16), CTDD_TCQ_ROW(true, false, __nv_bfloat16),
+                                     CTDD_TCQ_ROW(false, true, __nv_bfloat16), CTDD_TCQ_ROW(true, true, __nv_bfloat16)};
 #undef CTDD_TCQ_ROW
   if (reinterpret_cast<uintptr_t>(p->tc_static) % tc::ST_ALIGN) {
     set_error("ctdd_reverse_step: tc_static must be aligned to ctdd_tc_static_align() = %zu bytes", tc::ST_ALIGN);
@@ -842,9 +843,9 @@ int launch_step_tcq(const ctdd_step_params* p, cudaStream_t st) {
   a.num_tiles = (int)((a.rows + NT - 1) / NT);
   const int pairs = tc::pair_count(launch_state, "ctdd_reverse_step", kerns, smem_bytes, a.num_tiles);
   if (!pairs) return 1;
-  // rows of kerns: fp32 logits, fused head, bf16 logits
-  const int ki = ((p->branch == CTDD_BRANCH_TAULDR) ? 1 : 0) +
-                 (p->head != CTDD_HEAD_LOGITS ? 2 : (p->logits_dtype == CTDD_DTYPE_BF16 ? 4 : 0));
+  // rows of kerns: fp32 logits, fused head on fp32 (mu, log_scale), bf16 logits, fused head on bf16 (mu, log_scale)
+  const int ki = ((p->branch == CTDD_BRANCH_TAULDR) ? 1 : 0) + (p->head != CTDD_HEAD_LOGITS ? 2 : 0) +
+                 ((p->head != CTDD_HEAD_LOGITS ? p->head_dtype : p->logits_dtype) == CTDD_DTYPE_BF16 ? 4 : 0);
   int kj = 0;
   if (p->mode == CTDD_MODE_RATES_ONLY) kj = 2;
   else if (p->mode == CTDD_MODE_TAU_LEAP_CORR) kj = 1;

@@ -53,8 +53,8 @@ struct Args {
   unsigned long long* stats;
   int num_tiles;
   int head_fix;              // fused truncated-logistic head (HEAD kernels): fix_logistic
-  const float* head_mu;
-  const float* head_ls;
+  const void* head_mu;       // fp32 or bf16 (HEAD kernels: the logits-type template argument names the head's type)
+  const void* head_ls;
   long long head_bs;         // elements between consecutive n
 };
 

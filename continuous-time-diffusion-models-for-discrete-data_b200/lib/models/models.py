@@ -11,7 +11,10 @@ lib/networks/unet.py:450-452) into an (B, D, S) logits tensor with ~20 elementwi
   (`ctdd_logistic_logits`) when no gradient is required;
 * with gradients enabled (training) the head is one `autograd.Function`: the same forward kernel, and a backward kernel
   (`ctdd_logistic_logits_backward`) that recomputes the head from (mu, log_scale) and reads the incoming (B, D, S) gradient
-  once — instead of autograd through ~20 saved (B, D, S) tensors.  Host or non-fp32 inputs are refused (no fallback).
+  once — instead of autograd through ~20 saved (B, D, S) tensors.  Host inputs are refused (no fallback), and so are
+  dtypes other than fp32 or bf16 for both.  bf16 (mu, log_scale) — a network under torch.autocast(dtype=torch.bfloat16),
+  or one converted to bf16 — give bf16 logits: the fp32 values rounded once, which the losses read as they are
+  (DESIGN.md §3).
 """
 from __future__ import annotations
 
@@ -26,14 +29,18 @@ def log_minus_exp(a, b, eps=1e-6):
 
 
 def _logistic_logits_autograd(mu, log_scale, S, fix_logistic):
-    """Differentiable head on the training path: CUDA forward + backward kernels (fp32 CUDA tensors; like the rest of the
-    package there is no CPU / PyTorch fallback)."""
+    """Differentiable head on the training path: CUDA forward + backward kernels (CUDA tensors; like the rest of the
+    package there is no CPU / PyTorch fallback).  fp32 (mu, log_scale) give fp32 logits, bf16 ones bf16 logits."""
     if not (mu.is_cuda and log_scale.is_cuda):
         raise RuntimeError("ctdd_b200: the truncated-logistic head runs on CUDA tensors only (no CPU fallback)")
-    if mu.dtype != torch.float32 or log_scale.dtype != torch.float32:
-        raise RuntimeError(f"ctdd_b200: the truncated-logistic head takes float32 (mu, log_scale); got {mu.dtype}, "
-                           f"{log_scale.dtype} - run the head outside autocast or cast the network output")
-    return ops.logistic_logits_autograd(mu, log_scale, S, fix_logistic).view(*mu.shape, S)
+    if mu.dtype == torch.bfloat16 and log_scale.dtype == torch.bfloat16:
+        out_dtype = torch.bfloat16
+    elif mu.dtype == torch.float32 and log_scale.dtype == torch.float32:
+        out_dtype = torch.float32
+    else:
+        raise RuntimeError(f"ctdd_b200: the truncated-logistic head takes float32 or bfloat16 (mu, log_scale), both of one "
+                           f"dtype; got {mu.dtype}, {log_scale.dtype} - cast the network output")
+    return ops.logistic_logits_autograd(mu, log_scale, S, fix_logistic, out_dtype=out_dtype).view(*mu.shape, S)
 
 
 def sample_logistic(net_out, B, C, D, S, fix_logistic, device):

@@ -96,14 +96,16 @@ class StepEngine:
         return self._t_all[tidx]
 
     def _fast_step(self, mode, logits, x_eval, tidx, h, reject_multi, x_base, row):
-        """The common case of step(): dense contiguous fp32 / bf16 logits or an un-materialised head, state update only."""
+        """The common case of step(): dense contiguous fp32 / bf16 logits or an un-materialised head (fp32 or bf16
+        (mu, log_scale)), state update only."""
         N, D, S = self.N, self.D, self.S
         p = self._p
         if isinstance(logits, ops.LogisticHead):
             mu, ls, fix = logits.as_tuple()
-            mu, ls, head_bs = ops._head_views(mu, ls, N, D)
+            mu, ls, head_bs, head_dt = ops._head_views(mu, ls, N, D)
             p.head = nat.HEAD_LOGISTIC_FIX if fix else nat.HEAD_LOGISTIC
             p.head_mu, p.head_log_scale, p.head_batch_stride, p.logits = mu.data_ptr(), ls.data_ptr(), int(head_bs), None
+            p.head_dtype = head_dt      # rewritten every call, like logits_dtype: the struct is reused
         else:
             p.head, p.head_mu, p.head_log_scale, p.head_batch_stride = nat.HEAD_LOGITS, None, None, 0
             p.logits = logits.data_ptr()

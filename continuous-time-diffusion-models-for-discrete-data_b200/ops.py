@@ -59,14 +59,15 @@ def reverse_step(mode, branch, logits, x_eval, Q, QT, Rb, RbT, beta, h, eps, *, 
     """One fused reverse-rate evaluation (+ state update). Returns dict(x=..., rr=..., ratio=...).
 
     `head=(mu, log_scale, fix_logistic)` replaces `logits` (pass None) by the parameters of the truncated-logistic
-    output head (reference lib/models/models.py:248-282): mu / log_scale are (N, D)-shaped fp32 views whose batch
-    stride may exceed D (the two torch.chunk halves of a (B, 2C, H, W) network output).  On the tcgen05 path the
-    logits are never materialised; elsewhere they are built once with `logistic_logits`."""
+    output head (reference lib/models/models.py:248-282): mu / log_scale are (N, D)-shaped views whose batch
+    stride may exceed D (the two torch.chunk halves of a (B, 2C, H, W) network output), fp32, or bf16 both (read as
+    they are).  On the tcgen05 path the logits are never materialised; elsewhere they are built once with
+    `logistic_logits`, as fp32."""
     dev = x_eval.device
-    head_kind, head_mu, head_ls, head_bs = nat.HEAD_LOGITS, None, None, 0
+    head_kind, head_mu, head_ls, head_bs, head_dt = nat.HEAD_LOGITS, None, None, 0, nat.DTYPE_F32
     if head is not None:
         mu, ls, fix = head
-        mu, ls, head_bs = _head_views(mu, ls, N, D)
+        mu, ls, head_bs, head_dt = _head_views(mu, ls, N, D)
         use_tc = S == 256 and tc_tables is not None and impl != nat.IMPL_SIMT and mode != nat.MODE_EXACT and \
             branch in (nat.BRANCH_TAULDR, nat.BRANCH_SDDM_REVERSE_PROB)
         if use_tc:
@@ -101,24 +102,30 @@ def reverse_step(mode, branch, logits, x_eval, Q, QT, Rb, RbT, beta, h, eps, *, 
         stats_out=(stats.data_ptr() if stats is not None else None), workspace=nat.ptr(workspace),
         head=head_kind, head_mu=(head_mu.data_ptr() if head_mu is not None else None),
         head_log_scale=(head_ls.data_ptr() if head_ls is not None else None), head_batch_stride=int(head_bs),
-        logits_dtype=(nat.logits_dtype_of(logits) if logits is not None else nat.DTYPE_F32))
+        logits_dtype=(nat.logits_dtype_of(logits) if logits is not None else nat.DTYPE_F32), head_dtype=head_dt)
     nat.check(nat.lib().ctdd_reverse_step(p, nat.stream()), "ctdd_reverse_step")
     return {"x": x_out, "rr": rr, "ratio": ratio}
 
 
 class _LogisticLogitsFn(torch.autograd.Function):
-    """Differentiable truncated-logistic head: forward `ctdd_logistic_logits`, backward `ctdd_logistic_logits_backward`
-    (recomputes the head from its two inputs; nothing of size (N, D, S) is saved)."""
+    """Differentiable truncated-logistic head: forward `ctdd_logistic_logits_ex`, backward `ctdd_logistic_logits_backward_ex`
+    (recomputes the head from its two inputs; nothing of size (N, D, S) is saved).
+
+    bf16 (mu, log_scale) are saved and read as they are, and a bf16 or fp32 incoming gradient is read as it is; other
+    dtypes are widened to fp32 copies.  The kernels widen on load, so the gradients equal those of the fp32 call on the
+    widened tensors bit for bit; they are returned in the inputs' dtypes."""
 
     @staticmethod
-    def forward(ctx, mu, log_scale, S, fix_logistic):
+    def forward(ctx, mu, log_scale, S, fix_logistic, out_dtype):
         N = mu.shape[0]
         D = mu.numel() // N
-        mu_c = mu.detach().reshape(N, D).contiguous().float()
-        ls_c = log_scale.detach().reshape(N, D).contiguous().float()
+        mu_c = mu.detach().reshape(N, D).contiguous()
+        ls_c = log_scale.detach().reshape(N, D).contiguous()
+        if not (mu_c.dtype == torch.bfloat16 and ls_c.dtype == torch.bfloat16):
+            mu_c, ls_c = mu_c.float(), ls_c.float()
         ctx.save_for_backward(mu_c, ls_c)
         ctx.meta = (S, bool(fix_logistic), tuple(mu.shape), mu.dtype, log_scale.dtype)
-        return logistic_logits(mu_c, ls_c, S, fix_logistic)
+        return logistic_logits(mu_c, ls_c, S, fix_logistic, out_dtype=out_dtype)
 
     @staticmethod
     @nat.on_tensor_device
@@ -126,18 +133,27 @@ class _LogisticLogitsFn(torch.autograd.Function):
         mu_c, ls_c = ctx.saved_tensors
         S, fix, shape, dt_mu, dt_ls = ctx.meta
         N, D = mu_c.shape
-        g = grad_logits.contiguous().float()
-        dmu, dls = torch.empty_like(mu_c), torch.empty_like(ls_c)
-        nat.check(nat.lib().ctdd_logistic_logits_backward(mu_c.data_ptr(), ls_c.data_ptr(), nat.ptr(g), N, D, D, S,
-                                                          1 if fix else 0, dmu.data_ptr(), dls.data_ptr(), nat.stream()),
-                  "ctdd_logistic_logits_backward")
-        return dmu.view(shape).to(dt_mu), dls.view(shape).to(dt_ls), None, None
+        g = grad_logits.contiguous()
+        if g.dtype not in (torch.float32, torch.bfloat16):
+            g = g.float()
+        elif g.dtype == torch.bfloat16 and g.data_ptr() % 8:
+            # the kernel's accumulation order depends on 4-element alignment: keep the order of an aligned fp32 gradient
+            g = g.clone()
+        dmu = torch.empty((N, D), dtype=torch.float32, device=mu_c.device)
+        dls = torch.empty_like(dmu)
+        nat.check(nat.lib().ctdd_logistic_logits_backward_ex(mu_c.data_ptr(), ls_c.data_ptr(), nat.logits_dtype_of(mu_c),
+                                                             nat.ptr(g), nat.logits_dtype_of(g), N, D, D, S,
+                                                             1 if fix else 0, dmu.data_ptr(), dls.data_ptr(), nat.stream()),
+                  "ctdd_logistic_logits_backward_ex")
+        return dmu.view(shape).to(dt_mu), dls.view(shape).to(dt_ls), None, None, None
 
 
 @nat.on_tensor_device
-def logistic_logits_autograd(mu, log_scale, S, fix_logistic=False):
-    """(N, D, S) logits of the head, differentiable w.r.t. mu and log_scale (training path)."""
-    return _LogisticLogitsFn.apply(mu, log_scale, S, fix_logistic)
+def logistic_logits_autograd(mu, log_scale, S, fix_logistic=False, out_dtype=None):
+    """(N, D, S) logits of the head, differentiable w.r.t. mu and log_scale (training path).  `out_dtype` is
+    torch.float32 (the default, None) or torch.bfloat16: the fp32 logits rounded once to bf16, which is what the
+    bf16 loss path (`loss_terms`) reads; its gradient then arrives as bf16 and is read as it is."""
+    return _LogisticLogitsFn.apply(mu, log_scale, S, fix_logistic, torch.float32 if out_dtype is None else out_dtype)
 
 
 # Opt-in for the un-materialised head: only code that knows how to consume an ops.LogisticHead (this package's samplers,
@@ -197,12 +213,16 @@ class LogisticHead:
 
 
 def _head_views(mu, ls, N, D):
-    """(mu, log_scale) as fp32 CUDA tensors addressable as base[n * batch_stride + d]; returns (mu, ls, batch_stride).
-    Accepts (N, D) or (N, C, H, W) tensors, contiguous or the two halves of torch.chunk(out, 2, dim=1)."""
+    """(mu, log_scale) as CUDA tensors addressable as base[n * batch_stride + d]; returns (mu, ls, batch_stride, dtype)
+    with dtype nat.DTYPE_BF16 when both are bf16 (read as they are; the kernels widen on load) and nat.DTYPE_F32
+    otherwise (any other dtype, or a bf16 / fp32 mix, is widened to fp32).  Accepts (N, D) or (N, C, H, W) tensors,
+    contiguous or the two halves of torch.chunk(out, 2, dim=1)."""
+    keep = mu.dtype == torch.bfloat16 and ls.dtype == torch.bfloat16
+
     def flat(t):
         if not t.is_cuda:
             raise RuntimeError("ctdd_b200 kernels need CUDA tensors; got a host tensor (there is no CPU fallback)")
-        if t.dtype != torch.float32:
+        if not keep and t.dtype != torch.float32:
             t = t.float()
         if t.shape[0] != N or t.numel() != N * D:
             raise ValueError(f"head tensor of shape {tuple(t.shape)} does not hold N={N} x D={D} values")
@@ -216,21 +236,30 @@ def _head_views(mu, ls, N, D):
     ls, bs_ls = flat(ls)
     if bs_mu != bs_ls:
         mu, ls, bs_mu = mu.contiguous(), ls.contiguous(), D
-    return mu, ls, bs_mu
+    return mu, ls, bs_mu, (nat.DTYPE_BF16 if keep else nat.DTYPE_F32)
+
+
+_OUT_DTYPES = {torch.float32: nat.DTYPE_F32, torch.bfloat16: nat.DTYPE_BF16}
 
 
 @nat.on_tensor_device
-def logistic_logits(mu, log_scale, S, fix_logistic=False, out=None):
-    """Truncated-logistic head -> (N, D, S) fp32 logits in one pass (replaces sample_logistic, models.py:28-74)."""
+def logistic_logits(mu, log_scale, S, fix_logistic=False, out=None, out_dtype=torch.float32):
+    """Truncated-logistic head -> (N, D, S) logits in one pass (replaces sample_logistic, models.py:28-74).
+
+    bf16 (mu, log_scale) are read as they are; the logits are computed in fp32 either way and stored as `out_dtype`
+    (torch.float32, or torch.bfloat16: rounded once to nearest even)."""
+    if out_dtype not in _OUT_DTYPES:
+        raise ValueError(f"logistic_logits: out_dtype must be torch.float32 or torch.bfloat16, got {out_dtype}")
     N = mu.shape[0]
     D = mu.numel() // N
-    mu, ls, bs = _head_views(mu, log_scale, N, D)
+    mu, ls, bs, in_dt = _head_views(mu, log_scale, N, D)
     if out is None:
-        out = torch.empty((N, D, S), dtype=torch.float32, device=mu.device)
-    elif out.shape != (N, D, S) or out.dtype != torch.float32:
-        raise ValueError(f"out must be a float32 ({N}, {D}, {S}) tensor")
-    nat.check(nat.lib().ctdd_logistic_logits(mu.data_ptr(), ls.data_ptr(), N, D, int(bs), S, 1 if fix_logistic else 0,
-                                             nat.ptr(out), nat.stream()), "ctdd_logistic_logits")
+        out = torch.empty((N, D, S), dtype=out_dtype, device=mu.device)
+    elif out.shape != (N, D, S) or out.dtype != out_dtype:
+        raise ValueError(f"out must be a {out_dtype} ({N}, {D}, {S}) tensor")
+    nat.check(nat.lib().ctdd_logistic_logits_ex(mu.data_ptr(), ls.data_ptr(), in_dt, N, D, int(bs), S,
+                                                1 if fix_logistic else 0, nat.ptr(out), _OUT_DTYPES[out_dtype],
+                                                nat.stream()), "ctdd_logistic_logits_ex")
     return out
 
 

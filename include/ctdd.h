@@ -137,8 +137,8 @@ typedef struct ctdd_step_params {
    * (lib/models/models.py:28-74, :248-282) on the fly, so the logits never exist in memory.  tcgen05 path (S == 256)
    * only; for other shapes materialise them with ctdd_logistic_logits first. */
   int32_t head;                 /* CTDD_HEAD_* */
-  const float* head_mu;         /* row (n,d) at head_mu[n*head_batch_stride + d] */
-  const float* head_log_scale;  /* same addressing */
+  const void* head_mu;          /* of head_dtype; row (n,d) at head_mu[n*head_batch_stride + d] */
+  const void* head_log_scale;   /* same type and addressing */
   int64_t head_batch_stride;    /* elements between consecutive n (2*D for the two halves of a torch.chunk'ed (B,2C,H,W)) */
   /* Element type of `logits` (appended field; zero-initialised = fp32).  CTDD_DTYPE_BF16 takes the logits a network run
    * under torch.autocast(dtype=torch.bfloat16) emits without a widening copy: the kernels widen on load (exact) and then
@@ -148,6 +148,12 @@ typedef struct ctdd_step_params {
    * not goes to the CUDA-core path under CTDD_IMPL_AUTO and is refused under CTDD_IMPL_TC.  Ignored unless
    * head == CTDD_HEAD_LOGITS. */
   int32_t logits_dtype;         /* CTDD_DTYPE_* */
+  /* Element type of head_mu / head_log_scale (appended field; zero-initialised = fp32).  CTDD_DTYPE_BF16 takes the
+   * (mu, log_scale) a U-Net run under torch.autocast(dtype=torch.bfloat16) emits without a widening copy: the kernels
+   * widen on load (exact) and then run the fp32 head and step arithmetic, so the states, counters, rr_out and ratio_out
+   * equal those of the same call on the widened (mu, log_scale) bit for bit.  Ignored when head == CTDD_HEAD_LOGITS;
+   * otherwise an unknown value is refused with status 2 before any CUDA call. */
+  int32_t head_dtype;           /* CTDD_DTYPE_* */
 } ctdd_step_params;
 
 enum {
@@ -172,6 +178,20 @@ int ctdd_logistic_logits(const float* mu, const float* log_scale, int N, int D, 
 int ctdd_logistic_logits_backward(const float* mu, const float* log_scale, const float* grad_logits, int N, int D,
                                   int64_t batch_stride, int S, int fix_logistic, float* grad_mu, float* grad_log_scale,
                                   void* stream);
+/* The two calls above with explicit element types (CTDD_DTYPE_F32 / CTDD_DTYPE_BF16; the calls above are these with
+ * fp32 everywhere).  bf16 mu / log_scale / grad_logits are widened on load (exact) and the fp32 arithmetic runs unchanged:
+ *   - ctdd_logistic_logits_ex: fp32 logits_out equal those of the fp32 call on the widened inputs bit for bit; bf16
+ *     logits_out are those values rounded once, to nearest even.  Four logits are stored at once when S % 4 == 0 and
+ *     logits_out is aligned to 4 elements (16 bytes fp32, 8 bytes bf16), one at a time otherwise;
+ *   - ctdd_logistic_logits_backward_ex: grad_mu / grad_log_scale stay fp32 (at the addressing of mu) and equal those of
+ *     the fp32 call on the widened tensors bit for bit, provided grad_logits is aligned to 4 of its elements whenever the
+ *     widened copy is 16-byte aligned (the accumulation order depends on that alignment, not on the type).
+ * An unknown dtype is refused with status 2 before any launch. */
+int ctdd_logistic_logits_ex(const void* mu, const void* log_scale, int in_dtype, int N, int D, int64_t batch_stride, int S,
+                            int fix_logistic, void* logits_out, int out_dtype, void* stream);
+int ctdd_logistic_logits_backward_ex(const void* mu, const void* log_scale, int in_dtype, const void* grad_logits,
+                                     int grad_dtype, int N, int D, int64_t batch_stride, int S, int fix_logistic,
+                                     float* grad_mu, float* grad_log_scale, void* stream);
 
 int64_t ctdd_step_workspace_bytes(int64_t rows, int S, int impl);
 int ctdd_reverse_step(const ctdd_step_params* p, void* stream);

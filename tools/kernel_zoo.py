@@ -102,6 +102,35 @@ def steps():
             report("widening copy + " + name, what + " bf16 logits through .float() and the fp32 step", timed(lambda: run(lgb.float())),
                    bytes_=2.0 * B * D * S + 8.0 * B * D, note="the copy reads 2 and writes 4 bytes per logit on top of the step")
         del lgb
+    # C4 with the truncated-logistic head fused into the step (the CIFAR10 configuration's head): the (mu, log_scale) pair
+    # as the two torch.chunk halves of a (B, 2D) network output, fp32, bf16 (a U-Net under torch.autocast), and bf16
+    # through the former per-step widening (.float() of the (B, 2D) output, then the fp32 head step)
+    w, model = model_for("C4")
+    S, D, B = w["S"], w["D"], w["B"]
+    Q, QT, beta = model.qt0_tables([0.5], dev)
+    Rb, RbT = model.base_rate_tables(dev)
+    branch = nat.branch_for(w["loss"], None)
+    tc = ops.prep_tc_tables(Q, QT, Rb, 1e-9, branch)
+    tcs = ops.prep_tc_static(Rb)
+    gen = torch.Generator(device=dev).manual_seed(5)
+    out32 = torch.cat([torch.tanh(torch.randn((B, D), generator=gen, device=dev)),
+                       0.5 * torch.randn((B, D), generator=gen, device=dev) - 1.0], 1)
+    out16 = out32.to(torch.bfloat16)
+    x = torch.randint(0, S, (B, D), generator=gen, device=dev, dtype=torch.int32)
+    h = (w["max_t"] - w["min_t"]) / w["num_steps"]
+    for mname, mode, kname in (("tau_leap", nat.MODE_TAU_LEAP, "step_q_kernel<HEAD>"), ("euler", nat.MODE_EULER, "step_tc_kernel<HEAD>")):
+        def run_head(out, widen=False):
+            mu_v, ls_v = torch.chunk(out.float() if widen else out, 2, dim=1)
+            ops.reverse_step(mode, branch, None, x, Q[0], QT[0], Rb, RbT, beta[0], h, 1e-9, N=B, D=D, S=S, seed=1, offset=0,
+                             tc_tables=tc[0], tc_static=tcs, head=(mu_v, ls_v, False))
+        what = f"C4: S={S} D={D} N={B} {mname} t=0.5, fused head"
+        report(kname, what, timed(lambda: run_head(out32)), bytes_=8.0 * B * D + 8.0 * B * D, flop=2.0 * B * D * S * S)
+        report(kname, what + " bf16 (mu, log_scale)", timed(lambda: run_head(out16)), bytes_=4.0 * B * D + 8.0 * B * D,
+               flop=2.0 * B * D * S * S)
+        report("widening copy + " + kname, what + " bf16 (mu, log_scale) through .float() and the fp32 step",
+               timed(lambda: run_head(out16, True)), bytes_=4.0 * B * D + 8.0 * B * D,
+               note="the copy reads 2 and writes 4 bytes per head parameter on top of the step")
+    del out32, out16
     # CUDA-core block kernel at S = 256 (SDDM direct branch / cross-check path), and the exact-posterior branch sizes
     w, model = model_for("C3")
     S, D, B = 256, 784, 64
@@ -190,20 +219,68 @@ def losses():
 
 
 def head():
+    # fp32 head; bf16 (mu, log_scale) with bf16 logits and a bf16 incoming gradient (a U-Net under torch.autocast feeding
+    # the bf16 loss path); and the former route for bf16 network output: .float() of mu / log_scale, then the fp32 head
     B, D, S = 128, 3072, 256
-    mu = torch.tanh(torch.randn(B, D, device=dev)).requires_grad_(True)
-    ls = torch.randn(B, D, device=dev).requires_grad_(True)
-    with torch.no_grad():
-        report("logistic_logits_kernel", f"head forward B={B} D={D} S=256", timed(lambda: ops.logistic_logits(mu, ls, S, False)),
-               bytes_=4.0 * B * D * S)
-    g = torch.randn(B, D, S, device=dev)
+    mu32 = torch.tanh(torch.randn(B, D, device=dev))
+    ls32 = torch.randn(B, D, device=dev)
+    g32 = torch.randn(B, D, S, device=dev)
+    for tag, dt, widen in (("", torch.float32, False), (" bf16 in / bf16 out / bf16 gradient", torch.bfloat16, False),
+                           (" bf16 in through .float(), fp32 head", torch.bfloat16, True)):
+        mu = mu32.to(dt).requires_grad_(True)
+        ls = ls32.to(dt).requires_grad_(True)
+        out_dt = torch.bfloat16 if (dt == torch.bfloat16 and not widen) else torch.float32
+        esz = 2 if out_dt == torch.bfloat16 else 4
+        g = g32.to(out_dt)
 
-    def fb():
-        out = ops.logistic_logits_autograd(mu, ls, S, False)
-        out.backward(g.view_as(out))
-        mu.grad = ls.grad = None
-    report("logistic_logits_kernel + logistic_backward_kernel", f"head forward + backward B={B} D={D} S=256", timed(fb),
-           bytes_=8.0 * B * D * S)
+        def fwd():
+            if widen:
+                return ops.logistic_logits_autograd(mu.float(), ls.float(), S, False)
+            return ops.logistic_logits_autograd(mu, ls, S, False, out_dtype=out_dt)
+        with torch.no_grad():
+            report("logistic_logits_kernel", f"head forward B={B} D={D} S=256{tag}", timed(fwd), bytes_=esz * B * D * S)
+
+        def fb():
+            out = fwd()
+            out.backward(g.view_as(out))
+            mu.grad = ls.grad = None
+        report("logistic_logits_kernel + logistic_backward_kernel", f"head forward + backward B={B} D={D} S=256{tag}",
+               timed(fb), bytes_=2.0 * esz * B * D * S)
+    del g32, g
+    # The image training leg: head + SDDMElbo loss terms (tensor-core path), forward + backward, from bf16 network output
+    # (torch.autocast) against the cast-to-fp32 route (fp32 head, fp32 logits into the loss, fp32 gradient back)
+    w, model = model_for("C5")
+    Rb, _ = model.base_rate_tables(dev)
+    for B in (64, 512):
+        gen = torch.Generator(device=dev).manual_seed(B)
+        Q, QT, beta = model.qt0_tables([0.05 + 0.9 * (i + 0.5) / B for i in range(B)], dev)
+        beta = torch.tensor([float(b) for b in beta], dtype=torch.float32, device=dev)
+        x0 = torch.randint(0, S, (B, D), generator=gen, device=dev, dtype=torch.int32)
+        _, xtil = ops.noise_xt(Q, Rb, beta, x0, 3, 0)
+        mu = torch.tanh(torch.randn(B, D, generator=gen, device=dev)).to(torch.bfloat16).requires_grad_(True)
+        ls = (torch.randn(B, D, generator=gen, device=dev) - 1.0).to(torch.bfloat16).requires_grad_(True)
+
+        def leg(widen):
+            if widen:
+                logits = ops.logistic_logits_autograd(mu.float(), ls.float(), S, False)
+            else:
+                logits = ops.logistic_logits_autograd(mu, ls, S, False, out_dtype=torch.bfloat16)
+            outs = ops.loss_terms(logits, nat.LOSS_SDDM, Q, QT, Rb, beta, x0, xtil, eps=1e-9,
+                                  logit_branch=nat.BRANCH_SDDM_REVERSE_PROB)
+            (outs[0].sum() + outs[1].sum() + 0.01 * outs[4].sum()).backward()
+            mu.grad = ls.grad = None
+
+        def peak(widen):
+            torch.cuda.synchronize()
+            base = torch.cuda.memory_allocated()
+            torch.cuda.reset_peak_memory_stats()
+            leg(widen)
+            torch.cuda.synchronize()
+            return torch.cuda.max_memory_allocated() - base
+        for tag, widen in ((" bf16 (mu, log_scale), bf16 logits", False), (" bf16 (mu, log_scale) through .float(), fp32 logits", True)):
+            report("head + SDDM loss_terms", f"image training leg B={B} D={D} S=256 forward + backward{tag}",
+                   timed(lambda: leg(widen)), note="torch autograd glue included", peak=peak(widen))
+        del Q, QT, mu, ls
 
 
 if __name__ == "__main__":
