@@ -41,12 +41,14 @@ extern "C" int ctdd_reverse_step(const ctdd_step_params* p, void* stream) {
   if (p->mode < CTDD_MODE_TAU_LEAP || p->mode > CTDD_MODE_EXACT) { set_error("ctdd_reverse_step: unknown mode %d", p->mode); return 2; }
   if (p->branch < CTDD_BRANCH_TAULDR || p->branch > CTDD_BRANCH_SDDM_REVERSE_LOGSCALE) { set_error("ctdd_reverse_step: unknown branch %d", p->branch); return 2; }
   if (p->head < CTDD_HEAD_LOGITS || p->head > CTDD_HEAD_LOGISTIC_FIX) { set_error("ctdd_reverse_step: unknown head %d", p->head); return 2; }
-  if (p->head == CTDD_HEAD_LOGITS && p->logits_dtype != CTDD_DTYPE_F32 && p->logits_dtype != CTDD_DTYPE_BF16) {
-    set_error("ctdd_reverse_step: unknown logits_dtype %d (CTDD_DTYPE_F32 = 0, CTDD_DTYPE_BF16 = 1)", p->logits_dtype);
+  if (p->head == CTDD_HEAD_LOGITS && p->logits_dtype != CTDD_DTYPE_F32 && p->logits_dtype != CTDD_DTYPE_BF16 &&
+      p->logits_dtype != CTDD_DTYPE_F16) {
+    set_error("ctdd_reverse_step: unknown logits_dtype %d (CTDD_DTYPE_F32 = 0, CTDD_DTYPE_BF16 = 1, CTDD_DTYPE_F16 = 2)",
+              p->logits_dtype);
     return 2;
   }
   if (p->head != CTDD_HEAD_LOGITS && p->head_dtype != CTDD_DTYPE_F32 && p->head_dtype != CTDD_DTYPE_BF16) {
-    set_error("ctdd_reverse_step: unknown head_dtype %d (CTDD_DTYPE_F32 = 0, CTDD_DTYPE_BF16 = 1)", p->head_dtype);
+    set_error("ctdd_reverse_step: head_dtype %d is not taken (CTDD_DTYPE_F32 = 0, CTDD_DTYPE_BF16 = 1)", p->head_dtype);
     return 2;
   }
   if (p->head == CTDD_HEAD_LOGITS ? !p->logits : (!p->head_mu || !p->head_log_scale || p->head_batch_stride < p->D)) {

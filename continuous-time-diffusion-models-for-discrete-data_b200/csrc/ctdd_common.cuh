@@ -3,7 +3,9 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <stdint.h>
+#include <type_traits>
 #include <math.h>
 #include "../../include/ctdd.h"
 
@@ -90,20 +92,41 @@ __device__ __forceinline__ Philox4 philox_keyed(uint32_t c0, uint32_t c1, uint32
   return o;
 }
 
-// Logits of the reverse step are fp32 or bf16 (ctdd_step_params::logits_dtype), and so are the truncated-logistic head's
-// (mu, log_scale) and incoming gradient.  Widening bf16 to fp32 is exact (the 16 bits are the upper half of the fp32
-// pattern), so a kernel that widens on load and then runs its fp32 code returns the results of the same call on the
-// widened inputs bit for bit.
+// Logits of the reverse step are fp32, bf16 or fp16 (ctdd_step_params::logits_dtype); the truncated-logistic head's
+// (mu, log_scale) are fp32 or bf16, its logits and incoming gradient fp32, bf16 or fp16.  Widening bf16 or fp16 to fp32
+// is exact (bf16: the 16 bits are the upper half of the fp32 pattern; fp16: the hardware conversion, subnormals
+// included), so a kernel that widens on load and then runs its fp32 code returns the results of the same call on the
+// widened inputs bit for bit.  The 2-byte types share one layout: only the widening differs.
 __device__ __forceinline__ float ld_logit(const float* p) { return __ldg(p); }
 __device__ __forceinline__ float ld_logit(const __nv_bfloat16* p) {
   return __uint_as_float((uint32_t)__ldg(reinterpret_cast<const unsigned short*>(p)) << 16);
+}
+// (loaded as 16 raw bits: with __ldg(const __half*) the fp16 loss_kernel<*, 32> spilled under its 128-register cap)
+__device__ __forceinline__ float ld_logit(const __half* p) {
+  return __half2float(__ushort_as_half(__ldg(reinterpret_cast<const unsigned short*>(p))));
 }
 // 4 consecutive bf16 (element 0 in the low half of w.x) -> fp32
 __device__ __forceinline__ void widen_bf16x4(uint2 w, float& v0, float& v1, float& v2, float& v3) {
   v0 = __uint_as_float(w.x << 16); v1 = __uint_as_float(w.x & 0xFFFF0000u);
   v2 = __uint_as_float(w.y << 16); v3 = __uint_as_float(w.y & 0xFFFF0000u);
 }
+// 4 consecutive fp16 (element 0 in the low half of w.x) -> fp32
+__device__ __forceinline__ void widen_f16x4(uint2 w, float& v0, float& v1, float& v2, float& v3) {
+  const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&w.x));
+  const float2 b = __half22float2(*reinterpret_cast<const __half2*>(&w.y));
+  v0 = a.x; v1 = a.y; v2 = b.x; v3 = b.y;
+}
+// 4 consecutive elements of the 2-byte type LT -> fp32
+template <typename LT>
+__device__ __forceinline__ void widen2x4(uint2 w, float& v0, float& v1, float& v2, float& v3) {
+  static_assert(sizeof(LT) == 2, "widen2x4 widens 2-byte types");
+  if constexpr (std::is_same<LT, __half>::value) widen_f16x4(w, v0, v1, v2, v3);
+  else widen_bf16x4(w, v0, v1, v2, v3);
+}
 #endif
+
+// bytes of one element of a CTDD_DTYPE_* type
+inline size_t dtype_bytes(int t) { return t == CTDD_DTYPE_F32 ? 4 : 2; }
 
 // Tau-leap draws of one GLOBAL row: the states are cut into chunks of JUMP_CHUNK consecutive states; chunk q draws its
 // own total and picks from Philox calls (q << 16) + c of the row's stream, counter = (call, grow, offset_lo, stream | ...).

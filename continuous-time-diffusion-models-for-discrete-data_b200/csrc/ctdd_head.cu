@@ -26,7 +26,8 @@ __device__ __forceinline__ void logsig_pair(float z, float& log_u, float& log_v,
   log_v = fminf(-z, 0.f) - ld;
 }
 
-// Stores of the forward kernel: fp32, or bf16 rounded once to nearest even (VEC = 4: one 16-byte / one 8-byte store).
+// Stores of the forward kernel: fp32, or bf16 / fp16 rounded once to nearest even (VEC = 4: one 16-byte / one 8-byte
+// store).
 __device__ __forceinline__ void st_logits4(float* p, const float (&o)[4]) {
   *reinterpret_cast<float4*>(p) = make_float4(o[0], o[1], o[2], o[3]);
 }
@@ -35,21 +36,30 @@ __device__ __forceinline__ void st_logits4(__nv_bfloat16* p, const float (&o)[4]
   const __nv_bfloat162 hi = __halves2bfloat162(__float2bfloat16_rn(o[2]), __float2bfloat16_rn(o[3]));
   *reinterpret_cast<uint2*>(p) = make_uint2(*reinterpret_cast<const uint32_t*>(&lo), *reinterpret_cast<const uint32_t*>(&hi));
 }
+__device__ __forceinline__ void st_logits4(__half* p, const float (&o)[4]) {
+  const __half2 lo = __halves2half2(__float2half_rn(o[0]), __float2half_rn(o[1]));
+  const __half2 hi = __halves2half2(__float2half_rn(o[2]), __float2half_rn(o[3]));
+  *reinterpret_cast<uint2*>(p) = make_uint2(*reinterpret_cast<const uint32_t*>(&lo), *reinterpret_cast<const uint32_t*>(&hi));
+}
 __device__ __forceinline__ void st_logit(float* p, float o) { *p = o; }
 __device__ __forceinline__ void st_logit(__nv_bfloat16* p, float o) { *p = __float2bfloat16_rn(o); }
+__device__ __forceinline__ void st_logit(__half* p, float o) { *p = __float2half_rn(o); }
 
-// Incoming gradient of the backward kernel, widened on load: VEC = 4 reads one 16-byte (fp32) or 8-byte (bf16) word.
+// Incoming gradient of the backward kernel, widened on load: VEC = 4 reads one 16-byte (fp32) or 8-byte (bf16, fp16)
+// word.
 __device__ __forceinline__ void ld_grad4(const float* p, float (&gr)[4]) {
   const float4 q = __ldg(reinterpret_cast<const float4*>(p));
   gr[0] = q.x; gr[1] = q.y; gr[2] = q.z; gr[3] = q.w;
 }
-__device__ __forceinline__ void ld_grad4(const __nv_bfloat16* p, float (&gr)[4]) {
-  widen_bf16x4(__ldg(reinterpret_cast<const uint2*>(p)), gr[0], gr[1], gr[2], gr[3]);
+template <typename GT>
+__device__ __forceinline__ void ld_grad4(const GT* p, float (&gr)[4]) {     // the 2-byte types
+  widen2x4<GT>(__ldg(reinterpret_cast<const uint2*>(p)), gr[0], gr[1], gr[2], gr[3]);
 }
 
 // one thread per VEC consecutive states of a row (VEC + 1 bin edges); row scalars are recomputed per thread.
-// IT: type of mu / log_scale, OT: type of the logits (float or __nv_bfloat16); bf16 inputs are widened on load (exact),
-// every logit is computed in fp32 as for fp32 inputs, and a bf16 output is that value rounded once at the store.
+// IT: type of mu / log_scale (float or __nv_bfloat16), OT: type of the logits (float, __nv_bfloat16 or __half); bf16
+// inputs are widened on load (exact), every logit is computed in fp32 as for fp32 inputs, and a 2-byte output is that
+// value rounded once at the store.
 template <int VEC, typename IT, typename OT>
 __global__ void __launch_bounds__(256) logistic_logits_kernel(const IT* __restrict__ mu, const IT* __restrict__ log_scale,
                                                               long long rows, int D, long long batch_stride, int S, int fix,
@@ -97,9 +107,9 @@ __global__ void __launch_bounds__(256) logistic_logits_kernel(const IT* __restri
 //     d/dmu = inv (-v_{s+1} + kappa u_s v_s / A),   d/dls = -z_{s+1} v_{s+1} + (kappa u_s v_s z_s - w (1-kappa) v_s) / A
 //   logits_2 = log v_s + log B,      B = kappa u_{s+1} + 1e-6
 //     d/dmu = inv (u_s - kappa u_{s+1} v_{s+1} / B), d/dls = z_s u_s - (kappa u_{s+1} v_{s+1} z_{s+1} + w (1-kappa) u_{s+1}) / B
-// IT: type of mu / log_scale, GT: type of grad_logits (float or __nv_bfloat16), both widened on load.  A bf16 gradient is
-// read with the VEC, lane -> state assignment and accumulation order of the fp32 one, so the results equal those of the
-// fp32 kernel on the widened tensors bit for bit.  dmu / dls are fp32.
+// IT: type of mu / log_scale (float or __nv_bfloat16), GT: type of grad_logits (float, __nv_bfloat16 or __half), both
+// widened on load.  A 2-byte gradient is read with the VEC, lane -> state assignment and accumulation order of the fp32
+// one, so the results equal those of the fp32 kernel on the widened tensors bit for bit.  dmu / dls are fp32.
 template <int VEC, typename IT, typename GT>
 __global__ void __launch_bounds__(256) logistic_backward_kernel(const IT* __restrict__ mu, const IT* __restrict__ log_scale,
                                                                 const GT* __restrict__ grad_logits, long long rows, int D,
@@ -185,8 +195,20 @@ void launch_backward(const void* mu, const void* log_scale, const void* grad, lo
     logistic_backward_kernel<1, IT, GT><<<blocks, 256, 0, st>>>(m, l, g, rows, D, batch_stride, S, fix, dmu, dls);
 }
 
-bool known_dtype(int t) { return t == CTDD_DTYPE_F32 || t == CTDD_DTYPE_BF16; }
-size_t dtype_bytes(int t) { return t == CTDD_DTYPE_BF16 ? 2 : 4; }
+// (mu, log_scale) are fp32 or bf16; the logits and their gradient also fp16
+bool known_in_dtype(int t) { return t == CTDD_DTYPE_F32 || t == CTDD_DTYPE_BF16; }
+bool known_logits_dtype(int t) { return known_in_dtype(t) || t == CTDD_DTYPE_F16; }
+
+template <typename IT>
+decltype(&launch_logits<IT, float>) logits_launcher(int out_dtype) {
+  return out_dtype == CTDD_DTYPE_BF16 ? launch_logits<IT, __nv_bfloat16>
+                                      : (out_dtype == CTDD_DTYPE_F16 ? launch_logits<IT, __half> : launch_logits<IT, float>);
+}
+template <typename IT>
+decltype(&launch_backward<IT, float>) backward_launcher(int grad_dtype) {
+  return grad_dtype == CTDD_DTYPE_BF16 ? launch_backward<IT, __nv_bfloat16>
+                                       : (grad_dtype == CTDD_DTYPE_F16 ? launch_backward<IT, __half> : launch_backward<IT, float>);
+}
 
 }  // namespace
 }  // namespace ctdd
@@ -196,8 +218,9 @@ extern "C" int ctdd_logistic_logits_ex(const void* mu, const void* log_scale, in
                                        void* stream) {
   using namespace ctdd;
   if (!mu || !log_scale || !logits_out) { set_error("ctdd_logistic_logits: null pointer"); return 2; }
-  if (!known_dtype(in_dtype) || !known_dtype(out_dtype)) {
-    set_error("ctdd_logistic_logits: unknown dtype in=%d out=%d (CTDD_DTYPE_F32 = 0, CTDD_DTYPE_BF16 = 1)", in_dtype, out_dtype);
+  if (!known_in_dtype(in_dtype) || !known_logits_dtype(out_dtype)) {
+    set_error("ctdd_logistic_logits: unknown dtype in=%d out=%d (in: CTDD_DTYPE_F32 = 0, CTDD_DTYPE_BF16 = 1; out: also "
+              "CTDD_DTYPE_F16 = 2)", in_dtype, out_dtype);
     return 2;
   }
   if (N <= 0 || D <= 0 || S < 2 || batch_stride < D) { set_error("ctdd_logistic_logits: bad sizes N=%d D=%d S=%d stride=%lld", N, D, S, (long long)batch_stride); return 2; }
@@ -205,13 +228,11 @@ extern "C" int ctdd_logistic_logits_ex(const void* mu, const void* log_scale, in
   int dev = 0, sms = 148;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  // VEC = 4 stores 4 logits at once: 16 bytes (fp32) or 8 bytes (bf16), so the output must be aligned to that
+  // VEC = 4 stores 4 logits at once: 16 bytes (fp32) or 8 bytes (bf16, fp16), so the output must be aligned to that
   const bool vec4 = (S % 4 == 0) && ((reinterpret_cast<uintptr_t>(logits_out) & (4 * dtype_bytes(out_dtype) - 1)) == 0);
   long long blocks = ((vec4 ? total / 4 : total) + 255) / 256;
   if (blocks > (long long)sms * 16) blocks = (long long)sms * 16;
-  auto launch = (in_dtype == CTDD_DTYPE_BF16)
-                    ? (out_dtype == CTDD_DTYPE_BF16 ? launch_logits<__nv_bfloat16, __nv_bfloat16> : launch_logits<__nv_bfloat16, float>)
-                    : (out_dtype == CTDD_DTYPE_BF16 ? launch_logits<float, __nv_bfloat16> : launch_logits<float, float>);
+  auto launch = (in_dtype == CTDD_DTYPE_BF16) ? logits_launcher<__nv_bfloat16>(out_dtype) : logits_launcher<float>(out_dtype);
   launch(mu, log_scale, rows, D, batch_stride, S, fix_logistic, logits_out, vec4, (unsigned)blocks, (cudaStream_t)stream);
   CTDD_CHECK_LAUNCH("logistic_logits_kernel");
   return 0;
@@ -227,8 +248,9 @@ extern "C" int ctdd_logistic_logits_backward_ex(const void* mu, const void* log_
                                                 float* grad_mu, float* grad_log_scale, void* stream) {
   using namespace ctdd;
   if (!mu || !log_scale || !grad_logits || !grad_mu || !grad_log_scale) { set_error("ctdd_logistic_logits_backward: null pointer"); return 2; }
-  if (!known_dtype(in_dtype) || !known_dtype(grad_dtype)) {
-    set_error("ctdd_logistic_logits_backward: unknown dtype in=%d grad=%d (CTDD_DTYPE_F32 = 0, CTDD_DTYPE_BF16 = 1)", in_dtype, grad_dtype);
+  if (!known_in_dtype(in_dtype) || !known_logits_dtype(grad_dtype)) {
+    set_error("ctdd_logistic_logits_backward: unknown dtype in=%d grad=%d (in: CTDD_DTYPE_F32 = 0, CTDD_DTYPE_BF16 = 1; "
+              "grad: also CTDD_DTYPE_F16 = 2)", in_dtype, grad_dtype);
     return 2;
   }
   if (N <= 0 || D <= 0 || S < 2 || batch_stride < D) { set_error("ctdd_logistic_logits_backward: bad sizes N=%d D=%d S=%d stride=%lld", N, D, S, (long long)batch_stride); return 2; }
@@ -238,11 +260,9 @@ extern "C" int ctdd_logistic_logits_backward_ex(const void* mu, const void* log_
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   long long blocks = (rows + 7) / 8;      // 8 warps per block, one row per warp per iteration
   if (blocks > (long long)sms * 8) blocks = (long long)sms * 8;
-  // VEC = 4 reads 4 gradient entries at once: 16 bytes (fp32) or 8 bytes (bf16)
+  // VEC = 4 reads 4 gradient entries at once: 16 bytes (fp32) or 8 bytes (bf16, fp16)
   const bool vec4 = (S % 4 == 0) && ((reinterpret_cast<uintptr_t>(grad_logits) & (4 * dtype_bytes(grad_dtype) - 1)) == 0);
-  auto launch = (in_dtype == CTDD_DTYPE_BF16)
-                    ? (grad_dtype == CTDD_DTYPE_BF16 ? launch_backward<__nv_bfloat16, __nv_bfloat16> : launch_backward<__nv_bfloat16, float>)
-                    : (grad_dtype == CTDD_DTYPE_BF16 ? launch_backward<float, __nv_bfloat16> : launch_backward<float, float>);
+  auto launch = (in_dtype == CTDD_DTYPE_BF16) ? backward_launcher<__nv_bfloat16>(grad_dtype) : backward_launcher<float>(grad_dtype);
   launch(mu, log_scale, grad_logits, rows, D, batch_stride, S, fix_logistic, grad_mu, grad_log_scale, vec4, (unsigned)blocks,
          (cudaStream_t)stream);
   CTDD_CHECK_LAUNCH("logistic_backward_kernel");

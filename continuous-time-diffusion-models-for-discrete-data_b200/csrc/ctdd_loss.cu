@@ -10,10 +10,11 @@
 // Q once per 8 rows and was L2-bandwidth bound at ~15 TFLOP/s); other S keep ROWS = 8.  The k order of every dot
 // product is the same in both forms, so the results are bit-identical.
 // Per-sample reductions are returned as [B] vectors; the final means / weights are combined by the Python classes.
-// Logits and their gradient are fp32 or bf16 (ctdd_loss_params::logits_dtype; template argument LT of every kernel that
-// touches them).  bf16 is widened on load, which is exact, and the fp32 code runs unchanged; the gradient is rounded once
-// (round-to-nearest-even) when it is stored.  A bf16 call therefore returns the per-sample terms of the same call on the
-// widened logits (bit for bit up to the order of the cross-CTA atomicAdds) and that call's gradient rounded to bf16.
+// Logits and their gradient are fp32, bf16 or fp16 (ctdd_loss_params::logits_dtype; template argument LT of every kernel
+// that touches them).  The 2-byte types are widened on load, which is exact, and the fp32 code runs unchanged; the
+// gradient is rounded once (round-to-nearest-even) when it is stored.  A bf16 or fp16 call therefore returns the
+// per-sample terms of the same call on the widened logits (bit for bit up to the order of the cross-CTA atomicAdds) and
+// that call's gradient rounded to the logits' type.
 #include "ctdd_common.cuh"
 
 namespace ctdd {
@@ -196,16 +197,17 @@ __device__ __forceinline__ void rows_times_matrix(const float* __restrict__ in, 
   }
 }
 
-// One logits element as fp32.  fp32 keeps a plain load (ld_logit's __ldg would change the fp32 kernels' code); bf16 is
-// widened by ld_logit.
+// One logits element as fp32.  fp32 keeps a plain load (ld_logit's __ldg would change the fp32 kernels' code); bf16 and
+// fp16 are widened by ld_logit.
 template <typename LT>
 __device__ __forceinline__ float logit_at(const LT* p) {
   if constexpr (sizeof(LT) == 4) return *p;
   else return ld_logit(p);
 }
-// One gradient element: fp32 stored as it is, bf16 rounded to nearest even.
+// One gradient element: fp32 stored as it is, bf16 and fp16 rounded to nearest even.
 __device__ __forceinline__ void st_grad(float* p, float v) { *p = v; }
 __device__ __forceinline__ void st_grad(__nv_bfloat16* p, float v) { *p = __float2bfloat16_rn(v); }
+__device__ __forceinline__ void st_grad(__half* p, float v) { *p = __float2half_rn(v); }
 
 template <bool BWD, int ROWS, typename LT = float>
 __global__ void __launch_bounds__(256, ROWS == 32 ? 2 : 1) loss_kernel(const Args a) {
@@ -418,9 +420,9 @@ __global__ void __launch_bounds__(256, ROWS == 32 ? 2 : 1) loss_kernel(const Arg
 //   tc_terms_kernel u from bufU: the per-(row, s) terms and their per-sample sums            (forward)
 //                   or the cotangent V = dL/du -> bufA                                        (backward)
 //   tc_post_kernel  dp = V Q^T from bufU: softmax Jacobian + cross-entropy gradient -> grad   (backward)
-// The arithmetic per element is loss_kernel's (phases 1, 3 and 5).  With bf16 logits (LT) tc_pre_kernel and
+// The arithmetic per element is loss_kernel's (phases 1, 3 and 5).  With bf16 or fp16 logits (LT) tc_pre_kernel and
 // tc_post_kernel read a row as two 8-byte loads per lane and tc_post_kernel stores the gradient as two 8-byte stores of
-// packed bf16; lanes own the same states, and the scratch (bufA, bufU, lse, fix) stays fp32.
+// packed 2-byte values; lanes own the same states, and the scratch (bufA, bufU, lse, fix) stays fp32.
 constexpr int TC_S = 256;
 constexpr int TC_ROWS = 32;      // rows of ONE sample per CTA (8 warps x 4 rows): one atomicAdd per CTA and output
 
@@ -433,19 +435,25 @@ __device__ __forceinline__ void store_row8(float* p, int lane, const float (&v)[
   reinterpret_cast<float4*>(p)[lane] = make_float4(v[0], v[1], v[2], v[3]);
   reinterpret_cast<float4*>(p + 128)[lane] = make_float4(v[4], v[5], v[6], v[7]);
 }
-__device__ __forceinline__ Row8 load_row8(const __nv_bfloat16* p, int lane) {
+template <typename LT>
+__device__ __forceinline__ Row8 load_row8(const LT* p, int lane) {     // the 2-byte types
   const uint2 a = __ldg(reinterpret_cast<const uint2*>(p) + lane), b = __ldg(reinterpret_cast<const uint2*>(p + 128) + lane);
   Row8 r;
-  widen_bf16x4(a, r.v[0], r.v[1], r.v[2], r.v[3]);
-  widen_bf16x4(b, r.v[4], r.v[5], r.v[6], r.v[7]);
+  widen2x4<LT>(a, r.v[0], r.v[1], r.v[2], r.v[3]);
+  widen2x4<LT>(b, r.v[4], r.v[5], r.v[6], r.v[7]);
   return r;
 }
-__device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {     // lo -> low half, round-to-nearest-even
+// two values rounded to nearest even, packed (lo -> low half)
+__device__ __forceinline__ uint32_t pack2(__nv_bfloat16*, float lo, float hi) {
   return (uint32_t)__bfloat16_as_ushort(__float2bfloat16_rn(lo)) | ((uint32_t)__bfloat16_as_ushort(__float2bfloat16_rn(hi)) << 16);
 }
-__device__ __forceinline__ void store_row8(__nv_bfloat16* p, int lane, const float (&v)[8]) {
-  reinterpret_cast<uint2*>(p)[lane] = make_uint2(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]));
-  reinterpret_cast<uint2*>(p + 128)[lane] = make_uint2(pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
+__device__ __forceinline__ uint32_t pack2(__half*, float lo, float hi) {
+  return (uint32_t)__half_as_ushort(__float2half_rn(lo)) | ((uint32_t)__half_as_ushort(__float2half_rn(hi)) << 16);
+}
+template <typename LT>
+__device__ __forceinline__ void store_row8(LT* p, int lane, const float (&v)[8]) {     // the 2-byte types
+  reinterpret_cast<uint2*>(p)[lane] = make_uint2(pack2(p, v[0], v[1]), pack2(p, v[2], v[3]));
+  reinterpret_cast<uint2*>(p + 128)[lane] = make_uint2(pack2(p, v[4], v[5]), pack2(p, v[6], v[7]));
 }
 __device__ __forceinline__ int state_of(int lane, int e) { return (e < 4 ? 0 : 128) + 4 * lane + (e & 3); }
 // value of element `s` of a row held as Row8 across the warp
@@ -625,14 +633,35 @@ __global__ void __launch_bounds__(256) tc_post_kernel(const Args a) {
 }  // namespace ctdd
 
 namespace {
+template <typename LT>
+void reserve_loss_smem() {
+  using ctdd::loss::loss_kernel;
+  cudaFuncSetAttribute(loss_kernel<false, 8, LT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+  cudaFuncSetAttribute(loss_kernel<true, 8, LT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+  cudaFuncSetAttribute(loss_kernel<false, 32, LT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+  cudaFuncSetAttribute(loss_kernel<true, 32, LT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+}
+
+template <typename LT>
+void launch_loss_kernel(const ctdd::loss::Args& a, bool bwd, int ROWS, dim3 grid, int threads, size_t smem, cudaStream_t st) {
+  using ctdd::loss::loss_kernel;
+  if (ROWS == 32) {
+    if (bwd) loss_kernel<true, 32, LT><<<grid, threads, smem, st>>>(a);
+    else loss_kernel<false, 32, LT><<<grid, threads, smem, st>>>(a);
+  } else {
+    if (bwd) loss_kernel<true, 8, LT><<<grid, threads, smem, st>>>(a);
+    else loss_kernel<false, 8, LT><<<grid, threads, smem, st>>>(a);
+  }
+}
+
 int run_loss(const ctdd_loss_params* p, void* stream, bool bwd) {
   using namespace ctdd;
   using namespace ctdd::loss;
   if (!p) { set_error("ctdd_loss: null params"); return 2; }
   if (p->B <= 0 || p->D <= 0 || p->S < 2) { set_error("ctdd_loss: bad sizes"); return 2; }
   if (p->kind < CTDD_LOSS_CTELBO || p->kind > CTDD_LOSS_SDDM) { set_error("ctdd_loss: unknown kind %d", p->kind); return 2; }
-  if (p->logits_dtype != CTDD_DTYPE_F32 && p->logits_dtype != CTDD_DTYPE_BF16) {
-    set_error("ctdd_loss: unknown logits_dtype %d (CTDD_DTYPE_F32 = 0, CTDD_DTYPE_BF16 = 1)", p->logits_dtype);
+  if (p->logits_dtype != CTDD_DTYPE_F32 && p->logits_dtype != CTDD_DTYPE_BF16 && p->logits_dtype != CTDD_DTYPE_F16) {
+    set_error("ctdd_loss: unknown logits_dtype %d (CTDD_DTYPE_F32 = 0, CTDD_DTYPE_BF16 = 1, CTDD_DTYPE_F16 = 2)", p->logits_dtype);
     return 2;
   }
   if (!p->logits || !p->Q || !p->QT || !p->Rb || !p->beta || !p->x0 || !p->xt) { set_error("ctdd_loss: null input"); return 2; }
@@ -645,8 +674,8 @@ int run_loss(const ctdd_loss_params* p, void* stream, bool bwd) {
   if (bwd && (!p->ga || !p->gb || !p->gd || !p->gn || !p->grad_logits)) { set_error("ctdd_loss_backward: null gradient pointer"); return 2; }
   if (!bwd && (!p->out_a || !p->out_b || !p->out_c || !p->out_d || !p->out_nll)) { set_error("ctdd_loss_forward: null output pointer"); return 2; }
   // S == 256, SDDM / CRM kinds with a scratch buffer: the tensor-core path (below).  Its streaming kernels read the logits
-  // and write the gradient in 16-byte (fp32) / 8-byte (bf16) pieces per lane: both must be 16-byte aligned.
-  const bool bf16 = p->logits_dtype == CTDD_DTYPE_BF16;
+  // and write the gradient in 16-byte (fp32) / 8-byte (bf16, fp16) pieces per lane: both must be 16-byte aligned.
+  const int dt = p->logits_dtype;
   const bool tc_path = p->S == 256 && p->tc_scratch && p->kind != CTDD_LOSS_CTELBO && p->logit_type != CTDD_BRANCH_SDDM_DIRECT;
   if (tc_path && ((reinterpret_cast<uintptr_t>(p->logits) | (bwd ? reinterpret_cast<uintptr_t>(p->grad_logits) : 0)) & 15)) {
     set_error("ctdd_loss: logits and grad_logits must be 16-byte aligned on the tensor-core path (S = 256, tc_scratch)");
@@ -661,14 +690,9 @@ int run_loss(const ctdd_loss_params* p, void* stream, bool bwd) {
   int dev = 0;
   cudaGetDevice(&dev);
   if (dev < 0 || dev >= 64 || !((attr_done >> dev) & 1ull)) {
-    cudaFuncSetAttribute(loss_kernel<false, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    cudaFuncSetAttribute(loss_kernel<true, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    cudaFuncSetAttribute(loss_kernel<false, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    cudaFuncSetAttribute(loss_kernel<true, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    cudaFuncSetAttribute(loss_kernel<false, 8, __nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    cudaFuncSetAttribute(loss_kernel<true, 8, __nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    cudaFuncSetAttribute(loss_kernel<false, 32, __nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    cudaFuncSetAttribute(loss_kernel<true, 32, __nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    reserve_loss_smem<float>();
+    reserve_loss_smem<__nv_bfloat16>();
+    reserve_loss_smem<__half>();
     if (dev >= 0 && dev < 64) attr_done |= 1ull << dev;
   }
   Args a;
@@ -711,7 +735,8 @@ int run_loss(const ctdd_loss_params* p, void* stream, bool bwd) {
     a.fix = a.lse + (size_t)p->B * p->D;
     dim3 tgrid((p->D + TC_ROWS - 1) / TC_ROWS, p->B);
     if (!bwd) {
-      if (bf16) tc_pre_kernel<__nv_bfloat16><<<tgrid, 256, 0, st>>>(a);
+      if (dt == CTDD_DTYPE_BF16) tc_pre_kernel<__nv_bfloat16><<<tgrid, 256, 0, st>>>(a);
+      else if (dt == CTDD_DTYPE_F16) tc_pre_kernel<__half><<<tgrid, 256, 0, st>>>(a);
       else tc_pre_kernel<<<tgrid, 256, 0, st>>>(a);
       CTDD_CHECK_LAUNCH("tc_pre_kernel");
       if (int rc = ctdd_bgemm256_tc(a.bufA, p->QT, p->B, p->D, a.bufU, stream)) return rc;      // u[s] = sum_k p[k] Q[k][s]
@@ -725,7 +750,8 @@ int run_loss(const ctdd_loss_params* p, void* stream, bool bwd) {
       } else {
         if (int rc = ctdd_bgemm256_tc(a.bufA, p->Q, p->B, p->D, a.bufU, stream)) return rc;     // dp[k] = sum_s V[s] Q[k][s]
       }
-      if (bf16) tc_post_kernel<__nv_bfloat16><<<tgrid, 256, 0, st>>>(a);
+      if (dt == CTDD_DTYPE_BF16) tc_post_kernel<__nv_bfloat16><<<tgrid, 256, 0, st>>>(a);
+      else if (dt == CTDD_DTYPE_F16) tc_post_kernel<__half><<<tgrid, 256, 0, st>>>(a);
       else tc_post_kernel<<<tgrid, 256, 0, st>>>(a);
       CTDD_CHECK_LAUNCH("tc_post_kernel");
     }
@@ -736,23 +762,9 @@ int run_loss(const ctdd_loss_params* p, void* stream, bool bwd) {
   if (threads > 256) threads = 256;
   if (threads < 64) threads = 64;
   dim3 grid((p->D + ROWS - 1) / ROWS, p->B);
-  if (ROWS == 32) {
-    if (bf16) {
-      if (bwd) loss_kernel<true, 32, __nv_bfloat16><<<grid, threads, smem, st>>>(a);
-      else loss_kernel<false, 32, __nv_bfloat16><<<grid, threads, smem, st>>>(a);
-    } else {
-      if (bwd) loss_kernel<true, 32><<<grid, threads, smem, st>>>(a);
-      else loss_kernel<false, 32><<<grid, threads, smem, st>>>(a);
-    }
-  } else {
-    if (bf16) {
-      if (bwd) loss_kernel<true, 8, __nv_bfloat16><<<grid, threads, smem, st>>>(a);
-      else loss_kernel<false, 8, __nv_bfloat16><<<grid, threads, smem, st>>>(a);
-    } else {
-      if (bwd) loss_kernel<true, 8><<<grid, threads, smem, st>>>(a);
-      else loss_kernel<false, 8><<<grid, threads, smem, st>>>(a);
-    }
-  }
+  if (dt == CTDD_DTYPE_BF16) launch_loss_kernel<__nv_bfloat16>(a, bwd, ROWS, grid, threads, smem, st);
+  else if (dt == CTDD_DTYPE_F16) launch_loss_kernel<__half>(a, bwd, ROWS, grid, threads, smem, st);
+  else launch_loss_kernel<float>(a, bwd, ROWS, grid, threads, smem, st);
   CTDD_CHECK_LAUNCH("loss_kernel");
   return 0;
 }

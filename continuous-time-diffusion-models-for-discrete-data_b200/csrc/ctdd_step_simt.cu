@@ -28,7 +28,7 @@ struct StepArgs {
   int mode, branch, D, S, reject_multi;
   long long rows;        // N*D
   long long row_offset;  // multiple of 8
-  const void* logits;    // fp32 or bf16 (the kernel's logits-type template argument)
+  const void* logits;    // fp32, bf16 or fp16 (the kernel's logits-type template argument)
   long long ld, batch_stride;
   const int* x_eval;
   const int* x_base;
@@ -146,7 +146,8 @@ constexpr int SMALL_MINB = 8;
 constexpr unsigned SMALL_GRIDCAP = 64u;   // CTAs per SM of the capped grid
 // LEAN: the launch has dense logits and no rr_out / ratio_out (the samplers' call): the strided-row loads and the
 // (predicated, but issued) rate stores drop out as well.
-// LT: element type of the logits, float or __nv_bfloat16 (widened on load; everything after the load is the fp32 code).
+// LT: element type of the logits, float, __nv_bfloat16 or __half (widened on load; everything after the load is the fp32
+// code).
 template <int S, int MODE = -1, int BRANCH = -1, bool LEAN = false, typename LT = float>
 __global__ void __launch_bounds__(128, (LEAN && S == 2 && MODE == CTDD_MODE_TAU_LEAP) ? SMALL_MINB : 0) step_small_kernel(StepArgs a_in) {
   StepArgs a = a_in;
@@ -193,11 +194,11 @@ __global__ void __launch_bounds__(128, (LEAN && S == 2 && MODE == CTDD_MODE_TAU_
     g += (long long)gridDim.x * blockDim.x;
     const int nr = (a.rows - r0) < 8 ? (int)(a.rows - r0) : 8;
     float lg[8][S];
-    // (bf16: the 16-byte loads also need a 16-byte aligned tensor; r0 * S * 2 is a multiple of 16)
+    // (2-byte types: the 16-byte loads also need a 16-byte aligned tensor; r0 * S * 2 is a multiple of 16)
     const bool contiguous = (a.ld == S) && (a.batch_stride == (long long)a.D * S) && nr == 8 &&
                             (sizeof(LT) == 4 || (reinterpret_cast<uintptr_t>(a.logits) & 15) == 0);
     if (contiguous) {
-      if constexpr (sizeof(LT) == 2) {     // 8 rows of S bf16: S 16-byte loads
+      if constexpr (sizeof(LT) == 2) {     // 8 rows of S 2-byte elements: S 16-byte loads
         const uint4* p = reinterpret_cast<const uint4*>(static_cast<const LT*>(a.logits) + r0 * S);
         uint4 buf[S];
 #pragma unroll
@@ -205,8 +206,8 @@ __global__ void __launch_bounds__(128, (LEAN && S == 2 && MODE == CTDD_MODE_TAU_
         float f[8 * S];
 #pragma unroll
         for (int i = 0; i < S; ++i) {
-          widen_bf16x4(make_uint2(buf[i].x, buf[i].y), f[8 * i], f[8 * i + 1], f[8 * i + 2], f[8 * i + 3]);
-          widen_bf16x4(make_uint2(buf[i].z, buf[i].w), f[8 * i + 4], f[8 * i + 5], f[8 * i + 6], f[8 * i + 7]);
+          widen2x4<LT>(make_uint2(buf[i].x, buf[i].y), f[8 * i], f[8 * i + 1], f[8 * i + 2], f[8 * i + 3]);
+          widen2x4<LT>(make_uint2(buf[i].z, buf[i].w), f[8 * i + 4], f[8 * i + 5], f[8 * i + 6], f[8 * i + 7]);
         }
 #pragma unroll
         for (int r = 0; r < 8; ++r)
@@ -489,7 +490,7 @@ __global__ void __launch_bounds__(128, (LEAN && S == 2 && MODE == CTDD_MODE_TAU_
 // terms), small per-row scalars.
 constexpr int BLK_ROWS = 8;
 
-// LT: element type of the logits, float or __nv_bfloat16 (every logits load goes through ld_logit)
+// LT: element type of the logits, float, __nv_bfloat16 or __half (every logits load goes through ld_logit)
 template <typename LT = float>
 __global__ void __launch_bounds__(256) step_block_kernel(StepArgs a) {
   extern __shared__ float smem[];
@@ -657,7 +658,7 @@ __global__ void __launch_bounds__(256) step_block_kernel(StepArgs a) {
   flush_stats(st, a.stats);
 }
 
-// The small-S dispatch table, the same for both logits types.
+// The small-S dispatch table, the same for every logits type.
 template <typename LT>
 void launch_step_small(const StepArgs& a, int S, bool lean, unsigned blocks, int threads, cudaStream_t st) {
   switch (S) {
@@ -704,14 +705,15 @@ int launch_step_simt(const ctdd_step_params* p, cudaStream_t st) {
   a.x_out = p->x_out; a.rr_out = p->rr_out; a.ratio_out = p->ratio_out;
   a.stats = reinterpret_cast<unsigned long long*>(p->stats_out);
   philox_key_schedule(p->seed, a.pk);
-  const bool bf16 = p->logits_dtype == CTDD_DTYPE_BF16;
+  const int dt = p->logits_dtype;
   const int S = p->S;
   if (S <= 8 && S >= 2) {
     const long long groups = (a.rows + 7) / 8;
     const int threads = 128;
     unsigned blocks = (unsigned)((groups + threads - 1) / threads);
     const bool lean = !a.rr_out && !a.ratio_out && a.ld == S && a.batch_stride == (long long)a.D * S;
-    if (bf16) launch_step_small<__nv_bfloat16>(a, S, lean, blocks, threads, st);
+    if (dt == CTDD_DTYPE_BF16) launch_step_small<__nv_bfloat16>(a, S, lean, blocks, threads, st);
+    else if (dt == CTDD_DTYPE_F16) launch_step_small<__half>(a, S, lean, blocks, threads, st);
     else launch_step_small<float>(a, S, lean, blocks, threads, st);
     CTDD_CHECK_LAUNCH("step_small_kernel");
     return 0;
@@ -724,13 +726,15 @@ int launch_step_simt(const ctdd_step_params* p, cudaStream_t st) {
   if (dev < 0 || dev >= 64 || !((attr_done >> dev) & 1ull)) {
     cudaFuncSetAttribute(step_block_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
     cudaFuncSetAttribute(step_block_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    cudaFuncSetAttribute(step_block_kernel<__half>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
     if (dev >= 0 && dev < 64) attr_done |= 1ull << dev;
   }
   int threads = ((S + 31) / 32) * 32;
   if (threads > 256) threads = 256;
   if (threads < 64) threads = 64;
   const unsigned blocks = (unsigned)((a.rows + BLK_ROWS - 1) / BLK_ROWS);
-  if (bf16) step_block_kernel<__nv_bfloat16><<<blocks, threads, smem, st>>>(a);
+  if (dt == CTDD_DTYPE_BF16) step_block_kernel<__nv_bfloat16><<<blocks, threads, smem, st>>>(a);
+  else if (dt == CTDD_DTYPE_F16) step_block_kernel<__half><<<blocks, threads, smem, st>>>(a);
   else step_block_kernel<float><<<blocks, threads, smem, st>>>(a);
   CTDD_CHECK_LAUNCH("step_block_kernel");
   return 0;

@@ -67,7 +67,7 @@ struct Smem {
   alignas(1024) uint8_t stage[STAGES][STAGE_BYTES];
   alignas(16) float gather[GBUF][NH][S];   // [row owned by this CTA][state]: accumulator values, then prefix sums
   Side side[RING][NH];
-  alignas(16) float lring[NUM_PROD_WARPS][LRING][2][S];   // raw logits rows, one pass ahead of their use (bf16: the
+  alignas(16) float lring[NUM_PROD_WARPS][LRING][2][S];   // raw logits rows, one pass ahead of their use (2-byte: the
                                                           // row pair packed into the first half of the slot)
   alignas(8) uint64_t full[STAGES];  // leader CTA: its 8 producer warps + 1 relayed arrival for the partner's 8
   uint64_t full_local[STAGES];       // partner CTA: its 8 producer warps; the partner's idle MMA warp relays the phase
@@ -108,11 +108,12 @@ __device__ __forceinline__ float widen_head(unsigned short v) { return __uint_as
 // ---------------------------------------------------------------------------------------------- the kernel
 // TAULDR: tauLDR rates (else SDDM reverse_prob); CORR: the corrector variant adds h * R_t[x,:] to the rates;
 // HEAD: the rows' softmax numerators come from the truncated-logistic head (mu, log_scale per row) instead of logits;
-// LT: element type of the logits, float or __nv_bfloat16 (a bf16 row pair travels packed, 2*S bytes per row, and is
-// widened on the producers' shared-memory load; the arithmetic after that load is the fp32 kernel's).  A HEAD kernel reads
-// no logits: LT is then the type of (mu, log_scale), widened on the producers' load
+// LT: element type of the logits, float, __nv_bfloat16 or __half (a 2-byte row pair travels packed, 2*S bytes per row,
+// and is widened on the producers' shared-memory load; the arithmetic after that load is the fp32 kernel's).  A HEAD
+// kernel reads no logits: LT is then the type of (mu, log_scale), float or __nv_bfloat16, widened on the producers' load
 template <bool TAULDR, bool CORR, bool HEAD, typename LT = float>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step_tc_kernel(const Args a) {
+  static_assert(!(HEAD && std::is_same<LT, __half>::value), "the fused head takes fp32 or bf16 (mu, log_scale)");
   constexpr uint32_t ROW_BYTES = S * sizeof(LT);
   extern __shared__ uint8_t smem_raw[];
   // aligned by offsetting the shared array itself (not through an integer): the compiler keeps `sm` a shared-space
@@ -287,7 +288,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
           // lane l16 widens the same elements 64c + 4*l16 .. +3 as in the fp32 kernel, one 64-bit load each
           const uint32_t src = smem_u32(&sm.lring[pw][rslot][0][0]) + half * ROW_BYTES + 8 * l16;
 #pragma unroll
-          for (int c = 0; c < 4; ++c) widen_bf16x4(lds64(src + 128 * c), v[4 * c], v[4 * c + 1], v[4 * c + 2], v[4 * c + 3]);
+          for (int c = 0; c < 4; ++c) widen2x4<LT>(lds64(src + 128 * c), v[4 * c], v[4 * c + 1], v[4 * c + 2], v[4 * c + 3]);
         } else {
           const uint32_t src = smem_u32(&sm.lring[pw][rslot][half][4 * l16]);
 #pragma unroll
@@ -664,8 +665,8 @@ bool tc_supports(const ctdd_step_params* p) {
         p->mode == CTDD_MODE_RATES_ONLY))
     return false;
   if (!p->tc_tables || !p->tc_static) return false;
-  // rows are bulk-copied: 16-byte aligned (4 fp32 or 8 bf16 elements)
-  const int64_t row_align = p->logits_dtype == CTDD_DTYPE_BF16 ? 7 : 3;
+  // rows are bulk-copied: 16-byte aligned (4 fp32 or 8 bf16 / fp16 elements)
+  const int64_t row_align = (int64_t)(16 / dtype_bytes(p->logits_dtype)) - 1;
   if (p->head == CTDD_HEAD_LOGITS &&
       ((p->ld_logits & row_align) || (p->batch_stride_logits & row_align) || (reinterpret_cast<uintptr_t>(p->logits) & 15)))
     return false;
@@ -688,18 +689,21 @@ int launch_step_tc(const ctdd_step_params* p, cudaStream_t st) {
   const size_t smem_bytes = sizeof(Smem) + 1024;
   typedef void (*kern_t)(const Args);
 #define CTDD_TC_ROW(T, H, LT) step_tc_kernel<T, false, H, LT>, step_tc_kernel<T, true, H, LT>
-  static const kern_t kerns[16] = {CTDD_TC_ROW(false, false, float), CTDD_TC_ROW(true, false, float),
+  static const kern_t kerns[20] = {CTDD_TC_ROW(false, false, float), CTDD_TC_ROW(true, false, float),
                                      CTDD_TC_ROW(false, true, float), CTDD_TC_ROW(true, true, float),
                                      CTDD_TC_ROW(false, false, __nv_bfloat16), CTDD_TC_ROW(true, false, __nv_bfloat16),
-                                     CTDD_TC_ROW(false, true, __nv_bfloat16), CTDD_TC_ROW(true, true, __nv_bfloat16)};
+                                     CTDD_TC_ROW(false, true, __nv_bfloat16), CTDD_TC_ROW(true, true, __nv_bfloat16),
+                                     CTDD_TC_ROW(false, false, __half), CTDD_TC_ROW(true, false, __half)};
 #undef CTDD_TC_ROW
   Args a = make_args(p);
   a.num_tiles = (int)((a.rows + NT - 1) / NT);
   const int pairs = pair_count(launch_state, "ctdd_reverse_step", kerns, smem_bytes, a.num_tiles);
   if (!pairs) return 1;
-  // rows of kerns: fp32 logits, fused head on fp32 (mu, log_scale), bf16 logits, fused head on bf16 (mu, log_scale)
+  // rows of kerns: fp32 logits, fused head on fp32 (mu, log_scale), bf16 logits, fused head on bf16 (mu, log_scale),
+  // fp16 logits (the head takes no fp16: ctdd_reverse_step refuses it)
+  const int dt = p->head != CTDD_HEAD_LOGITS ? p->head_dtype : p->logits_dtype;
   const int ki = ((p->branch == CTDD_BRANCH_TAULDR) ? 1 : 0) + (p->head != CTDD_HEAD_LOGITS ? 2 : 0) +
-                 ((p->head != CTDD_HEAD_LOGITS ? p->head_dtype : p->logits_dtype) == CTDD_DTYPE_BF16 ? 4 : 0);
+                 (dt == CTDD_DTYPE_BF16 ? 4 : (dt == CTDD_DTYPE_F16 ? 8 : 0));
   const int kj = (p->mode == CTDD_MODE_EULER_CORR) ? 1 : 0;
   kerns[2 * ki + kj]<<<2 * pairs, NUM_THREADS, smem_bytes, st>>>(a);
   CTDD_CHECK_LAUNCH("step_tc_kernel");

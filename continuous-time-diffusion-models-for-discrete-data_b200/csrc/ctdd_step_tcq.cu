@@ -82,7 +82,7 @@ constexpr uint32_t CONTRIB_TX_BYTES = (NUM_EPI_WARPS / 2) * 2 * 32 * 4;   // rec
 struct Smem {
   alignas(1024) uint8_t stage[STAGES][STAGE_BYTES];
   alignas(16) float lring[LRING][NPW][2][S];   // raw logits rows, LRING passes of every producer warp ahead of their use
-                                               // (bf16: a round's 8 rows packed into the first half of its group's slots)
+                                               // (2-byte: a round's 8 rows packed into the first half of its group's slots)
   alignas(16) float2 scal_c[RING][NT];         // (c1, c0) of the tile's rows: rows 0..63 from CTA 0, 64..127 from CTA 1
   uint32_t scal_x[RING][NT];                   // chunk mask of the band (bits 0-7) | valid << 8 | x << 10 (= table-row byte offset)
   alignas(16) float scratch[NUM_EPI_WARPS][32][SCR_LD];   // per epilogue warp: lam[row][state of the chunk] (lane = state -> lane = row)
@@ -109,11 +109,12 @@ static_assert(RING > STAGES + ACC + CBUF, "row-scalar ring shorter than the pipe
 
 // TAULDR: tauLDR rates (else SDDM reverse_prob); KM: KM_JUMP / KM_CORR / KM_RATES / KM_DRIFT;
 // HEAD: the rows' softmax numerators come from the truncated-logistic head (mu, log_scale per row) instead of logits;
-// LT: element type of the logits, float or __nv_bfloat16 (bf16 rows travel packed, 2*S bytes each, and are widened on
-// the producers' shared-memory load; the arithmetic after that load is the fp32 kernel's).  A HEAD kernel reads no logits:
-// LT is then the type of (mu, log_scale), widened on the loader warp's load
+// LT: element type of the logits, float, __nv_bfloat16 or __half (2-byte rows travel packed, 2*S bytes each, and are
+// widened on the producers' shared-memory load; the arithmetic after that load is the fp32 kernel's).  A HEAD kernel reads
+// no logits: LT is then the type of (mu, log_scale), float or __nv_bfloat16, widened on the loader warp's load
 template <bool TAULDR, int KM, bool HEAD, typename LT = float>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step_q_kernel(const Args a) {
+  static_assert(!(HEAD && std::is_same<LT, __half>::value), "the fused head takes fp32 or bf16 (mu, log_scale)");
   constexpr uint32_t ROW_BYTES = S * sizeof(LT);
   extern __shared__ uint8_t smem_raw[];
   Smem& sm = *reinterpret_cast<Smem*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
@@ -260,12 +261,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) step
         head_numerators_rec(hr, a.head_fix != 0, l16, v);
       } else {
         if constexpr (sizeof(LT) == 2) {
-          // the round's 8 bf16 rows lie packed from the group's first slot: this half's row is number 2 * (pw % GSZ) + half;
+          // the round's 8 2-byte rows lie packed from the group's first slot: this half's row is number 2 * (pw % GSZ) + half;
           // lane l16 widens the same elements 64c + 4*l16 .. +3 as in the fp32 kernel, one 64-bit load each
           const uint32_t src = smem_u32(&sm.lring[rslot][pw - pw % GSZ][0][0]) + (uint32_t)(2 * (pw % GSZ) + half) * ROW_BYTES +
                                8 * l16;
 #pragma unroll
-          for (int c = 0; c < 4; ++c) widen_bf16x4(lds64(src + 128 * c), v[4 * c], v[4 * c + 1], v[4 * c + 2], v[4 * c + 3]);
+          for (int c = 0; c < 4; ++c) widen2x4<LT>(lds64(src + 128 * c), v[4 * c], v[4 * c + 1], v[4 * c + 2], v[4 * c + 3]);
         } else {
           const uint32_t src = smem_u32(&sm.lring[rslot][pw][half][4 * l16]);
 #pragma unroll
@@ -826,10 +827,11 @@ int launch_step_tcq(const ctdd_step_params* p, cudaStream_t st) {
 #define CTDD_TCQ_ROW(T, H, LT)                                                                                            \
   step_q_kernel<T, tc::KM_JUMP, H, LT>, step_q_kernel<T, tc::KM_CORR, H, LT>, step_q_kernel<T, tc::KM_RATES, H, LT>,    \
       step_q_kernel<T, tc::KM_DRIFT, H, LT>
-  static const kern_t kerns[32] = {CTDD_TCQ_ROW(false, false, float), CTDD_TCQ_ROW(true, false, float),
+  static const kern_t kerns[40] = {CTDD_TCQ_ROW(false, false, float), CTDD_TCQ_ROW(true, false, float),
                                      CTDD_TCQ_ROW(false, true, float), CTDD_TCQ_ROW(true, true, float),
                                      CTDD_TCQ_ROW(false, false, __nv_bfloat16), CTDD_TCQ_ROW(true, false, __nv_bfloat16),
-                                     CTDD_TCQ_ROW(false, true, __nv_bfloat16), CTDD_TCQ_ROW(true, true, __nv_bfloat16)};
+                                     CTDD_TCQ_ROW(false, true, __nv_bfloat16), CTDD_TCQ_ROW(true, true, __nv_bfloat16),
+                                     CTDD_TCQ_ROW(false, false, __half), CTDD_TCQ_ROW(true, false, __half)};
 #undef CTDD_TCQ_ROW
   if (reinterpret_cast<uintptr_t>(p->tc_static) % tc::ST_ALIGN) {
     set_error("ctdd_reverse_step: tc_static must be aligned to ctdd_tc_static_align() = %zu bytes", tc::ST_ALIGN);
@@ -843,9 +845,11 @@ int launch_step_tcq(const ctdd_step_params* p, cudaStream_t st) {
   a.num_tiles = (int)((a.rows + NT - 1) / NT);
   const int pairs = tc::pair_count(launch_state, "ctdd_reverse_step", kerns, smem_bytes, a.num_tiles);
   if (!pairs) return 1;
-  // rows of kerns: fp32 logits, fused head on fp32 (mu, log_scale), bf16 logits, fused head on bf16 (mu, log_scale)
+  // rows of kerns: fp32 logits, fused head on fp32 (mu, log_scale), bf16 logits, fused head on bf16 (mu, log_scale),
+  // fp16 logits (the head takes no fp16: ctdd_reverse_step refuses it)
+  const int dt = p->head != CTDD_HEAD_LOGITS ? p->head_dtype : p->logits_dtype;
   const int ki = ((p->branch == CTDD_BRANCH_TAULDR) ? 1 : 0) + (p->head != CTDD_HEAD_LOGITS ? 2 : 0) +
-                 ((p->head != CTDD_HEAD_LOGITS ? p->head_dtype : p->logits_dtype) == CTDD_DTYPE_BF16 ? 4 : 0);
+                 (dt == CTDD_DTYPE_BF16 ? 4 : (dt == CTDD_DTYPE_F16 ? 8 : 0));
   int kj = 0;
   if (p->mode == CTDD_MODE_RATES_ONLY) kj = 2;
   else if (p->mode == CTDD_MODE_TAU_LEAP_CORR) kj = 1;

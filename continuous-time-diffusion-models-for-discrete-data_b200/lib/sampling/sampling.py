@@ -96,8 +96,8 @@ class StepEngine:
         return self._t_all[tidx]
 
     def _fast_step(self, mode, logits, x_eval, tidx, h, reject_multi, x_base, row):
-        """The common case of step(): dense contiguous fp32 / bf16 logits or an un-materialised head (fp32 or bf16
-        (mu, log_scale)), state update only."""
+        """The common case of step(): dense contiguous fp32 / bf16 / fp16 logits or an un-materialised head (fp32 or
+        bf16 (mu, log_scale)), state update only."""
         N, D, S = self.N, self.D, self.S
         p = self._p
         if isinstance(logits, ops.LogisticHead):
@@ -109,7 +109,7 @@ class StepEngine:
         else:
             p.head, p.head_mu, p.head_log_scale, p.head_batch_stride = nat.HEAD_LOGITS, None, None, 0
             p.logits = logits.data_ptr()
-            # the struct is reused across calls, whose logits may alternate between fp32 and bf16
+            # the struct is reused across calls, whose logits may alternate between fp32, bf16 and fp16
             p.logits_dtype = nat.logits_dtype_of(logits)
         xe = x_eval.data_ptr()
         xb = x_base.data_ptr() if x_base is not None else 0
@@ -150,7 +150,7 @@ class StepEngine:
                 and (x_base is None or (x_base.dtype == torch.int32 and x_base.is_contiguous()))
                 and torch.cuda.current_device() == (self.device.index or 0)
                 and ((head is not None and self.tc_tables is not None)
-                     or (head is None and logits.dtype in (torch.float32, torch.bfloat16) and logits.is_contiguous()
+                     or (head is None and logits.dtype in ops._LOGITS_DTYPES and logits.is_contiguous()
                          and logits.is_cuda)))
         if fast:
             x_out = self._fast_step(mode, ops.LogisticHead(*head) if head is not None else logits, x_eval, tidx, h,
@@ -204,7 +204,7 @@ def _dense(logits, S):
 
 def _final_argmax(model, x, min_t, N, device):
     out = model(x.long(), min_t * torch.ones((N,), device=device))
-    p_0gt = F.softmax(_dense(out, getattr(model, "S", None)), dim=2, dtype=torch.float32)   # bf16 logits: fp32 ties as for fp32
+    p_0gt = F.softmax(_dense(out, getattr(model, "S", None)), dim=2, dtype=torch.float32)   # 2-byte logits: fp32 ties as for fp32
     return torch.max(p_0gt, dim=2)[1]
 
 

@@ -8,6 +8,10 @@ import torch
 
 from . import _native as nat
 
+# dtypes of (N, D, S) logits and of their gradients that the kernels read and write as they are (2-byte ones are widened
+# on load, exactly); any other dtype is widened to an fp32 copy first
+_LOGITS_DTYPES = (torch.float32, torch.bfloat16, torch.float16)
+
 
 @nat.on_tensor_device
 def build_qt0(U, Uinv, lam, d_int, normalize=True, clamp_below=1e-8, want_transpose=False):
@@ -61,8 +65,8 @@ def reverse_step(mode, branch, logits, x_eval, Q, QT, Rb, RbT, beta, h, eps, *, 
     `head=(mu, log_scale, fix_logistic)` replaces `logits` (pass None) by the parameters of the truncated-logistic
     output head (reference lib/models/models.py:248-282): mu / log_scale are (N, D)-shaped views whose batch
     stride may exceed D (the two torch.chunk halves of a (B, 2C, H, W) network output), fp32, or bf16 both (read as
-    they are).  On the tcgen05 path the logits are never materialised; elsewhere they are built once with
-    `logistic_logits`, as fp32."""
+    they are; any other dtype is widened to fp32).  On the tcgen05 path the logits are never materialised; elsewhere
+    they are built once with `logistic_logits`, as fp32.  Dense `logits` are read as they are in fp32, bf16 or fp16."""
     dev = x_eval.device
     head_kind, head_mu, head_ls, head_bs, head_dt = nat.HEAD_LOGITS, None, None, 0, nat.DTYPE_F32
     if head is not None:
@@ -76,7 +80,7 @@ def reverse_step(mode, branch, logits, x_eval, Q, QT, Rb, RbT, beta, h, eps, *, 
         else:
             logits = logistic_logits(mu, ls, S, fix)
     if logits is not None:
-        if logits.dtype not in (torch.float32, torch.bfloat16):     # bf16 is read as it is (widened on load, exactly)
+        if logits.dtype not in _LOGITS_DTYPES:     # bf16 / fp16 are read as they are (widened on load, exactly)
             logits = logits.float()
         logits = logits.contiguous()
     if mode == nat.MODE_RATES_ONLY:
@@ -111,8 +115,8 @@ class _LogisticLogitsFn(torch.autograd.Function):
     """Differentiable truncated-logistic head: forward `ctdd_logistic_logits_ex`, backward `ctdd_logistic_logits_backward_ex`
     (recomputes the head from its two inputs; nothing of size (N, D, S) is saved).
 
-    bf16 (mu, log_scale) are saved and read as they are, and a bf16 or fp32 incoming gradient is read as it is; other
-    dtypes are widened to fp32 copies.  The kernels widen on load, so the gradients equal those of the fp32 call on the
+    bf16 (mu, log_scale) are saved and read as they are, and an fp32, bf16 or fp16 incoming gradient is read as it is;
+    other dtypes are widened to fp32 copies.  The kernels widen on load, so the gradients equal those of the fp32 call on the
     widened tensors bit for bit; they are returned in the inputs' dtypes."""
 
     @staticmethod
@@ -134,9 +138,9 @@ class _LogisticLogitsFn(torch.autograd.Function):
         S, fix, shape, dt_mu, dt_ls = ctx.meta
         N, D = mu_c.shape
         g = grad_logits.contiguous()
-        if g.dtype not in (torch.float32, torch.bfloat16):
+        if g.dtype not in _LOGITS_DTYPES:
             g = g.float()
-        elif g.dtype == torch.bfloat16 and g.data_ptr() % 8:
+        elif g.dtype != torch.float32 and g.data_ptr() % 8:
             # the kernel's accumulation order depends on 4-element alignment: keep the order of an aligned fp32 gradient
             g = g.clone()
         dmu = torch.empty((N, D), dtype=torch.float32, device=mu_c.device)
@@ -151,8 +155,9 @@ class _LogisticLogitsFn(torch.autograd.Function):
 @nat.on_tensor_device
 def logistic_logits_autograd(mu, log_scale, S, fix_logistic=False, out_dtype=None):
     """(N, D, S) logits of the head, differentiable w.r.t. mu and log_scale (training path).  `out_dtype` is
-    torch.float32 (the default, None) or torch.bfloat16: the fp32 logits rounded once to bf16, which is what the
-    bf16 loss path (`loss_terms`) reads; its gradient then arrives as bf16 and is read as it is."""
+    torch.float32 (the default, None), torch.bfloat16 or torch.float16: the fp32 logits rounded once to that type,
+    which is what the 2-byte loss path (`loss_terms`) reads; its gradient then arrives in that type and is read as it
+    is."""
     return _LogisticLogitsFn.apply(mu, log_scale, S, fix_logistic, torch.float32 if out_dtype is None else out_dtype)
 
 
@@ -239,7 +244,7 @@ def _head_views(mu, ls, N, D):
     return mu, ls, bs_mu, (nat.DTYPE_BF16 if keep else nat.DTYPE_F32)
 
 
-_OUT_DTYPES = {torch.float32: nat.DTYPE_F32, torch.bfloat16: nat.DTYPE_BF16}
+_OUT_DTYPES = {torch.float32: nat.DTYPE_F32, torch.bfloat16: nat.DTYPE_BF16, torch.float16: nat.DTYPE_F16}
 
 
 @nat.on_tensor_device
@@ -247,9 +252,9 @@ def logistic_logits(mu, log_scale, S, fix_logistic=False, out=None, out_dtype=to
     """Truncated-logistic head -> (N, D, S) logits in one pass (replaces sample_logistic, models.py:28-74).
 
     bf16 (mu, log_scale) are read as they are; the logits are computed in fp32 either way and stored as `out_dtype`
-    (torch.float32, or torch.bfloat16: rounded once to nearest even)."""
+    (torch.float32, or torch.bfloat16 / torch.float16: rounded once to nearest even)."""
     if out_dtype not in _OUT_DTYPES:
-        raise ValueError(f"logistic_logits: out_dtype must be torch.float32 or torch.bfloat16, got {out_dtype}")
+        raise ValueError(f"logistic_logits: out_dtype must be torch.float32, torch.bfloat16 or torch.float16, got {out_dtype}")
     N = mu.shape[0]
     D = mu.numel() // N
     mu, ls, bs, in_dt = _head_views(mu, log_scale, N, D)
@@ -405,9 +410,10 @@ class _LossTerms(torch.autograd.Function):
     """Per-sample loss terms (out_a, out_b, out_c, out_d, out_nll), each (B,), differentiable w.r.t. `logits`
     through the fused backward kernel (include/ctdd.h: ctdd_loss_forward / ctdd_loss_backward).
 
-    fp32 and bf16 logits are read as they are; bf16 ones (a network under torch.autocast(dtype=torch.bfloat16)) get a
-    bf16 gradient, equal to the fp32 gradient of their widening rounded to bf16.  Other dtypes are widened to an fp32
-    copy and autograd casts the gradient back."""
+    fp32, bf16 and fp16 logits are read as they are; bf16 and fp16 ones (a network under torch.autocast, with
+    dtype=torch.bfloat16 or its default fp16) get a gradient of their own dtype, equal to the fp32 gradient of their
+    widening rounded once to that dtype (fp16: +-inf where it overflows, which a GradScaler detects).  Other dtypes are
+    widened to an fp32 copy and autograd casts the gradient back."""
     #: S == 256: run the two contractions on tcgen05 (set False to force the CUDA-core kernel, e.g. as a cross-check)
     use_tc = True
 
@@ -415,7 +421,7 @@ class _LossTerms(torch.autograd.Function):
     def forward(ctx, logits, kind, logit_branch, crm_type, Q, QT, Rb, beta, x0, xt, x_tilde, eps):
         B, D, S = logits.shape
         dev = logits.device
-        if logits.dtype == torch.bfloat16:
+        if logits.dtype in (torch.bfloat16, torch.float16):
             logits = logits.contiguous()
             if logits.data_ptr() % 16:          # e.g. a contiguous view at an odd storage offset: 16-byte rows needed
                 logits = logits.clone()
@@ -452,7 +458,7 @@ class _LossTerms(torch.autograd.Function):
         B, D, S = logits.shape
         z = lambda g: (g if g is not None else torch.zeros((B,), device=logits.device)).contiguous().float()
         ga, gb, gd, gn = z(ga), z(gb), z(gd), z(gn)
-        grad = torch.empty_like(logits)             # the logits' dtype: bf16 logits get a bf16 gradient
+        grad = torch.empty_like(logits)             # the logits' dtype: bf16 / fp16 logits get a bf16 / fp16 gradient
         p = nat.LossParams(kind=kind, logit_type=logit_branch, crm_type=crm_type, B=B, D=D, S=S,
                            logits=nat.ptr(logits), Q=nat.ptr(Q), QT=nat.ptr(QT), Rb=nat.ptr(Rb), beta=nat.ptr(beta),
                            x0=nat.ptr(x0), xt=nat.ptr(xt), x_tilde=(nat.ptr(x_tilde) if has_tilde else None), eps=eps,

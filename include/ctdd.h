@@ -140,25 +140,27 @@ typedef struct ctdd_step_params {
   const void* head_mu;          /* of head_dtype; row (n,d) at head_mu[n*head_batch_stride + d] */
   const void* head_log_scale;   /* same type and addressing */
   int64_t head_batch_stride;    /* elements between consecutive n (2*D for the two halves of a torch.chunk'ed (B,2C,H,W)) */
-  /* Element type of `logits` (appended field; zero-initialised = fp32).  CTDD_DTYPE_BF16 takes the logits a network run
-   * under torch.autocast(dtype=torch.bfloat16) emits without a widening copy: the kernels widen on load (exact) and then
-   * run the fp32 arithmetic, so the states, counters, rr_out and ratio_out equal those of the same call on the widened
-   * logits bit for bit.  The outputs stay fp32 / int32.  The tcgen05 path (S == 256) needs 16-byte aligned rows:
-   * logits 16-byte aligned, ld_logits and batch_stride_logits multiples of 8 bf16 elements (4 fp32 ones); a view that is
-   * not goes to the CUDA-core path under CTDD_IMPL_AUTO and is refused under CTDD_IMPL_TC.  Ignored unless
-   * head == CTDD_HEAD_LOGITS. */
+  /* Element type of `logits` (appended field; zero-initialised = fp32): fp32, bf16 or fp16.  CTDD_DTYPE_BF16 and
+   * CTDD_DTYPE_F16 take the logits a network run under torch.autocast (bf16 or its default fp16) emits without a widening
+   * copy: the kernels widen on load (exact) and then run the fp32 arithmetic, so the states, counters, rr_out and
+   * ratio_out equal those of the same call on the widened logits bit for bit.  The outputs stay fp32 / int32.  The
+   * tcgen05 path (S == 256) needs 16-byte aligned rows: logits 16-byte aligned, ld_logits and batch_stride_logits
+   * multiples of 8 elements for the 2-byte types (4 for fp32); a view that is not goes to the CUDA-core path under
+   * CTDD_IMPL_AUTO and is refused under CTDD_IMPL_TC.  Ignored unless head == CTDD_HEAD_LOGITS. */
   int32_t logits_dtype;         /* CTDD_DTYPE_* */
   /* Element type of head_mu / head_log_scale (appended field; zero-initialised = fp32).  CTDD_DTYPE_BF16 takes the
    * (mu, log_scale) a U-Net run under torch.autocast(dtype=torch.bfloat16) emits without a widening copy: the kernels
    * widen on load (exact) and then run the fp32 head and step arithmetic, so the states, counters, rr_out and ratio_out
-   * equal those of the same call on the widened (mu, log_scale) bit for bit.  Ignored when head == CTDD_HEAD_LOGITS;
-   * otherwise an unknown value is refused with status 2 before any CUDA call. */
+   * equal those of the same call on the widened (mu, log_scale) bit for bit.  fp32 or bf16 only: fp16 (mu, log_scale)
+   * are O(N*D) and are widened by the caller.  Ignored when head == CTDD_HEAD_LOGITS; otherwise any other value is
+   * refused with status 2 before any CUDA call. */
   int32_t head_dtype;           /* CTDD_DTYPE_* */
 } ctdd_step_params;
 
 enum {
   CTDD_DTYPE_F32 = 0,          /* float32 logits */
-  CTDD_DTYPE_BF16 = 1          /* bfloat16 logits */
+  CTDD_DTYPE_BF16 = 1,         /* bfloat16 logits */
+  CTDD_DTYPE_F16 = 2           /* float16 (IEEE half) logits */
 };
 
 enum {
@@ -178,15 +180,18 @@ int ctdd_logistic_logits(const float* mu, const float* log_scale, int N, int D, 
 int ctdd_logistic_logits_backward(const float* mu, const float* log_scale, const float* grad_logits, int N, int D,
                                   int64_t batch_stride, int S, int fix_logistic, float* grad_mu, float* grad_log_scale,
                                   void* stream);
-/* The two calls above with explicit element types (CTDD_DTYPE_F32 / CTDD_DTYPE_BF16; the calls above are these with
- * fp32 everywhere).  bf16 mu / log_scale / grad_logits are widened on load (exact) and the fp32 arithmetic runs unchanged:
- *   - ctdd_logistic_logits_ex: fp32 logits_out equal those of the fp32 call on the widened inputs bit for bit; bf16
- *     logits_out are those values rounded once, to nearest even.  Four logits are stored at once when S % 4 == 0 and
- *     logits_out is aligned to 4 elements (16 bytes fp32, 8 bytes bf16), one at a time otherwise;
+/* The two calls above with explicit element types (the calls above are these with fp32 everywhere).  in_dtype (mu /
+ * log_scale) is CTDD_DTYPE_F32 or CTDD_DTYPE_BF16; out_dtype (logits_out) and grad_dtype (grad_logits) are
+ * CTDD_DTYPE_F32, CTDD_DTYPE_BF16 or CTDD_DTYPE_F16.  2-byte inputs are widened on load (exact) and the fp32 arithmetic
+ * runs unchanged:
+ *   - ctdd_logistic_logits_ex: fp32 logits_out equal those of the fp32 call on the widened inputs bit for bit; bf16 and
+ *     fp16 logits_out are those values rounded once, to nearest even (fp16: overflow gives +-inf, small values become
+ *     subnormals).  Four logits are stored at once when S % 4 == 0 and logits_out is aligned to 4 elements (16 bytes
+ *     fp32, 8 bytes for the 2-byte types), one at a time otherwise;
  *   - ctdd_logistic_logits_backward_ex: grad_mu / grad_log_scale stay fp32 (at the addressing of mu) and equal those of
  *     the fp32 call on the widened tensors bit for bit, provided grad_logits is aligned to 4 of its elements whenever the
  *     widened copy is 16-byte aligned (the accumulation order depends on that alignment, not on the type).
- * An unknown dtype is refused with status 2 before any launch. */
+ * Any other dtype is refused with status 2 before any launch. */
 int ctdd_logistic_logits_ex(const void* mu, const void* log_scale, int in_dtype, int N, int D, int64_t batch_stride, int S,
                             int fix_logistic, void* logits_out, int out_dtype, void* stream);
 int ctdd_logistic_logits_backward_ex(const void* mu, const void* log_scale, int in_dtype, const void* grad_logits,
@@ -278,21 +283,21 @@ typedef struct ctdd_loss_params {
   float* out_nll;        /* sum_d CrossEntropy(logits[b,d,:], x0[b,d])                            */
   /* backward: grad_logits[b] = ga[b]*d out_a + gb[b]*d out_b + gd[b]*d out_d + gn[b]*d out_nll */
   const float* ga; const float* gb; const float* gd; const float* gn;
-  void* grad_logits;     /* [B,D,S] of logits_dtype (bf16 logits get a bf16 gradient) */
+  void* grad_logits;     /* [B,D,S] of logits_dtype (bf16 / fp16 logits get a bf16 / fp16 gradient) */
   void* workspace;       /* >= ctdd_loss_workspace_bytes(kind, B, S); written by forward, read by backward */
   /* appended field (zero-initialised = CUDA-core contractions).  S == 256, kinds SDDM and CRM with reverse_prob /
    * reverse_logscale: >= ctdd_loss_tc_scratch_bytes(B, D, S) bytes, 16-byte aligned; the two (B*D x S)(S x S) contractions
    * then run on tcgen05 (ctdd_bgemm256_tc).  Written by forward, read AND overwritten by backward: pass the same buffer to
    * both calls, untouched in between.  Ignored for CT-ELBO and the `direct` logit type. */
   void* tc_scratch;
-  /* Element type of `logits` and `grad_logits` (appended field; zero-initialised = fp32): CTDD_DTYPE_F32 or
-   * CTDD_DTYPE_BF16, as in ctdd_step_params.  bf16 takes the logits a network run under
-   * torch.autocast(dtype=torch.bfloat16) emits without a widening copy: the kernels widen on load (exact), run the fp32
-   * arithmetic, and round the gradient once (to nearest even) when they store it.  The per-sample outputs equal those of
-   * the same call on the widened logits up to the order of the per-CTA atomicAdds, and grad_logits equals that call's
-   * fp32 gradient rounded to bf16, bit for bit.  The outputs, ga..gn, workspace and tc_scratch stay fp32.  On the
-   * tensor-core path (tc_scratch at S == 256) logits and grad_logits must be 16-byte aligned for either type; other
-   * pointers are refused with status 2 before any launch. */
+  /* Element type of `logits` and `grad_logits` (appended field; zero-initialised = fp32): CTDD_DTYPE_F32,
+   * CTDD_DTYPE_BF16 or CTDD_DTYPE_F16, as in ctdd_step_params.  bf16 and fp16 take the logits a network run under
+   * torch.autocast (bf16 or its default fp16) emits without a widening copy: the kernels widen on load (exact), run the
+   * fp32 arithmetic, and round the gradient once (to nearest even) when they store it.  The per-sample outputs equal
+   * those of the same call on the widened logits up to the order of the per-CTA atomicAdds, and grad_logits equals that
+   * call's fp32 gradient rounded to the logits' type, bit for bit (fp16: overflow gives +-inf, as a loss scaler expects).
+   * The outputs, ga..gn, workspace and tc_scratch stay fp32.  On the tensor-core path (tc_scratch at S == 256) logits and
+   * grad_logits must be 16-byte aligned for every type; other pointers are refused with status 2 before any launch. */
   int32_t logits_dtype;  /* CTDD_DTYPE_* */
 } ctdd_loss_params;
 

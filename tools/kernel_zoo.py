@@ -67,9 +67,10 @@ def model_for(wname):
 def steps():
     # C1 / C2 also at 16 x the configuration's batch (VERDICT r1 #10: the HBM-rate claim of the small-S kernels is made there;
     # at the configurations' own batch the inputs fit in L2 and back-to-back Python calls time the host).  The C4 Euler line
-    # times the Euler kernel at the C4 shape: no configuration samples with Euler at S = 256.  Every line has a bf16 twin
-    # (the logits a network run under torch.autocast(dtype=torch.bfloat16) emits), and the C4 tau-leap step is also timed
-    # through the route bf16 logits took before the kernels read them: a .float() copy, then the fp32 step.
+    # times the Euler kernel at the C4 shape: no configuration samples with Euler at S = 256.  Every line has a bf16 and an
+    # fp16 twin (the logits a network run under torch.autocast emits, with dtype=torch.bfloat16 or its default fp16), and
+    # the C4 tau-leap step is also timed through the route 2-byte logits took before the kernels read them: a .float()
+    # copy, then the fp32 step.
     for wname, t, mult, mname in (("C1", 0.5, 1, None), ("C1", 0.5, 16, None), ("C2", 0.1, 1, None), ("C2", 0.1, 16, None),
                                   ("C3", 0.5, 1, None), ("C4", 0.5, 1, None), ("C4", 0.5, 1, "euler")):
         w, model = model_for(wname)
@@ -94,14 +95,17 @@ def steps():
         what = f"{wname}: S={S} D={D} N={B} {mname} t={t}"
         report(name, what, timed(lambda: run(lg)), bytes_=4.0 * B * D * S + 8.0 * B * D,
                flop=2.0 * B * D * S * S if S == 256 else None)
-        lgb = lg.to(torch.bfloat16)
+        lgb, lgh = lg.to(torch.bfloat16), lg.to(torch.float16)
         del lg
-        report(name, what + " bf16 logits", timed(lambda: run(lgb)), bytes_=2.0 * B * D * S + 8.0 * B * D,
-               flop=2.0 * B * D * S * S if S == 256 else None)
+        for tag, lg2 in ((" bf16 logits", lgb), (" fp16 logits", lgh)):
+            report(name, what + tag, timed(lambda: run(lg2)), bytes_=2.0 * B * D * S + 8.0 * B * D,
+                   flop=2.0 * B * D * S * S if S == 256 else None)
         if wname == "C4" and mname == "tau_leap":
-            report("widening copy + " + name, what + " bf16 logits through .float() and the fp32 step", timed(lambda: run(lgb.float())),
-                   bytes_=2.0 * B * D * S + 8.0 * B * D, note="the copy reads 2 and writes 4 bytes per logit on top of the step")
-        del lgb
+            for tag, lg2 in ((" bf16 logits", lgb), (" fp16 logits", lgh)):
+                report("widening copy + " + name, what + tag + " through .float() and the fp32 step",
+                       timed(lambda: run(lg2.float())), bytes_=2.0 * B * D * S + 8.0 * B * D,
+                       note="the copy reads 2 and writes 4 bytes per logit on top of the step")
+        del lgb, lgh
     # C4 with the truncated-logistic head fused into the step (the CIFAR10 configuration's head): the (mu, log_scale) pair
     # as the two torch.chunk halves of a (B, 2D) network output, fp32, bf16 (a U-Net under torch.autocast), and bf16
     # through the former per-step widening (.float() of the (B, 2D) output, then the fp32 head step)
@@ -142,7 +146,7 @@ def steps():
     def run_block(logits):
         ops.reverse_step(nat.MODE_TAU_LEAP, nat.BRANCH_TAULDR, logits, x, Q[0], QT[0], Rb, RbT, beta[0], 1e-3, 1e-9, N=B, D=D, S=S,
                          seed=1, offset=0, impl=nat.IMPL_SIMT)
-    for logits, esz, tag in ((lg, 4, ""), (lg.to(torch.bfloat16), 2, " bf16 logits")):
+    for logits, esz, tag in ((lg, 4, ""), (lg.to(torch.bfloat16), 2, " bf16 logits"), (lg.to(torch.float16), 2, " fp16 logits")):
         report("step_block_kernel", f"S=256 D=784 N={B} tau_leap (CUDA-core path){tag}", timed(lambda: run_block(logits)),
                bytes_=esz * B * D * S + 8.0 * B * D, flop=2.0 * B * D * S * S)
 
@@ -172,10 +176,11 @@ def forward_process():
 
 
 def losses():
-    # Each line has a bf16 twin (the logits a network run under torch.autocast(dtype=torch.bfloat16) emits, read as they
-    # are, with a bf16 gradient) and a line for the route bf16 logits took before the kernels read them: a .float() copy
-    # before ops.loss_terms, the fp32 gradient cast back to bf16 by autograd.  The three run alternately, and each reports
-    # the peak device memory of one forward + backward over what was allocated before it.
+    # Each line has a bf16 and an fp16 twin (the logits a network run under torch.autocast emits, with
+    # dtype=torch.bfloat16 or its default fp16, read as they are, with a gradient of their dtype) and a line for the route
+    # 2-byte logits took before the kernels read them: a .float() copy before ops.loss_terms, the fp32 gradient cast back
+    # by autograd.  They run alternately, and each reports the peak device memory of one forward + backward over what was
+    # allocated before it.
     w, model = model_for("C4")
     S = 256
     Rb, _ = model.base_rate_tables(dev)
@@ -187,7 +192,7 @@ def losses():
         x0 = torch.randint(0, S, (B, D), device=dev, dtype=torch.int32)
         xt, xtil = ops.noise_xt(Q, Rb, beta, x0, 1, 0)
         lf32 = (torch.randn(B, D, S, device=dev) - (torch.arange(S, device=dev).view(1, 1, S) - x0.unsqueeze(-1)) ** 2 / 128.0)
-        lb16 = lf32.to(torch.bfloat16)
+        lb16, lh16 = lf32.to(torch.bfloat16), lf32.to(torch.float16)
 
         def fwd(logits):
             return ops.loss_terms(logits, kind, Q=Q, QT=QT, Rb=Rb, beta=beta, x0=x0, xt=xtil if kind != nat.LOSS_CRM else xt,
@@ -204,8 +209,9 @@ def losses():
             fwd_bwd(leaf, widen)
             torch.cuda.synchronize()
             return torch.cuda.max_memory_allocated() - base
-        for tag, leaf, esz, widen in (("", lf32, 4, False), (" bf16 logits", lb16, 2, False),
-                                      (" bf16 logits through .float()", lb16, 2, True)):
+        for tag, leaf, esz, widen in (("", lf32, 4, False), (" bf16 logits", lb16, 2, False), (" fp16 logits", lh16, 2, False),
+                                      (" bf16 logits through .float()", lb16, 2, True),
+                                      (" fp16 logits through .float()", lh16, 2, True)):
             leaf.requires_grad_(True)
             with torch.no_grad():
                 ms_f = timed(lambda: fwd(leaf.float() if widen else leaf))
@@ -220,17 +226,20 @@ def losses():
 
 def head():
     # fp32 head; bf16 (mu, log_scale) with bf16 logits and a bf16 incoming gradient (a U-Net under torch.autocast feeding
-    # the bf16 loss path); and the former route for bf16 network output: .float() of mu / log_scale, then the fp32 head
+    # the bf16 loss path); fp32 (mu, log_scale) with fp16 logits and an fp16 incoming gradient (what fp16 autocast runs:
+    # its fp16 (mu, log_scale) are widened); and the former route for bf16 network output: .float() of mu / log_scale,
+    # then the fp32 head
     B, D, S = 128, 3072, 256
     mu32 = torch.tanh(torch.randn(B, D, device=dev))
     ls32 = torch.randn(B, D, device=dev)
     g32 = torch.randn(B, D, S, device=dev)
-    for tag, dt, widen in (("", torch.float32, False), (" bf16 in / bf16 out / bf16 gradient", torch.bfloat16, False),
-                           (" bf16 in through .float(), fp32 head", torch.bfloat16, True)):
+    for tag, dt, out_dt, widen in (("", torch.float32, torch.float32, False),
+                                   (" bf16 in / bf16 out / bf16 gradient", torch.bfloat16, torch.bfloat16, False),
+                                   (" fp32 in / fp16 out / fp16 gradient", torch.float32, torch.float16, False),
+                                   (" bf16 in through .float(), fp32 head", torch.bfloat16, torch.float32, True)):
         mu = mu32.to(dt).requires_grad_(True)
         ls = ls32.to(dt).requires_grad_(True)
-        out_dt = torch.bfloat16 if (dt == torch.bfloat16 and not widen) else torch.float32
-        esz = 2 if out_dt == torch.bfloat16 else 4
+        esz = 2 if out_dt != torch.float32 else 4
         g = g32.to(out_dt)
 
         def fwd():
@@ -247,8 +256,8 @@ def head():
         report("logistic_logits_kernel + logistic_backward_kernel", f"head forward + backward B={B} D={D} S=256{tag}",
                timed(fb), bytes_=2.0 * esz * B * D * S)
     del g32, g
-    # The image training leg: head + SDDMElbo loss terms (tensor-core path), forward + backward, from bf16 network output
-    # (torch.autocast) against the cast-to-fp32 route (fp32 head, fp32 logits into the loss, fp32 gradient back)
+    # The image training leg: head + SDDMElbo loss terms (tensor-core path), forward + backward, from bf16 or fp16 network
+    # output (torch.autocast) against the cast-to-fp32 route (fp32 head, fp32 logits into the loss, fp32 gradient back)
     w, model = model_for("C5")
     Rb, _ = model.base_rate_tables(dev)
     for B in (64, 512):
@@ -257,30 +266,36 @@ def head():
         beta = torch.tensor([float(b) for b in beta], dtype=torch.float32, device=dev)
         x0 = torch.randint(0, S, (B, D), generator=gen, device=dev, dtype=torch.int32)
         _, xtil = ops.noise_xt(Q, Rb, beta, x0, 3, 0)
-        mu = torch.tanh(torch.randn(B, D, generator=gen, device=dev)).to(torch.bfloat16).requires_grad_(True)
-        ls = (torch.randn(B, D, generator=gen, device=dev) - 1.0).to(torch.bfloat16).requires_grad_(True)
+        mu32 = torch.tanh(torch.randn(B, D, generator=gen, device=dev))
+        ls32 = torch.randn(B, D, generator=gen, device=dev) - 1.0
+        mu, ls = mu32.to(torch.bfloat16).requires_grad_(True), ls32.to(torch.bfloat16).requires_grad_(True)
+        muh, lsh = mu32.to(torch.float16).requires_grad_(True), ls32.to(torch.float16).requires_grad_(True)
 
-        def leg(widen):
-            if widen:
+        def leg(widen, half=False):
+            if half:
+                logits = ops.logistic_logits_autograd(muh, lsh, S, False, out_dtype=torch.float16)
+            elif widen:
                 logits = ops.logistic_logits_autograd(mu.float(), ls.float(), S, False)
             else:
                 logits = ops.logistic_logits_autograd(mu, ls, S, False, out_dtype=torch.bfloat16)
             outs = ops.loss_terms(logits, nat.LOSS_SDDM, Q, QT, Rb, beta, x0, xtil, eps=1e-9,
                                   logit_branch=nat.BRANCH_SDDM_REVERSE_PROB)
             (outs[0].sum() + outs[1].sum() + 0.01 * outs[4].sum()).backward()
-            mu.grad = ls.grad = None
+            mu.grad = ls.grad = muh.grad = lsh.grad = None
 
-        def peak(widen):
+        def peak(widen, half):
             torch.cuda.synchronize()
             base = torch.cuda.memory_allocated()
             torch.cuda.reset_peak_memory_stats()
-            leg(widen)
+            leg(widen, half)
             torch.cuda.synchronize()
             return torch.cuda.max_memory_allocated() - base
-        for tag, widen in ((" bf16 (mu, log_scale), bf16 logits", False), (" bf16 (mu, log_scale) through .float(), fp32 logits", True)):
+        for tag, widen, half in ((" bf16 (mu, log_scale), bf16 logits", False, False),
+                                 (" fp16 (mu, log_scale), fp16 logits", False, True),
+                                 (" bf16 (mu, log_scale) through .float(), fp32 logits", True, False)):
             report("head + SDDM loss_terms", f"image training leg B={B} D={D} S=256 forward + backward{tag}",
-                   timed(lambda: leg(widen)), note="torch autograd glue included", peak=peak(widen))
-        del Q, QT, mu, ls
+                   timed(lambda: leg(widen, half)), note="torch autograd glue included", peak=peak(widen, half))
+        del Q, QT, mu, ls, muh, lsh
 
 
 if __name__ == "__main__":
