@@ -5,7 +5,11 @@ package; the product path (ctdd_b200) never does.
 
 The reference (TAUnSDDM) draws with torch.poisson / Categorical.sample / torch.rand and sets no seeds, so
 "identical inputs and injected uniforms" (BASELINE.json north_star) needs a shared uniform -> sample map.
-This module defines that map bit-for-bit the way the CUDA kernels evaluate it:
+This module defines that map with the fp32 roundings the CUDA kernels make (fused multiply-adds rounded once, like FFMA),
+except where a device math function has no bit-exact host twin: expf in the Poisson pmf recurrence and in P(K >= 1)
+(numpy's exp may differ by an ulp) and normcdfinvf in the Cornish-Fisher quantile (fp64 ndtri rounded to fp32 here: a
+few ulps apart).  Those can move a jump count only when its uniform sits within ~1e-6 (relative rate) of a threshold;
+poisson_count_margin finds such rows:
 
   * Philox4x32-10 (Salmon et al., SC'11; Random123 constants) keyed on (seed), counter =
     (state s | sub-index, global-row group, call offset, stream id);
@@ -124,7 +128,25 @@ def row_units_at(grow: np.ndarray, offset: int, stream: int, seed: int, sub: int
 
 
 def _fma32(a, b, c):
-    return (np.asarray(a, np.float64) * np.asarray(b, np.float64) + np.asarray(c, np.float64)).astype(np.float32)
+    """fp32 fused multiply-add (device FFMA): a * b + c rounded once to nearest even.
+
+    The product of two fp32 values is exact in fp64; the fp64 sum may round, and rounding that sum again to fp32 is
+    wrong only when the fp64 sum lands exactly halfway between two fp32 values: then the sign of the exact residual of
+    the sum (two-sum) decides."""
+    a, b, c = np.broadcast_arrays(np.asarray(a, np.float32).astype(np.float64), np.asarray(b, np.float32).astype(np.float64),
+                                  np.asarray(c, np.float32).astype(np.float64))
+    p = a * b
+    s = p + c
+    bv = s - p
+    err = (p - (s - bv)) + (c - bv)           # p + c == s + err exactly
+    with np.errstate(over="ignore", invalid="ignore"):
+        r = s.astype(np.float32)
+        up = s > r.astype(np.float64)
+        nxt = np.nextafter(r, np.where(up, np.float32(np.inf), np.float32(-np.inf)).astype(np.float32))
+        mid = (r.astype(np.float64) + nxt.astype(np.float64)) * 0.5
+        tie = (s != r.astype(np.float64)) & (s == mid) & (err != 0)
+        beyond = np.where(up, err > 0, err < 0)        # the exact value lies past the midpoint, towards nxt
+    return np.where(tie & beyond, nxt, r).astype(np.float32)
 
 
 def poisson_sf0(lam: np.ndarray) -> np.ndarray:
@@ -138,8 +160,23 @@ def poisson_sf0(lam: np.ndarray) -> np.ndarray:
     return np.where(lam < np.float32(0.015625), small, big)
 
 
+def _cornish_fisher(lam: np.ndarray, v: np.ndarray):
+    """lam > 64: (z, f) of the device's Cornish-Fisher quantile f = lam + sqrt(lam) z + (z^2 - 1) / 6, z the upper-tail
+    normal quantile of v, all fp32.  The device evaluates f as three fused multiply-adds (each rounded once):
+    t = fma(sqrtf(lam), z, lam), u = fma(z, z, -1), f = fma(u, 0.16666667, t).  Its z comes from normcdfinvf, this one
+    from fp64 ndtri rounded to fp32: the two may differ by a few ulps of z (poisson_rows_margin allows for it)."""
+    from scipy.special import ndtri
+    lb = np.minimum(np.asarray(lam, np.float32), np.float32(1.0e9))
+    z = (-ndtri(np.asarray(v, np.float32).astype(np.float64))).astype(np.float32)
+    t = _fma32(np.sqrt(lb).astype(np.float32), z, lb)
+    u = _fma32(z, z, np.float32(-1.0))
+    return z, _fma32(u, np.float32(0.16666667), t)
+
+
 def poisson_from_unit(lam: np.ndarray, v: np.ndarray) -> np.ndarray:
-    """Upper-tail inverse CDF  k = #{j >= 0 : v < P(K > j)}  (int64), same op order as the device code."""
+    """Upper-tail inverse CDF  k = #{j >= 0 : v < P(K > j)}  (int64), with the device's fp32 roundings: lam <= 64 the
+    pmf recurrence in the device's op order (exp may differ from the device's expf by an ulp); lam > 64 the
+    Cornish-Fisher quantile of _cornish_fisher (z may differ by a few ulps)."""
     lam = np.asarray(lam, dtype=np.float32)
     v = np.asarray(v, dtype=np.float32)
     k = np.zeros(lam.shape, dtype=np.int64)
@@ -173,11 +210,7 @@ def poisson_from_unit(lam: np.ndarray, v: np.ndarray) -> np.ndarray:
         out[si] = kk
     bi = np.flatnonzero(~small)
     if bi.size:
-        from scipy.special import ndtri
-        lb = np.minimum(l[bi], np.float32(1.0e9))
-        z = (-ndtri(vv[bi].astype(np.float64))).astype(np.float32)
-        kf = (lb + np.sqrt(lb).astype(np.float32) * z).astype(np.float32)
-        kf = (kf + ((z * z - np.float32(1.0)) * np.float32(0.16666667)).astype(np.float32)).astype(np.float32)
+        _, kf = _cornish_fisher(l[bi], vv[bi])
         kf = np.rint(kf)
         kf = np.where(kf > 1.0, kf, 1.0)
         kf = np.minimum(kf, 2.0e9)
@@ -248,9 +281,10 @@ def poisson_rows(lam: np.ndarray, row_offset: int, offset: int, seed: int):
 
     lam (rows, S) fp32 >= 0. Returns (counts (rows, S) int64, total (rows,) int64); counts.sum(1) == sum over the
     chunks of min(K_chunk, cap).  The S states are cut into chunks of JUMP_CHUNK = 32 consecutive states; every chunk
-    is an independent superposition draw.  Op order = device order of the CUDA-core kernels: sequential fp32 cumsum
-    over the chunk's states, total = last cumsum entry, K = poisson_from_unit(total, v0), pick j = first s with
-    cum[s] > min(v_j, 1 - 2^-24) * total; Philox call index of chunk c = (c << 16) + call.
+    is an independent superposition draw.  Op order of the CUDA-core kernels: sequential fp32 cumsum over the chunk's
+    states, total = last cumsum entry, K = poisson_from_unit(total, v0) (module docstring: expf / normcdfinvf are the
+    only host-device differences), pick j = first s with cum[s] > min(v_j, 1 - 2^-24) * total; Philox call index of
+    chunk c = (c << 16) + call.
     """
     lam = np.ascontiguousarray(lam, dtype=np.float32)
     rows, S = lam.shape
@@ -273,14 +307,47 @@ def poisson_rows(lam: np.ndarray, row_offset: int, offset: int, seed: int):
 # The parity tests assert that every mismatching row has a margin below the rate tolerance.
 
 
-def poisson_rows_margin(lam: np.ndarray, row_offset: int, offset: int, seed: int) -> np.ndarray:
+CF_Z_ULPS = 8   # normcdfinvf (device) against ndtri rounded to fp32 (oracle): a few ulps of z apart
+
+
+def poisson_count_margin(tot: np.ndarray, v0: np.ndarray) -> np.ndarray:
+    """fp64: smallest RELATIVE change of the rate total `tot` (fp32) that would move K = poisson_from_unit(tot, v0).
+
+    tot <= 64 (exact pmf recurrence): v0 against the two neighbouring thresholds P(K > j), j in {K-1, K}; a relative
+    change d of tot moves P(K > j) by pmf(j) * tot * d, so the margin is |v0 - P(K > j)| / (pmf(j) * tot).
+    tot > 64 (Cornish-Fisher): K = rint(f), f = tot + sqrt(tot) z + (z^2 - 1)/6 (_cornish_fisher), so K moves when f
+    crosses K -+ 1/2 (only K + 1/2 when K = 1 is the clamp); a relative change d moves f by
+    tot (1 + z / (2 sqrt(tot))) d.  The distance is first reduced by what CF_Z_ULPS ulps of z move f, so a row the two
+    quantile functions may decide differently has margin 0.  inf where tot <= 0."""
+    from scipy.stats import poisson as sp
+    tot = np.asarray(tot, np.float32)
+    v0 = np.asarray(v0, np.float32)
+    K = poisson_from_unit(tot, v0)
+    t = np.where(tot > 0, tot, np.float32(1.0)).astype(np.float64)
+    v = v0.astype(np.float64)
+    with np.errstate(divide="ignore", invalid="ignore", over="ignore", under="ignore"):
+        m = np.abs(v - sp.sf(K, t)) / np.maximum(sp.pmf(K, t) * t, 1e-300)
+        m1 = np.abs(v - sp.sf(K - 1, t)) / np.maximum(sp.pmf(np.maximum(K - 1, 0), t) * t, 1e-300)
+    m = np.where(K >= 1, np.minimum(m, m1), m)
+    big = (tot > np.float32(64.0)) & (v0 < poisson_sf0(np.where(tot > 0, tot, np.float32(1.0))))
+    if big.any():
+        z, f = _cornish_fisher(tot[big], v0[big])
+        z64, f64, t64, Kb = z.astype(np.float64), f.astype(np.float64), t[big], K[big]
+        dist = np.abs(f64 - (Kb + 0.5))
+        dist = np.where(Kb > 1, np.minimum(dist, np.abs(f64 - (Kb - 0.5))), dist)
+        dz = CF_Z_ULPS * np.spacing(np.abs(z)).astype(np.float64)
+        slack = (np.sqrt(t64) + np.abs(z64) / 3.0) * dz + np.spacing(np.abs(f)).astype(np.float64)
+        slope = np.maximum(t64 * (1.0 + z64 / (2.0 * np.sqrt(t64))), 1e-300)
+        m[big] = np.maximum(dist - slack, 0.0) / slope
+    return np.where(tot > 0, m, np.inf)
+
+
+def poisson_rows_margin(lam: np.ndarray, row_offset: int, offset: int, seed: int, picks: bool = True) -> np.ndarray:
     """fp64 (rows,): smallest RELATIVE rate change that would move a decision of poisson_rows on that row.
 
-    Per chunk: (a) the count: v0 against the two neighbouring thresholds P(K > j), j in {K-1, K}; a relative change
-    d of the chunk total Lam moves P(K > j) by pmf(j) * Lam * d, so the margin is |v0 - P(K > j)| / (pmf(j) * Lam);
-    (b) every pick: |v_j * total - cum[s]| / total for the two prefix sums around the chosen state.  inf when the row
-    has no positive rate."""
-    from scipy.stats import poisson as sp
+    Per chunk: (a) the count (poisson_count_margin of the chunk total); (b) with `picks`, every pick:
+    |v_j * total - cum[s]| / total for the two prefix sums around the chosen state.  inf when the row has no positive
+    rate."""
     lam = np.ascontiguousarray(lam, dtype=np.float32)
     rows, S = lam.shape
     grow = np.arange(rows, dtype=np.uint64) + np.uint64(row_offset)
@@ -289,27 +356,21 @@ def poisson_rows_margin(lam: np.ndarray, row_offset: int, offset: int, seed: int
         w = lam[:, c0:min(c0 + JUMP_CHUNK, S)]
         cum = np.cumsum(w, axis=1, dtype=np.float32).astype(np.float64)
         tot = cum[:, -1]
-        pos = tot > 0
-        v0 = count_units(grow, offset, seed, ci << 16, S <= JUMP_SHARED_MAX_S).astype(np.float64)
-        K = poisson_from_unit(tot.astype(np.float32), v0.astype(np.float32))
-        t = np.where(pos, tot, 1.0)
-        with np.errstate(divide="ignore", invalid="ignore", over="ignore", under="ignore"):
-            m = np.abs(v0 - sp.sf(K, t)) / np.maximum(sp.pmf(K, t) * t, 1e-300)
-            m1 = np.abs(v0 - sp.sf(K - 1, t)) / np.maximum(sp.pmf(np.maximum(K - 1, 0), t) * t, 1e-300)
-        m = np.where(K >= 1, np.minimum(m, m1), m)
-        margin = np.where(pos, np.minimum(margin, m), margin)
+        v0 = count_units(grow, offset, seed, ci << 16, S <= JUMP_SHARED_MAX_S)
+        K = poisson_from_unit(tot.astype(np.float32), v0)
+        margin = np.minimum(margin, poisson_count_margin(tot.astype(np.float32), v0))
         idx = np.flatnonzero(K > 0)
-        if idx.size == 0:
+        if idx.size == 0 or not picks:
             continue
         Kc = np.minimum(K[idx], JUMP_PICK_CAP)
         kmax = int(Kc.max())
-        picks = rowjump_pick_units(grow[idx], offset, seed, kmax, ci << 16).astype(np.float64)
+        pu = rowjump_pick_units(grow[idx], offset, seed, kmax, ci << 16).astype(np.float64)
         c = cum[idx]
         for j in range(kmax):
             live = np.flatnonzero(Kc > j)
             if live.size == 0:
                 break
-            target = np.minimum(picks[live, j], 0.99999994) * tot[idx[live]]
+            target = np.minimum(pu[live, j], 0.99999994) * tot[idx[live]]
             d = np.abs(c[live] - target[:, None]).min(axis=1) / tot[idx[live]]
             margin[idx[live]] = np.minimum(margin[idx[live]], d)
     return margin
